@@ -10,6 +10,10 @@ bit-identical to the two kernels back to back, which --no-overlap times instead)
 
     python bench.py [--gpus N] [--steps K] [--warmup W]            # this repo's CUDA path
     python bench.py --impl reference [...]                          # the reference algorithm on the host cores
+    python bench.py --dump-outputs DIR [...]                        # also save a sample of the last timed step's results
+
+`--dump-outputs` writes what the last timed step returned to its caller as DIR/<name>.npy (float64, a fixed seeded sample
+of the satellites, under 64 MB in all), so that two builds run with the same arguments can be compared output for output.
 
 Under torchrun (N>1) every rank processes its own 4096-satellite shard (weak scaling) and the discretized
 matrices are all-gathered over NVLink inside the timed step, as north_star asks (fused into the kernel: peer stores;
@@ -101,6 +105,26 @@ def make_constellation(n_sats, seed=20240531):
     Y[:, 3], Y[:, 4] = (ca * y[3] - sa * y[4]) * f, (sa * y[3] + ca * y[4]) * f
     Y[:, 5] = y[5] * f
     return Y, const
+
+
+DUMP_BYTES = 48 << 20
+
+
+def dump_outputs(path, out, x, u, status_prop, status_disc):
+    """--dump-outputs: the arrays the step hands its caller (the [105, N*(K-1)] matrices, the propagated states [N,7,K] and
+    inputs [N,3,K], both status arrays), restricted to a seeded sample of satellites that depends on N and K only, with
+    every interval of a sampled satellite kept; at most DUMP_BYTES of float64 (status codes as numbers)."""
+    import torch
+    N, _, K = x.shape
+    per_sat = 8 * (105 * (K - 1) + 10 * K + 1 + (K - 1))
+    n = min(N, max(1, DUMP_BYTES // per_sat))
+    sats = np.sort(np.random.default_rng(0).choice(N, size=n, replace=False))
+    cols = (sats[:, None] * (K - 1) + np.arange(K - 1)).ravel()
+    si, ci = torch.from_numpy(sats).to(x.device), torch.from_numpy(cols).to(x.device)
+    os.makedirs(path, exist_ok=True)
+    for name, a in (("out", out[:, ci]), ("x", x[si]), ("u", u[si]), ("status_prop", status_prop[si]),
+                    ("status_disc", status_disc[ci])):
+        np.save(os.path.join(path, name + ".npy"), a.cpu().numpy().astype(np.float64))
 
 
 class ClockSampler(threading.Thread):
@@ -511,6 +535,9 @@ def gpu_arm(args):
         torch.cuda.synchronize(dev)
         step_ms.append(e0.elapsed_time(e3))
     launches = M.launch_count() - launches0
+    if args.dump_outputs:
+        # before the stand-alone kernel timings below overwrite the buffers
+        dump_outputs(args.dump_outputs, out, x, u, stp, std)
     # The two kernels on their own (same inputs, same L2 flush, same clock sampling window): the discretization
     # kernel's launch duration is what `roofline` is computed from.  Inside the overlapped step the same kernel runs
     # as windows beside the propagation, so it cannot be bracketed by events there.
@@ -760,7 +787,13 @@ def main():
     ap.add_argument("--prop", default="rk45", choices=["rk45", "rk4"],
                     help="propagator: the reference's RK45 replayed step for step (default) or fixed-step RK4")
     ap.add_argument("--windows", type=int, default=0, help="windows along k of the overlapped pass (0 = library default)")
+    ap.add_argument("--dump-outputs", dest="dump_outputs", metavar="DIR", default=None,
+                    help="write a seeded sample of the last timed step's results to DIR/<name>.npy (one GPU)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.gpus != 1 or int(os.environ.get("WORLD_SIZE", "1")) != 1):
+        ap.error("--dump-outputs needs the CUDA path on one GPU")
     if args.impl == "reference":
         reference_arm(args)
     else:

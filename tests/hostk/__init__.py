@@ -11,6 +11,7 @@ This is a checker, like oracle/: nothing in mpconstellation_b200/ may import it,
 shipped, and it says nothing about performance.
 """
 import ctypes
+import fcntl
 import os
 import re
 import subprocess
@@ -40,23 +41,35 @@ def build(force=False, sanitize=False):
 def _build(SO, force, opt):
     srcs = [os.path.join(CSRC, s) for s in SOURCES] + [os.path.join(HERE, "hostk_main.cpp"),
                                                        os.path.join(HERE, "include", "hostk_shim.h"), __file__]
-    if not force and os.path.exists(SO) and all(os.path.getmtime(SO) >= os.path.getmtime(s) for s in srcs):
+
+    def fresh():
+        return os.path.exists(SO) and all(os.path.getmtime(SO) >= os.path.getmtime(s) for s in srcs)
+    if not force and fresh():
         return SO
     os.makedirs(BUILD, exist_ok=True)
-    n_sub = 0
-    for s in SOURCES:
-        text = open(os.path.join(CSRC, s)).read()
-        for pat, rep in _SEEDS:
-            text, n = re.subn(pat, rep, text)
-            n_sub += n
-        assert "asm(" not in text, f"{s}: inline PTX the host build does not know"
-        open(os.path.join(BUILD, s), "w").write(text)
-    assert n_sub == 3, "expected exactly the three MUFU seeds (fast_rcp, fast_rcp1, fast_rsqrt) to be replaced"
-    cmd = ["g++"] + opt + ["-std=c++17", "-pthread", "-shared", "-fPIC", "-mfma", "-ffp-contract=fast", "-fno-math-errno", "-w",
-           "-I", os.path.join(HERE, "include"), "-I", BUILD, "-o", SO, os.path.join(HERE, "hostk_main.cpp")]
-    res = subprocess.run(cmd, capture_output=True, text=True)
-    if res.returncode != 0:
-        raise RuntimeError("g++ failed:\n" + res.stdout + res.stderr)
+    # Several processes can ask for the library at once (the spawned ranks of tests/test_distributed_cpu.py on a fresh
+    # checkout): one builds while the others wait, and the library is renamed into place, so that no process loads a
+    # partly written file.
+    with open(os.path.join(BUILD, ".lock"), "w") as lock:
+        fcntl.flock(lock, fcntl.LOCK_EX)
+        if not force and fresh():
+            return SO
+        n_sub = 0
+        for s in SOURCES:
+            text = open(os.path.join(CSRC, s)).read()
+            for pat, rep in _SEEDS:
+                text, n = re.subn(pat, rep, text)
+                n_sub += n
+            assert "asm(" not in text, f"{s}: inline PTX the host build does not know"
+            open(os.path.join(BUILD, s), "w").write(text)
+        assert n_sub == 3, "expected exactly the three MUFU seeds (fast_rcp, fast_rcp1, fast_rsqrt) to be replaced"
+        tmp = f"{SO}.{os.getpid()}.tmp"
+        cmd = ["g++"] + opt + ["-std=c++17", "-pthread", "-shared", "-fPIC", "-mfma", "-ffp-contract=fast", "-fno-math-errno",
+               "-w", "-I", os.path.join(HERE, "include"), "-I", BUILD, "-o", tmp, os.path.join(HERE, "hostk_main.cpp")]
+        res = subprocess.run(cmd, capture_output=True, text=True)
+        if res.returncode != 0:
+            raise RuntimeError("g++ failed:\n" + res.stdout + res.stderr)
+        os.replace(tmp, SO)
     return SO
 
 
