@@ -405,7 +405,8 @@ int64_t mpc_launch_count(void);
  * results).  23 / 24 / 25: the thread-group kernel for small batches (8 lanes per interval) off / on / at any batch size
  * (results equal to rounding).  26..29: k-windows of the streamed host pass (mpc_propagate_discretize_host_layout) 16 / 32 /
  * 48 / 64 (same results).  37 / 38: the 21-node Euler-Maclaurin form of the 101-node trapezoid sums (n_sub = 100) off / on
- * (quadrature equal to 1e-13, A_k to 1e-11). */
+ * (quadrature equal to 1e-13, A_k to 1e-11).  39 / 40: where the 21-node form applies, its 11-node form on ten
+ * fifth-order Nystrom steps off / on (quadrature equal to 1e-12, A_k to 1e-11). */
 int mpc_set_tuning(int variant);
 
 /* Options of the fused (in-kernel store) all-gather, applied by mpc_discretize_batch / _multi:

@@ -108,9 +108,10 @@ discretize_group_kernel(const double *__restrict__ x, const double *__restrict__
     const double hn = tf * h;                  // node spacing of the unscaled system
     // two-node steps where discretize_pair_kernel takes them (even number of panels, step short against the orbital rate)
     // ... and the 21-node form of the 101-node sums (kEmW, discretize_kernel.cuh) where discretize_pair_kernel takes it:
-    // 20 steps of five nodes, the step ends are the nodes of the rule
+    // 20 steps of five nodes, the step ends are the nodes of the rule; or its 11-node form kEmW3 on 10 fifth-order steps
+    // (state_step5 / column_step5, the code of discretize_thread) under the same per-interval conditions
     bool pairmode;
-    int em = 0;                     // 1: 20 steps + kEmW, 2: 50 steps + kEmW2
+    int em = 0;                     // 1: 20 steps + kEmW, 2: 50 steps + kEmW2, 3: 10 fifth-order steps + kEmW3
     {
         const double r2 = fma(rx, rx, fma(ry, ry, rz * rz));
         const double w2H2 = P.mu * (4.0 * hn * hn) / (r2 * sqrt(r2));
@@ -120,11 +121,13 @@ discretize_group_kernel(const double *__restrict__ x, const double *__restrict__
             const double e0x = hold.u0x + hold.dux, e0y = hold.u0y + hold.duy, e0z = hold.u0z + hold.duz;
             const double a2 = fma(hold.u0x, hold.u0x, fma(hold.u0y, hold.u0y, hold.u0z * hold.u0z));
             const double b2 = fma(e0x, e0x, fma(e0y, e0y, e0z * e0z));
-            if (d2 <= 0.0625 * fmax(a2, b2)) em = (w2H2 * 6.25 <= 1.2e-5) ? 1 : ((w2H2 <= 1.94e-5) ? 2 : 0);
+            if (d2 <= 0.0625 * fmax(a2, b2))
+                em = (w2H2 * 6.25 <= 1.2e-5) ? ((dst.em >= 2 && d2 <= 0.015625 * fmax(a2, b2)) ? 3 : 1)
+                                              : ((w2H2 <= 1.94e-5) ? 2 : 0);
         }
         if (em) pairmode = false;
     }
-    const int nodes_per_step = (em == 1) ? 5 : ((em == 2 || pairmode) ? 2 : 1);
+    const int nodes_per_step = (em == 3) ? 10 : (em == 1) ? 5 : ((em == 2 || pairmode) ? 2 : 1);
     const int n_steps = n_sub / nodes_per_step;
     const double H = hn * (double)nodes_per_step;      // integrator step
     // step-normalised variables as in discretize_kernel, with the step H
@@ -190,7 +193,8 @@ discretize_group_kernel(const double *__restrict__ x, const double *__restrict__
         s1.dz = -tz * im * dflag;
         const double md1 = -un * Ph.inv_ve;
         {
-            const double w = (em == 1) ? 5.0 * kEmW[j] : ((em == 2) ? 2.0 * kEmW2[j] : ((j == 0 || j == n_steps) ? 0.5 : 1.0));
+            const double w = (em == 3) ? 10.0 * kEmW3[j] : (em == 1) ? 5.0 * kEmW[j] :
+                             ((em == 2) ? 2.0 * kEmW2[j] : ((j == 0 || j == n_steps) ? 0.5 : 1.0));
             const double bs = -P.inv_ve * iun;
             const double b[3] = {bs * ux, bs * uy, bs * uz};
             const double cr[3] = {grp_bcast(pr[0], 6), grp_bcast(pr[1], 6), grp_bcast(pr[2], 6)};
@@ -199,6 +203,24 @@ discretize_group_kernel(const double *__restrict__ x, const double *__restrict__
             grp_node(A, pr, pv, cr, cv, vv, aa, gr, b, im * H, md1, (iun != 0.0) ? md1 : 0.0, w, w * (jn * inv_n), sgn, row6);
         }
         if (j == n_steps) break;
+
+        if (em == 3) {   // ---- the fifth-order step: state (every lane) and this lane's column ------------------------
+            StageLin s2, s3, s4;
+            double ue[3], uue, iune;
+            state_step5<J2>(Ph, hold, jn * inv_n, 10.0 * inv_n, eps2, rx, ry, rz, vx, vy, vz, m, a1x, a1y, a1z, md1, s2, s3, s4,
+                            ue, uue, iune, bad);
+            s2.dx *= dflag; s2.dy *= dflag; s2.dz *= dflag;
+            s3.dx *= dflag; s3.dy *= dflag; s3.dz *= dflag;
+            s4.dx *= dflag; s4.dy *= dflag; s4.dz *= dflag;
+            column_step5<true>(pr, pv, s1, s2, s3, s4);
+            ux = ue[0];
+            uy = ue[1];
+            uz = ue[2];
+            iun = iune;
+            un = uue * iune;
+            jn += 10.0;
+            continue;
+        }
 
         // ---- inputs and masses at the middle and the end of the step --------------------------------------------------
         const double sm = (jn + 0.5 * (double)nodes_per_step) * inv_n, se = (jn + (double)nodes_per_step) * inv_n;

@@ -335,7 +335,8 @@ struct DstTab {  // destination buffers of the (optionally multi-destination) So
     // consecutive columns -- whole 256-byte lines per warp, also to the peers -- instead of 13-column fragments.
     long long km_ntot, km_soff;
     // != 0: the launch may evaluate the 101-node trapezoid sums of an interval through their Euler-Maclaurin expansion
-    // (kEmW below; discretize_pair_kernel decides per interval).  Set by the launcher, mpc_set_tuning(37/38).
+    // (kEmW, kEmW2 below; discretize_pair_kernel decides per interval); >= 2: also through the 11-node form kEmW3 on
+    // fifth-order steps.  Set by the launcher, mpc_set_tuning(37/38) and (39/40).
     int em;
 };
 
@@ -599,10 +600,120 @@ __device__ __constant__ double kEmW2[51] = {
     703.0 / 1024, 171.0 / 128, 703.0 / 1024, 665.0 / 512, 703.0 / 1024, 665.0 / 512, 185.0 / 256, 665.0 / 512, 703.0 /
     1024, 665.0 / 512, 703.0 / 1024, 171.0 / 128, 703.0 / 1024, 665.0 / 512, 703.0 / 1024, 665.0 / 512, 185.0 / 512};
 constexpr int kEmSteps2 = 50;
+// The same construction on every 10th node, for the intervals of kEmW whose integrands are smoothest: the sums over every
+// 10th, 20th, 50th and 100th node, w = (11189689/8000000, -13088691/32000000, 2089791/200000000, -110789/800000000)
+// (sum w n^2r = 1, r = 0..3), one rule on the 11 nodes j = 0, 10, ..., 100 (weights in units of 10 h; they add up to 10).
+// Its remainder is 1e-16 of the 101-node sum where the integrand turns by 0.07 rad across the interval (the orbital motion
+// of a 0.01-orbit interval), 1e-15 at 0.25 rad and 2.5e-13 at 0.5 rad, so it is used for a smooth held input only.  The
+// 11 nodes are the ends of 10 steps of Nystrom's 4-stage fifth-order method (column_step5), whose own error at the step
+// 10 h is at rounding on 0.01-orbit intervals.
+__device__ __constant__ double kEmW3[11] = {
+    12630557.0 / 40000000, 11189689.0 / 8000000, 9290687.0 / 16000000, 11189689.0 / 8000000, 9290687.0 / 16000000,
+    14509559.0 / 10000000, 9290687.0 / 16000000, 11189689.0 / 8000000, 9290687.0 / 16000000, 11189689.0 / 8000000,
+    12630557.0 / 40000000};
+constexpr int kEmSteps3 = 10;
+
+// Nystrom's 4-stage fifth-order method (1925) for p'' = F(t, p), in units of the step:
+//     c = (0, 1/5, 2/3, 1),  P_s = p + c_s p' + sum_j abar_sj k_j,  k_s = F(c_s, P_s),
+//     abar_21 = 1/50,  abar_3 = (-1/27, 7/27),  abar_4 = (3/10, -2/35, 9/35),
+//     p+ = p + p' + (14 k1 + 100 k2 + 54 k3) / 336,   p'+ = p' + (14 k1 + 125 k2 + 162 k3 + 35 k4) / 336
+// One column of Phi through one step, with the stage matrices G_s (and d_s, MASSCOL) of the same scheme applied to the
+// state, so that Phi stays the exact derivative of the numerical flow (as column_step).
+template <bool MASSCOL>
+__device__ __forceinline__ void column_step5(double (&pr)[3], double (&pv)[3], const StageLin &s1, const StageLin &s2,
+                                             const StageLin &s3, const StageLin &s4)
+{
+    double k1[3], k2[3], k3[3], k4[3], q[3], b[3];
+    if (MASSCOL) sym_mul_add(s1.g, pr[0], pr[1], pr[2], s1.dx, s1.dy, s1.dz, k1[0], k1[1], k1[2]);
+    else sym_mul(s1.g, pr[0], pr[1], pr[2], k1[0], k1[1], k1[2]);
+#pragma unroll
+    for (int i = 0; i < 3; ++i) q[i] = fma(1.0 / 50, k1[i], fma(0.2, pv[i], pr[i]));
+    if (MASSCOL) sym_mul_add(s2.g, q[0], q[1], q[2], s2.dx, s2.dy, s2.dz, k2[0], k2[1], k2[2]);
+    else sym_mul(s2.g, q[0], q[1], q[2], k2[0], k2[1], k2[2]);
+#pragma unroll
+    for (int i = 0; i < 3; ++i) q[i] = fma(7.0 / 27, k2[i], fma(-1.0 / 27, k1[i], fma(2.0 / 3, pv[i], pr[i])));
+    if (MASSCOL) sym_mul_add(s3.g, q[0], q[1], q[2], s3.dx, s3.dy, s3.dz, k3[0], k3[1], k3[2]);
+    else sym_mul(s3.g, q[0], q[1], q[2], k3[0], k3[1], k3[2]);
+#pragma unroll
+    for (int i = 0; i < 3; ++i) {
+        b[i] = pv[i] + pr[i];
+        q[i] = fma(9.0 / 35, k3[i], fma(-2.0 / 35, k2[i], fma(0.3, k1[i], b[i])));
+    }
+    if (MASSCOL) sym_mul_add(s4.g, q[0], q[1], q[2], s4.dx, s4.dy, s4.dz, k4[0], k4[1], k4[2]);
+    else sym_mul(s4.g, q[0], q[1], q[2], k4[0], k4[1], k4[2]);
+#pragma unroll
+    for (int i = 0; i < 3; ++i) {
+        pr[i] = fma(9.0 / 56, k3[i], fma(25.0 / 84, k2[i], fma(1.0 / 24, k1[i], b[i])));
+        pv[i] = fma(5.0 / 48, k4[i], fma(27.0 / 56, k3[i], fma(125.0 / 336, k2[i], fma(1.0 / 24, k1[i], pv[i]))));
+    }
+}
+
+// Acceleration of the state at one stage: gravity at (rx, ry, rz) plus the held input over the stage's mass, and the
+// stage's StageLin (d = -u/m^2).
+template <bool J2>
+__device__ __forceinline__ void stage_accel(const DiscParams &Ph, double rx, double ry, double rz, double ux, double uy,
+                                            double uz, double mass, double &ax, double &ay, double &az, StageLin &s)
+{
+    gravity<J2>(Ph, rx, ry, rz, ax, ay, az, s.g);
+    const double im = fast_rcp(mass);
+    const double qx = ux * im, qy = uy * im, qz = uz * im;
+    ax += qx;
+    ay += qy;
+    az += qz;
+    s.dx = -qx * im;
+    s.dy = -qy * im;
+    s.dz = -qz * im;
+}
+
+// The state through one step of the fifth-order method above, from stage 1 (a1 = the acceleration at the step's start,
+// md1 = its mass flow) -- shared by discretize_thread and discretize_group_kernel.  The held input is evaluated at the
+// stage abscissae s0 + c_s ds (u at the end is returned in ue, with its guarded inverse norm); the mass is a quadrature
+// of mdot(tau): the cubic through mdot at the four abscissae, integrated exactly to each c_s (to c = 1 that is the
+// velocity weights b).  Returns the stage matrices of stages 2..4 for the variational columns.
+template <bool J2>
+__device__ __forceinline__ void state_step5(const DiscParams &Ph, const UHold<false> &hold, double s0, double ds, double eps2,
+                                            double &rx, double &ry, double &rz, double &vx, double &vy, double &vz, double &m,
+                                            double a1x, double a1y, double a1z, double md1, StageLin &s2, StageLin &s3,
+                                            StageLin &s4, double (&ue)[3], double &uue, double &iune, int &bad)
+{
+    double u2[3], u3[3];
+    hold.at(fma(0.2, ds, s0), 0.0, u2[0], u2[1], u2[2]);
+    hold.at(fma(2.0 / 3, ds, s0), 0.0, u3[0], u3[1], u3[2]);
+    hold.at(s0 + ds, 0.0, ue[0], ue[1], ue[2]);
+    const double uu2 = fma(u2[0], u2[0], fma(u2[1], u2[1], u2[2] * u2[2]));
+    const double uu3 = fma(u3[0], u3[0], fma(u3[1], u3[1], u3[2] * u3[2]));
+    uue = fma(ue[0], ue[0], fma(ue[1], ue[1], ue[2] * ue[2]));
+    iune = inv_norm_guarded(uue, eps2);
+    const double md2 = -(uu2 * inv_norm_guarded(uu2, eps2)) * Ph.inv_ve;
+    const double md3 = -(uu3 * inv_norm_guarded(uu3, eps2)) * Ph.inv_ve;
+    const double md4 = -(uue * iune) * Ph.inv_ve;
+    const double m2 = fma(17.0 / 6000, md4, fma(-81.0 / 7000, md3, fma(209.0 / 1680, md2, fma(253.0 / 3000, md1, m))));
+    const double m3 = fma(-2.0 / 81, md4, fma(5.0 / 21, md3, fma(250.0 / 567, md2, fma(1.0 / 81, md1, m))));
+    const double m4 = fma(5.0 / 48, md4, fma(27.0 / 56, md3, fma(125.0 / 336, md2, fma(1.0 / 24, md1, m))));
+    bad |= !(m4 > 0.0);
+
+    double a2x, a2y, a2z, a3x, a3y, a3z, a4x, a4y, a4z;
+    stage_accel<J2>(Ph, fma(1.0 / 50, a1x, fma(0.2, vx, rx)), fma(1.0 / 50, a1y, fma(0.2, vy, ry)),
+                    fma(1.0 / 50, a1z, fma(0.2, vz, rz)), u2[0], u2[1], u2[2], m2, a2x, a2y, a2z, s2);
+    stage_accel<J2>(Ph, fma(7.0 / 27, a2x, fma(-1.0 / 27, a1x, fma(2.0 / 3, vx, rx))),
+                    fma(7.0 / 27, a2y, fma(-1.0 / 27, a1y, fma(2.0 / 3, vy, ry))),
+                    fma(7.0 / 27, a2z, fma(-1.0 / 27, a1z, fma(2.0 / 3, vz, rz))), u3[0], u3[1], u3[2], m3, a3x, a3y, a3z, s3);
+    const double bx = vx + rx, by = vy + ry, bz = vz + rz;
+    stage_accel<J2>(Ph, fma(9.0 / 35, a3x, fma(-2.0 / 35, a2x, fma(0.3, a1x, bx))),
+                    fma(9.0 / 35, a3y, fma(-2.0 / 35, a2y, fma(0.3, a1y, by))),
+                    fma(9.0 / 35, a3z, fma(-2.0 / 35, a2z, fma(0.3, a1z, bz))), ue[0], ue[1], ue[2], m4, a4x, a4y, a4z, s4);
+    rx = fma(9.0 / 56, a3x, fma(25.0 / 84, a2x, fma(1.0 / 24, a1x, bx)));
+    ry = fma(9.0 / 56, a3y, fma(25.0 / 84, a2y, fma(1.0 / 24, a1y, by)));
+    rz = fma(9.0 / 56, a3z, fma(25.0 / 84, a2z, fma(1.0 / 24, a1z, bz)));
+    vx = fma(5.0 / 48, a4x, fma(27.0 / 56, a3x, fma(125.0 / 336, a2x, fma(1.0 / 24, a1x, vx))));
+    vy = fma(5.0 / 48, a4y, fma(27.0 / 56, a3y, fma(125.0 / 336, a2y, fma(1.0 / 24, a1y, vy))));
+    vz = fma(5.0 / 48, a4z, fma(27.0 / 56, a3z, fma(125.0 / 336, a2z, fma(1.0 / 24, a1z, vz))));
+    m = m4;
+}
 
 #define ACC(e) acc[(e) * BLOCK]
-// EM = 1 / 2: n_sub is kEmSteps / kEmSteps2 and node n carries the weight kEmW[n] / kEmW2[n] instead of the trapezoid's
-// 1/2, 1, ..., 1, 1/2.
+// EM = 1 / 2 / 3: n_sub is kEmSteps / kEmSteps2 / kEmSteps3 and node n carries the weight kEmW[n] / kEmW2[n] / kEmW3[n]
+// instead of the trapezoid's 1/2, 1, ..., 1, 1/2.  EM = 3 takes the fifth-order steps (state_step5, column_step5).
 template <bool J2, int BLOCK, int NDST, bool GENU, int EM = 0>
 __device__ __forceinline__ void discretize_thread(const double *__restrict__ x, const double *__restrict__ u,
                                                   const double *__restrict__ tf_arr, const DiscParams &P, int K, int Ku,
@@ -697,12 +808,30 @@ __device__ __forceinline__ void discretize_thread(const double *__restrict__ x, 
         const double md1 = -un * Ph.inv_ve;  // hs * mass flow (simulator.py:160)
         {
             const double sfrac = (double)n * inv_n;                     // lambda+   (:61)
-            const double w = (EM == 1) ? kEmW[n] : ((EM == 2) ? kEmW2[n] : ((n == 0 || n == n_sub) ? 0.5 : 1.0));   // trapezoid end weights (:77-80)
+            const double w = (EM == 1) ? kEmW[n] : ((EM == 2) ? kEmW2[n] : ((EM == 3) ? kEmW3[n] :
+                             ((n == 0 || n == n_sub) ? 0.5 : 1.0)));   // trapezoid end weights (:77-80)
             const double ws = w * sfrac;
             // D Duf = [0; hs I/m; b^T];  hs D Sigma = [v~; a~; mdot~];  hs D xi' = -[v~; G~ r; mdot~_B]
             node_accumulate<BLOCK>(acc, pr, pv, P, im * hs, ux, uy, uz, iun, md1, vx, vy, vz, a1x, a1y, a1z, grx, gry, grz, w, ws);
         }
         if (n == n_sub) break;
+
+        if constexpr (EM == 3 && !GENU) {
+            // ---- stages 2..4 of the state and the columns: Nystrom's 4-stage fifth-order method ----------------------
+            StageLin s2, s3, s4;
+            double ue[3], uue, iune;
+            state_step5<J2>(Ph, hold, (double)n * inv_n, inv_n, eps2, rx, ry, rz, vx, vy, vz, m, a1x, a1y, a1z, md1, s2, s3,
+                            s4, ue, uue, iune, bad);
+            column_step5<true>(pr[6], pv[6], s1, s2, s3, s4);
+#pragma unroll
+            for (int c = 0; c < 6; ++c) column_step5<false>(pr[c], pv[c], s1, s2, s3, s4);
+            ux = ue[0];
+            uy = ue[1];
+            uz = ue[2];
+            iun = iune;
+            un = uue * iune;
+            continue;
+        }
 
         // ---- stages 2, 3 of the state: Nystrom's 3-stage fourth-order method for r'' = a(tau, r) ----------------
         // (the mass is a quadrature of mdot(tau): m at the half step from the quadratic through the three mdot

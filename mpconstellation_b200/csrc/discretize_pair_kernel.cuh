@@ -181,6 +181,13 @@ discretize_pair_kernel(const double *__restrict__ x, const double *__restrict__ 
             const double b2 = fma(e0x, e0x, fma(e0y, e0y, e0z * e0z));
             if (d2 <= 0.0625 * fmax(a2, b2)) {
                 if (w2H2 * 6.25 <= 1.2e-5) {
+                    // the same orbital bound (omega 10h <= 7e-3 rad) and a held input that changes by at most an eighth
+                    // of its size: 10 fifth-order steps and the 11-node rule kEmW3 (its remainder grows like the eighth
+                    // power of that change: 2.5e-13 of the 101-node sums at 1/8, 4e-11 at 1/4)
+                    if (dst.em >= 2 && d2 <= 0.015625 * fmax(a2, b2)) {
+                        discretize_thread<J2, BLOCK, NDST, false, 3>(x, u, tf_arr, P, K, K, kEmSteps3, dst, pitch, offset, status, gid, acc);
+                        return;
+                    }
                     discretize_thread<J2, BLOCK, NDST, false, 1>(x, u, tf_arr, P, K, K, kEmSteps, dst, pitch, offset, status, gid, acc);
                     return;
                 }

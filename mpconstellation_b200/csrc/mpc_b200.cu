@@ -117,6 +117,9 @@ int launch_disc_cfg(const double *x, const double *u, const double *tf, const mp
 // discretize_pair_kernel: integrator steps spanning two quadrature nodes (needs an even number of panels)
 // mpc_set_tuning(37 / 38): the 21-node Euler-Maclaurin form of the 101-node trapezoid sums off / on (kEmW)
 std::atomic<int> g_em{1};
+// mpc_set_tuning(39 / 40): the 11-node form on fifth-order steps (kEmW3) off / on, for the intervals of the 21-node form
+std::atomic<int> g_em3{1};
+int em_level() { return g_em.load(std::memory_order_relaxed) ? 1 + g_em3.load(std::memory_order_relaxed) : 0; }
 
 template <bool J2, int BLOCK, int MAXREG, int NDST>
 int launch_pair_cfg(const double *x, const double *u, const double *tf, const mpc::DiscParams &P, int n_sats, int K,
@@ -137,7 +140,7 @@ int launch_pair_cfg(const double *x, const double *u, const double *tf, const mp
     const long long n_int = (long long)n_sats * kc;
     const unsigned grid = (unsigned)((n_int + BLOCK - 1) / BLOCK);
     mpc::DstTab tab = dst;
-    tab.em = g_em.load(std::memory_order_relaxed);
+    tab.em = em_level();
     kern<<<grid, BLOCK, smem, st>>>(x, u, tf, P, n_sats, K, n_sub, tab, pitch, offset, status, k0, kc);
     g_launches.fetch_add(1, std::memory_order_relaxed);
     CUDA_TRY(cudaGetLastError());
@@ -161,7 +164,7 @@ int launch_group(const double *x, const double *u, const double *tf, const mpc::
     const long long n_int = (long long)n_sats * (K - 1);
     const unsigned grid = (unsigned)((n_int * 8 + BLOCK - 1) / BLOCK);
     mpc::DstTab tab = dst;
-    tab.em = g_em.load(std::memory_order_relaxed);
+    tab.em = em_level();
     mpc::discretize_group_kernel<J2, BLOCK><<<grid, BLOCK, 0, st>>>(x, u, tf, P, n_sats, K, n_sub, tab, pitch, offset, status);
     g_launches.fetch_add(1, std::memory_order_relaxed);
     CUDA_TRY(cudaGetLastError());
@@ -439,7 +442,7 @@ int launch_disc_drag(const double *x, const double *u, const double *tf, const m
                      int32_t *status, cudaStream_t st)
 {
     mpc::DstTab tab = dst;
-    tab.em = g_em.load(std::memory_order_relaxed);
+    tab.em = em_level();
     return launch_drag_unit(false, 0, 64, x, u, tf, P, J2, kf, L, n_sats, K, n_sub, 0.0, 0.0, 0.0, tab, pitch, offset, status,
                             nullptr, st);
 }
@@ -819,6 +822,10 @@ int mpc_set_tuning(int variant)
     }
     if (variant == 37 || variant == 38) {  // 101-node trapezoid sums through their Euler-Maclaurin expansion: off / on
         g_em.store(variant - 37);
+        return MPC_SUCCESS;
+    }
+    if (variant == 39 || variant == 40) {  // 11-node form of the 101-node sums on fifth-order steps: off / on
+        g_em3.store(variant - 39);
         return MPC_SUCCESS;
     }
     if (variant >= 20 && variant <= 22) {  // default-mode kernel: threads per CTA 32 / 128 / 256
