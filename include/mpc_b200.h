@@ -202,6 +202,36 @@ int mpc_propagate_batch_rk45(const double *y0, const double *tf, const mpc_param
                              int n_sats, int T, double rtol, double atol, double max_step, double *y, double *u_out,
                              int32_t *status, int32_t *n_steps, void *stream);
 
+/*
+ * Ragged batches: satellite s has its own node count K_s = K_sat[s] (2 <= K_s <= K_max), the reference's
+ * int(base_res * tf_s) of every satellite's own horizon.  x [n_sats][7][K_max] and u [n_sats][3][K_max] are padded: only
+ * the first K_s columns of satellite s are read.  The result keeps the rectangular layout of K_max:
+ * out[row][out_offset + s (K_max-1) + k] for k < K_s - 1, status / n_nodes [n_sats][K_max-1]; the padding columns are
+ * never written.  One launch for the whole batch, the threads mapped to live intervals only.  adaptive = 0: fixed-step
+ * mode (n_sub), 1: default mode (rtol, atol, max_step, n_nodes), as mpc_discretize_batch_ugrid.
+ *   K_sat      HOST array [n_sats] (validated; it also sizes the launch)
+ *   first      DEVICE scratch of n_sats + 1 int64, filled by the call (prefix sums of K_s - 1) and read by the kernel
+ * MPC_E_UNSUPPORTED: include_drag.
+ */
+int mpc_discretize_batch_ragged(const double *x, const double *u, const double *tf, const mpc_params *p, int n_sats,
+                                int K_max, const int32_t *K_sat, int64_t *first, int adaptive, int n_sub, double rtol,
+                                double atol, double max_step, double *out, int64_t out_pitch, int64_t out_offset,
+                                int32_t *status, int32_t *n_nodes, void *stream);
+
+/*
+ * mpc_propagate_batch_rk45 with a sample count per satellite: satellite s is sampled at linspace(0, 1, T_sat[s]) into the
+ * first T_sat[s] columns of y [n_sats][7][T_max] (and u_out [n_sats][3][T_max]); the padding columns are never written.
+ * The steps do not depend on the samples: n_steps equals a rectangular run of the same satellite.
+ *   T_sat          DEVICE array [n_sats] (not read by the host; the kernel keeps every count inside [0, T_max])
+ *   table_len_sat  MPC_CTRL_SEQUENCE with a per-satellite table [n_sats][3][table_len]: satellite s uses its first
+ *                  table_len_sat[s] columns (2 .. table_len; table_len stays the stride).  DEVICE array [n_sats] or NULL
+ *                  (every satellite: table_len)
+ */
+int mpc_propagate_batch_rk45_ragged(const double *y0, const double *tf, const mpc_params *p, const mpc_controller *ctrl,
+                                    int n_sats, int T_max, const int32_t *T_sat, const int32_t *table_len_sat, double rtol,
+                                    double atol, double max_step, double *y, double *u_out, int32_t *status,
+                                    int32_t *n_steps, void *stream);
+
 /* ---------------------------------------------------------------- host API */
 typedef struct mpc_ctx mpc_ctx;
 
@@ -245,6 +275,20 @@ int mpc_propagate_batch_rk45_host(mpc_ctx *ctx, const double *y0, const double *
                                   const mpc_controller *ctrl, int n_sats, int T, double rtol, double atol,
                                   double max_step, double *y_host, double *u_host, int32_t *status_host,
                                   int32_t *n_steps_host);
+
+/* Host-buffer form of mpc_discretize_batch_ragged: K_sat is a host array (validated: 2 <= K_s <= K_max), out_host is
+ * [105][n_sats (K_max-1)] with NaN in the padding columns, status_host / n_nodes_host [n_sats][K_max-1] with 0 there. */
+int mpc_discretize_batch_ragged_host(mpc_ctx *ctx, const double *x, const double *u, const double *tf, const mpc_params *p,
+                                     int n_sats, int K_max, const int32_t *K_sat, int adaptive, int n_sub, double rtol,
+                                     double atol, double max_step, double *out_host, int32_t *status_host,
+                                     int32_t *n_nodes_host);
+
+/* Host-buffer form of mpc_propagate_batch_rk45_ragged: T_sat and table_len_sat are host arrays (validated:
+ * 2 <= T_s <= T_max, 2 <= table length <= table_len); y_host / u_host padding columns are NaN. */
+int mpc_propagate_batch_rk45_ragged_host(mpc_ctx *ctx, const double *y0, const double *tf, const mpc_params *p,
+                                         const mpc_controller *ctrl, int n_sats, int T_max, const int32_t *T_sat,
+                                         const int32_t *table_len_sat, double rtol, double atol, double max_step,
+                                         double *y_host, double *u_host, int32_t *status_host, int32_t *n_steps_host);
 
 /*
  * SCP inner step on host buffers, fused on the device (control.py:180-188 pattern): propagate the

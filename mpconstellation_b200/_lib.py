@@ -133,6 +133,10 @@ def lib():
     L.mpc_propagate_batch.argtypes = [_DP, _DP, pp, pc, i, i, i, _DP, _DP, _DP, vp]
     L.mpc_propagate_batch_rk45.argtypes = [_DP, _DP, pp, pc, i, i, d, d, d, _DP, _DP, _DP, _DP, vp]
     L.mpc_propagate_batch_rk45_host.argtypes = [vp, _DP, _DP, pp, pc, i, i, d, d, d, _DP, _DP, _DP, _DP]
+    L.mpc_discretize_batch_ragged.argtypes = [_DP, _DP, _DP, pp, i, i, _DP, _DP, i, i, d, d, d, _DP, i64, i64, _DP, _DP, vp]
+    L.mpc_discretize_batch_ragged_host.argtypes = [vp, _DP, _DP, _DP, pp, i, i, _DP, i, i, d, d, d, _DP, _DP, _DP]
+    L.mpc_propagate_batch_rk45_ragged.argtypes = [_DP, _DP, pp, pc, i, i, _DP, _DP, d, d, d, _DP, _DP, _DP, _DP, vp]
+    L.mpc_propagate_batch_rk45_ragged_host.argtypes = [vp, _DP, _DP, pp, pc, i, i, _DP, _DP, d, d, d, _DP, _DP, _DP, _DP]
     L.mpc_ctx_create.argtypes = [i, ctypes.POINTER(vp)]
     L.mpc_ctx_destroy.argtypes = [vp]
     L.mpc_host_alloc.argtypes = [ctypes.c_size_t]
@@ -174,6 +178,8 @@ EXPORTED_SYMBOLS = [
     "mpc_discretize_batch", "mpc_discretize_batch_multi", "mpc_discretize_batch_adaptive", "mpc_discretize_batch_ugrid", "mpc_propagate_batch",
     "mpc_propagate_batch_rk45", "mpc_propagate_batch_rk45_host", "mpc_discretize_batch_gather", "mpc_propagate_discretize_gather",
     "mpc_propagate_discretize_host_layout",
+    "mpc_discretize_batch_ragged", "mpc_discretize_batch_ragged_host", "mpc_propagate_batch_rk45_ragged",
+    "mpc_propagate_batch_rk45_ragged_host",
     "mpc_ctx_create", "mpc_ctx_destroy", "mpc_host_alloc", "mpc_host_free",
     "mpc_discretize_batch_host", "mpc_discretize_batch_adaptive_host", "mpc_discretize_batch_ugrid_host", "mpc_propagate_batch_host", "mpc_propagate_discretize_host", "mpc_propagate_discretize", "mpc_propagate_discretize_multi",
     "mpc_constraint_terms", "mpc_constraint_terms_host", "mpc_discretize_batch_push", "mpc_fill_const_rows",

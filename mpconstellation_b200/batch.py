@@ -53,26 +53,33 @@ class DiscretizedBatch:
     layout "satmajor": column = s (K-1) + k (per-satellite blocks); "kmajor": column = k N + s (what the streamed host
     pass propagate_discretize(layout="kmajor") writes).  sat(s) returns (A_k, B_kp, B_kn, Sigma_k, xi_k) with the shapes
     and order of Discretizer.discretize (linearize_discretize.py:390); they are views in either layout, no copy is made.
+    Ragged batches (K_sat [N]: satellite s on its own K_s nodes) keep the layout of K = max K_s: satellite s owns the
+    columns s (K-1) + k, k < K_s - 1, and sat(s) returns its K_s - 1 intervals; the padding columns hold NaN (status 0).
     """
 
-    def __init__(self, soa, status, n_sats, K, layout="satmajor"):
+    def __init__(self, soa, status, n_sats, K, layout="satmajor", K_sat=None):
         self.soa, self.status, self.n_sats, self.K, self.layout = soa, status, n_sats, K, layout
+        self.K_sat = None if K_sat is None else np.asarray(K_sat, dtype=np.int32)
+
+    def _n(self, s):
+        return (self.K if self.K_sat is None else int(self.K_sat[s])) - 1
 
     def _rows(self, r0, nrows, s):
         n = self.K - 1
         if self.layout == "kmajor":
             return self.soa[r0:r0 + nrows, s::self.n_sats]
-        return self.soa[r0:r0 + nrows, s * n:(s + 1) * n]
+        return self.soa[r0:r0 + nrows, s * n:s * n + self._n(s)]
 
     def sat(self, s):
-        n = self.K - 1
+        n = self._n(s)
         A = self._rows(_lib.ROW_A, 49, s).T.reshape(n, 7, 7)
         Bp = self._rows(_lib.ROW_BP, 21, s).T.reshape(n, 7, 3)
         Bn = self._rows(_lib.ROW_BN, 21, s).T.reshape(n, 7, 3)
         return A, Bp, Bn, self._rows(_lib.ROW_SIGMA, 7, s), self._rows(_lib.ROW_XI, 7, s)
 
     def stacked(self):
-        """(A[N,K-1,7,7], B_kp[N,K-1,7,3], B_kn[N,K-1,7,3], Sigma[N,7,K-1], xi[N,7,K-1]) as views."""
+        """(A[N,K-1,7,7], B_kp[N,K-1,7,3], B_kn[N,K-1,7,3], Sigma[N,7,K-1], xi[N,7,K-1]) as views (ragged: padded, NaN
+        past K_s - 1)."""
         N, n = self.n_sats, self.K - 1
         if self.layout == "kmajor":
             v = self.soa.reshape(_lib.MPC_OUT_ROWS, n, N).transpose(0, 2, 1)      # [105, N, n], strided
@@ -100,8 +107,18 @@ def raise_on_status(status):
         raise FloatingPointError(f"non-finite result at unit {tuple(int(i) for i in idx)}")
 
 
+def _counts(c, n, cmax, what):
+    """per-satellite node / sample counts as int32 [n], each 2 <= c <= cmax"""
+    c = np.ascontiguousarray(c, dtype=np.int32)
+    if c.shape != (n,):
+        raise ValueError(f"{what} must have shape [{n}], got {c.shape}")
+    if n and (c.min() < 2 or c.max() > cmax):
+        raise ValueError(f"every {what} must be >= 2 and <= {cmax}")
+    return c
+
+
 def discretize_batch(x, u, tf, const, include_J2=False, include_drag=False, n_sub=100, out=None, status=None,
-                     device=0, check=True, adaptive=None, disc_drag=None):
+                     device=0, check=True, adaptive=None, disc_drag=None, K=None):
     """Discretize every interval of every satellite in one launch sequence (host arrays).
 
     x [N,7,K], u [N,3,K], tf scalar or [N]; `out` may be a preallocated (ideally pinned) [105, N*(K-1)]
@@ -113,8 +130,14 @@ def discretize_batch(x, u, tf, const, include_J2=False, include_drag=False, n_su
 
     include_drag=True needs disc_drag=(CD, rho): const.CD and the (constant) value of rho_func the reference's drag
     branch reads (linearize_discretize.py:162-168); without them the call is rejected like the reference's.
+
+    K=None: every satellite on the K = x.shape[2] nodes.  K = int array [N]: a ragged batch -- satellite s on its own
+    K_s <= x.shape[2] nodes (the first K_s columns of x[s], u[s]), one launch for all; the result keeps the layout of
+    Kmax = x.shape[2] with NaN in the padding columns (DiscretizedBatch.sat(s) returns K_s - 1 intervals).  u must be on
+    the nodes of x, and the drag linearisation is not available for ragged batches.
     """
     ctx = _ctx(device)
+    counts, K = K, None
     x = _f64(x)
     if x.ndim != 3 or x.shape[1] != 7:
         raise ValueError(f"x must be [N,7,K], got {x.shape}")
@@ -133,8 +156,20 @@ def discretize_batch(x, u, tf, const, include_J2=False, include_drag=False, n_su
         status = np.zeros(n_int, dtype=np.int32)
     p = _lib.make_params(const, include_J2, include_drag, disc_drag=disc_drag)
     n_nodes = None
-    with _lock(device):
+    K_sat = None
+    if counts is not None:
+        K_sat = _counts(counts, N, K, "K")
         if Ku != K:
+            raise ValueError("a ragged batch needs u on the nodes of x ([N,3,Kmax])")
+    with _lock(device):
+        if K_sat is not None:
+            ad = adaptive or {}
+            n_nodes = np.zeros(n_int, dtype=np.int32) if adaptive is not None else None
+            _lib.check(_lib.lib().mpc_discretize_batch_ragged_host(
+                ctx, _lib.addr(x), _lib.addr(u), _lib.addr(tfv), ctypes.byref(p), N, K, _lib.addr(K_sat),
+                int(adaptive is not None), int(n_sub), float(ad.get("rtol", 1e-3)), float(ad.get("atol", 1e-6)),
+                float(ad.get("max_step", 1e-2)), _lib.addr(out), _lib.addr(status), _lib.addr(n_nodes)))
+        elif Ku != K:
             ad = adaptive or {}
             n_nodes = np.zeros(n_int, dtype=np.int32) if adaptive is not None else None
             _lib.check(_lib.lib().mpc_discretize_batch_ugrid_host(
@@ -151,7 +186,7 @@ def discretize_batch(x, u, tf, const, include_J2=False, include_drag=False, n_su
                 ctx, _lib.addr(x), _lib.addr(u), _lib.addr(tfv), ctypes.byref(p), N, K, float(adaptive.get("rtol", 1e-3)),
                 float(adaptive.get("atol", 1e-6)), float(adaptive.get("max_step", 1e-2)), _lib.addr(out), _lib.addr(status),
                 _lib.addr(n_nodes)))
-    res = DiscretizedBatch(out, status.reshape(N, K - 1), N, K)
+    res = DiscretizedBatch(out, status.reshape(N, K - 1), N, K, K_sat=K_sat)
     res.n_nodes = None if n_nodes is None else n_nodes.reshape(N, K - 1)
     if check:
         res.raise_on_error()
@@ -183,6 +218,11 @@ def _ctrl_struct(spec, n_sats, table_addr=None, end_tau_addr=None):
     return c, keep
 
 
+def _rectangular_law(spec):
+    if spec.kind == _lib.CTRL_SEQUENCE and spec.table_len is not None:
+        raise ValueError("per-satellite table lengths (ControllerSpec.table_len) are taken by propagate_batch only")
+
+
 def default_n_sub(T, max_step=0.001):
     """RK4 steps between samples so that the step in tau is <= max_step (simulator.py:186)."""
     if T < 2:
@@ -197,6 +237,11 @@ def propagate_batch(y0, tf, controller, const, include_drag=True, include_J2=Tru
     y0 [N,7] normalized states; returns (y [N,7,T], u [N,3,T] or None, t [T], status [N]).
     ref: simulator.py:164-189 (+ extract_uk, linearize_discretize.py:393-411).
 
+    T = int array [N]: satellite s sampled at linspace(0, 1, T_s) (the reference's int(base_res * tf_s) of every
+    satellite's own horizon), one launch for all; y / u are [N,7,Tmax] / [N,3,Tmax] and t is [N,Tmax], NaN past T_s.
+    The steps do not depend on the samples (n_steps as for a rectangular run).  Reference integrator only (n_sub=None),
+    as is a sequence law with per-satellite table lengths (ControllerSpec.table_len).
+
     n_sub=None (default): the reference's own integrator, replayed on the device -- scipy's RK45 with its step-size
     controller exactly as simulator.py:185-187 calls it (max_step=0.001, rtol 1e-3, atol 1e-6, dense-output samples);
     `rk45=dict(rtol=, atol=, max_step=)` overrides those numbers, `n_steps` (int32 [N]) receives the steps attempted.
@@ -207,8 +252,16 @@ def propagate_batch(y0, tf, controller, const, include_drag=True, include_J2=Tru
     if y0.ndim != 2 or y0.shape[1] != 7:
         raise ValueError(f"y0 must be [N,7], got {y0.shape}")
     N = y0.shape[0]
-    T = int(T)
     spec = spec_from(controller)
+    T_sat = tab_len = None
+    if spec.kind == _lib.CTRL_SEQUENCE and spec.table_len is not None:
+        tab_len = _counts(spec.table_len, N, np.shape(spec.table)[-1], "table_len")
+    if np.ndim(T) != 0:
+        T_sat = _counts(T, N, int(np.max(T)) if N else 2, "T")
+        T = int(T_sat.max()) if N else 2
+    T = int(T)
+    if (T_sat is not None or tab_len is not None) and n_sub not in (None, 0):
+        raise ValueError("per-satellite sample counts / table lengths need the reference integrator (n_sub=None)")
     tfv = _tf_vec(tf, N)
     if n_sub is None:
         n_sub = 0
@@ -217,7 +270,12 @@ def propagate_batch(y0, tf, controller, const, include_drag=True, include_J2=Tru
     y = y_out if y_out is not None else _lib.pinned_empty((N, 7, T))
     uo = (u_out if u_out is not None else _lib.pinned_empty((N, 3, T))) if want_u else None
     status = np.zeros(N, dtype=np.int32)
-    t = np.linspace(0, 1, T)
+    if T_sat is None:
+        t = np.linspace(0, 1, T)
+    else:
+        t = np.full((N, T), np.nan)
+        for s_, ts in enumerate(T_sat):
+            t[s_, :ts] = np.linspace(0, 1, ts)
     if N == 0 or T == 0:
         return y, uo, t, status
     p = _lib.make_params(const, include_J2, include_drag)
@@ -227,10 +285,17 @@ def propagate_batch(y0, tf, controller, const, include_drag=True, include_J2=Tru
         if n_steps is not None and (n_steps.shape != (N,) or n_steps.dtype != np.int32):
             raise ValueError("n_steps must be int32 [N]")
         with _lock(device):
-            _lib.check(_lib.lib().mpc_propagate_batch_rk45_host(
-                ctx, _lib.addr(y0), _lib.addr(tfv), ctypes.byref(p), ctypes.byref(c), N, T, float(o.get("rtol", 1e-3)),
-                float(o.get("atol", 1e-6)), float(o.get("max_step", 1e-3)), _lib.addr(y), _lib.addr(uo),
-                _lib.addr(status), _lib.addr(n_steps)))
+            if T_sat is not None or tab_len is not None:
+                counts = T_sat if T_sat is not None else np.full(N, T, dtype=np.int32)
+                _lib.check(_lib.lib().mpc_propagate_batch_rk45_ragged_host(
+                    ctx, _lib.addr(y0), _lib.addr(tfv), ctypes.byref(p), ctypes.byref(c), N, T, _lib.addr(counts),
+                    _lib.addr(tab_len), float(o.get("rtol", 1e-3)), float(o.get("atol", 1e-6)), float(o.get("max_step", 1e-3)), _lib.addr(y),
+                    _lib.addr(uo), _lib.addr(status), _lib.addr(n_steps)))
+            else:
+                _lib.check(_lib.lib().mpc_propagate_batch_rk45_host(
+                    ctx, _lib.addr(y0), _lib.addr(tfv), ctypes.byref(p), ctypes.byref(c), N, T, float(o.get("rtol", 1e-3)),
+                    float(o.get("atol", 1e-6)), float(o.get("max_step", 1e-3)), _lib.addr(y), _lib.addr(uo),
+                    _lib.addr(status), _lib.addr(n_steps)))
     else:
         with _lock(device):
             _lib.check(_lib.lib().mpc_propagate_batch_host(ctx, _lib.addr(y0), _lib.addr(tfv), ctypes.byref(p),
@@ -254,6 +319,7 @@ def propagate_discretize(y0, tf, controller, const, T, prop_drag=False, prop_J2=
     N = y0.shape[0]
     T = int(T)
     spec = spec_from(controller)
+    _rectangular_law(spec)
     tfv = _tf_vec(tf, N)
     n_int = N * (T - 1)
     if n_sub_prop is None:
@@ -339,6 +405,7 @@ def propagate_batch_device(y0, tf, controller, const, include_drag=True, include
         u_out = torch.empty((N, 3, T), dtype=torch.float64, device=y0.device)
     if status is None:
         status = torch.empty(N, dtype=torch.int32, device=y0.device)
+    _rectangular_law(spec)
     tab_dev = et_dev = None
     if spec.kind == _lib.CTRL_SEQUENCE:
         tab_dev = torch.as_tensor(spec.table, dtype=torch.float64).to(y0.device).contiguous()
@@ -377,6 +444,7 @@ def propagate_discretize_device(y0, tf, controller, const, T, prop_drag=False, p
     assert y0.is_cuda and y0.dtype == torch.float64 and y0.is_contiguous() and y0.shape == (N, 7) and tf.shape == (N,)
     n_int = N * (T - 1)
     spec = spec_from(controller)
+    _rectangular_law(spec)
     if n_sub_prop is None:
         n_sub_prop = 0                    # the reference's RK45, replayed (see propagate_batch)
     if y is None:

@@ -23,6 +23,8 @@ class ControllerSpec:
     thrust: tuple = (0.0, 0.0, 0.0)
     table: np.ndarray = field(default=None, repr=False)   # (3,Ku) or (N,3,Ku)
     end_tau: object = 1.0                                  # scalar, or [N] array (one end_tau per satellite)
+    table_len: object = None                               # None, or int [N]: satellite s uses the first table_len[s]
+                                                           # columns of its (N,3,Ku) table (per-satellite horizons)
 
     def host_u_func(self):
         """u(x, tau) on the host, same arithmetic as the device law (used by extract_uk on the host

@@ -97,6 +97,16 @@ __device__ __forceinline__ void ad_end_node_input(AdStage &o, const double *__re
     o.un = uu * o.iun;
 }
 
+// ragged batches: u of the satellite is [3][ld] (ld = Kmax), its grid has Ku = K_s nodes
+template <typename Stage>
+__device__ __forceinline__ void ad_end_node_input_ld(Stage &o, const double *__restrict__ u_in, int sat, int ld, int Ku, int node)
+{
+    ref_node_input_ld(u_in + (long long)sat * 3 * ld, ld, Ku, node, 1.0, o.ux, o.uy, o.uz);
+    const double uu = fma(o.ux, o.ux, fma(o.uy, o.uy, o.uz * o.uz));
+    o.iun = (uu > 4.930380657631324e-32) ? fast_rsqrt(uu) : 0.0;
+    o.un = uu * o.iun;
+}
+
 #define SM(e) sm[(e) * BLOCK]
 
 template <int BLOCK, bool DRAG>

@@ -90,21 +90,32 @@ __device__ __forceinline__ void df_store_stage(volatile double *sm, int s, const
     }
 }
 
-template <bool J2, int BLOCK, bool GENU, bool DRAG>
+// RAG: a ragged batch (discretize_default_ragged_kernel): K is the padded stride Kmax, first[] the prefix sums of K_s - 1
+// (ragged_locate); threads map to live intervals only, gid below is the interval's output column s (Kmax-1) + k.
+template <bool J2, int BLOCK, bool GENU, bool DRAG, bool RAG = false>
 __device__ __forceinline__ void
 discretize_default_body(const double *__restrict__ x_in, const double *__restrict__ u_in,
                         const double *__restrict__ tf_arr, const DiscParams &P, int n_sats, int K, int Ku, double rtol, double atol,
                         double max_step, const DstTab &dst, long long pitch, long long offset, int32_t *__restrict__ status,
-                        int32_t *__restrict__ n_nodes, double kf, const DragLin *L)
+                        int32_t *__restrict__ n_nodes, double kf, const DragLin *L, const long long *__restrict__ first = nullptr)
 {
     constexpr int kStage = DRAG ? 18 : 9;
     extern __shared__ double acc_smem[];
-    const long long n_int = (long long)n_sats * (K - 1);
-    const long long gid = (long long)blockIdx.x * BLOCK + threadIdx.x;
-    if (gid >= n_int) return;
+    long long gid;
+    int sat, k, Kg = K;           // Kg: nodes of this satellite's grid
+    if constexpr (RAG) {
+        const long long tid = (long long)blockIdx.x * BLOCK + threadIdx.x;
+        if (tid >= first[n_sats] - first[0]) return;
+        ragged_locate(first, n_sats, tid, sat, k, Kg);
+        gid = (long long)sat * (K - 1) + k;
+    } else {
+        const long long n_int = (long long)n_sats * (K - 1);
+        gid = (long long)blockIdx.x * BLOCK + threadIdx.x;
+        if (gid >= n_int) return;
+        sat = (int)(gid / (K - 1));
+        k = (int)(gid - (long long)sat * (K - 1));
+    }
     volatile double *sm = acc_smem + threadIdx.x;
-    const int sat = (int)(gid / (K - 1));
-    const int k = (int)(gid - (long long)sat * (K - 1));
     const double tf = tf_arr[sat];
     const double *xs = x_in + ((long long)sat * 7) * K + k;
     double x[7];
@@ -113,8 +124,8 @@ discretize_default_body(const double *__restrict__ x_in, const double *__restric
     UHold<GENU> hold;
     hold.init(u_in, sat, k, K, Ku);
     // tau = np.linspace(0, 1, K) (:356): start + i*step, last point exactly 1
-    const double step = 1.0 / (double)(K - 1);
-    const double t0 = (double)k * step, t1 = (k + 1 == K - 1) ? 1.0 : (double)(k + 1) * step;
+    const double step = 1.0 / (double)(Kg - 1);
+    const double t0 = (double)k * step, t1 = (k + 1 == Kg - 1) ? 1.0 : (double)(k + 1) * step;
     const double ilen = 1.0 / (t1 - t0);
     // this thread's column of the output buffer: Phi scratch blocks at rows kDfPhiA.. and kDfPhiB..
     double *const col = dst.p[0] + offset + gid;
@@ -127,7 +138,8 @@ discretize_default_body(const double *__restrict__ x_in, const double *__restric
     for (int q = 0; q < 8; ++q) row6[(long long)q * pitch] = 0.0;
     if (!GENU) {       // input of the far end node as the reference looks it up: computed once, parked in the buffer
         double e[3];
-        ref_node_input(u_in + (long long)sat * 3 * K, K, k + 1, 1.0, e[0], e[1], e[2]);
+        if (RAG) ref_node_input_ld(u_in + (long long)sat * 3 * K, K, Kg, k + 1, 1.0, e[0], e[1], e[2]);
+        else ref_node_input(u_in + (long long)sat * 3 * K, K, k + 1, 1.0, e[0], e[1], e[2]);
 #pragma unroll
         for (int q = 0; q < 3; ++q) col[(long long)(kDfEndU + q) * pitch] = e[q];
     }
@@ -220,7 +232,9 @@ discretize_default_body(const double *__restrict__ x_in, const double *__restric
 
     // ---- solve_ivp main loop.  One trip per quadrature node: try steps from node j until one is accepted (none when
     // t has reached the end), then add node j with its full trapezoid weight, then move on. ---------------------------
-    ad_end_node_input<GENU>(st0, u_in, sat, K, k);       // the node term of tau_k reads the reference's lookup of u there
+    // the node term of tau_k reads the reference's lookup of u there
+    if (RAG) ad_end_node_input_ld(st0, u_in, sat, K, Kg, k);
+    else ad_end_node_input<GENU>(st0, u_in, sat, K, k);
     double half_prev = 0.0;       // (t_j - t_{j-1}) / 2
 #pragma unroll 1
     for (;;) {
@@ -481,6 +495,19 @@ discretize_default_drag_kernel(const double *__restrict__ x_in, const double *__
 {
     discretize_default_body<J2, BLOCK, false, true>(x_in, u_in, tf_arr, P, n_sats, K, 0, rtol, atol, max_step, dst, pitch, offset,
                                                     status, n_nodes, kf, &L);
+}
+
+// ragged batch: satellite s on K_s = first[s+1] - first[s] + 1 nodes, x / u padded to K = Kmax columns, results, status and
+// node counts in columns offset + s (Kmax-1) + k (k < K_s - 1); the padding columns are never written
+template <bool J2, int BLOCK>
+__global__ void __launch_bounds__(BLOCK)
+discretize_default_ragged_kernel(const double *__restrict__ x_in, const double *__restrict__ u_in,
+                                 const double *__restrict__ tf_arr, DiscParams P, int n_sats, int K, double rtol, double atol,
+                                 double max_step, DstTab dst, long long pitch, long long offset, int32_t *__restrict__ status,
+                                 int32_t *__restrict__ n_nodes, const long long *__restrict__ first)
+{
+    discretize_default_body<J2, BLOCK, false, false, true>(x_in, u_in, tf_arr, P, n_sats, K, K, rtol, atol, max_step, dst, pitch,
+                                                           offset, status, n_nodes, 0.0, nullptr, first);
 }
 
 }  // namespace mpc

@@ -244,6 +244,49 @@ __device__ __noinline__ void ref_node_input(const double *__restrict__ us, int K
     uz = f * __dadd_rn(__dmul_rn(ln, us[2 * (long long)Ku + kq]), __dmul_rn(lp, us[2 * (long long)Ku + kq + 1]));
 }
 
+// ref_node_input for ragged batches: u of the satellite is [3][ld] (ld = Kmax, the padded stride), its grid has Ku = K_s
+// nodes.  Same arithmetic; a copy rather than a shared body so that the rectangular kernels' code stays as it was.
+__device__ __noinline__ void ref_node_input_ld(const double *__restrict__ us, int ld, int Ku, int i, double f, double &ux,
+                                               double &uy, double &uz)
+{
+    if (i >= Ku - 1) {
+        ux = f * us[Ku - 1];
+        uy = f * us[ld + Ku - 1];
+        uz = f * us[2 * (long long)ld + Ku - 1];
+        return;
+    }
+    const double km1 = (double)(Ku - 1);
+    const double dtau = 1.0 / km1;
+    const double tau = (double)i * dtau;
+    int kq = i - (fma((double)i, dtau, -tau) > 0.0 ? 1 : 0);
+    kq = min(max(kq, 0), Ku - 2);
+    const double tk = (double)kq / km1, tk1 = (double)(kq + 1) / km1;
+    const double iw = 1.0 / (tk1 - tk);
+    const double ln = (tk1 - tau) * iw, lp = (tau - tk) * iw;
+    ux = f * __dadd_rn(__dmul_rn(ln, us[kq]), __dmul_rn(lp, us[kq + 1]));
+    uy = f * __dadd_rn(__dmul_rn(ln, us[ld + kq]), __dmul_rn(lp, us[ld + kq + 1]));
+    uz = f * __dadd_rn(__dmul_rn(ln, us[2 * (long long)ld + kq]), __dmul_rn(lp, us[2 * (long long)ld + kq + 1]));
+}
+
+// Ragged batches (satellite s on K_s nodes, buffers padded to Kmax): first[0..n_sats] are the prefix sums of K_s - 1 (a
+// chunk of a batch passes first + s0, so the sums need not start at 0).  Live interval `tid` of the launch -> (s, k, K_s).
+// Threads map to live intervals only: the binary search costs ~log2(n_sats) dependent loads at thread start.
+__device__ __forceinline__ void ragged_locate(const long long *__restrict__ first, int n_sats, long long tid, int &s, int &k,
+                                              int &Ks)
+{
+    const long long g = first[0] + tid;
+    int lo = 0, hi = n_sats;               // first[lo] <= g < first[hi]
+    while (hi - lo > 1) {
+        const int mid = (lo + hi) >> 1;
+        if (first[mid] <= g) lo = mid;
+        else hi = mid;
+    }
+    s = lo;
+    const long long f0 = first[lo];
+    k = (int)(g - f0);
+    Ks = (int)(first[lo + 1] - f0) + 1;
+}
+
 // Input hold u(tau).  GENU = false: u is given on the K nodes of x, so inside one interval the reference's
 // first-order hold (linearize_discretize.py:294-315) is the straight line between u_k and u_{k+1}.
 // GENU = true: u has its own column count Ku (the reference accepts that: u_FOH takes its grid from u itself,
@@ -714,15 +757,18 @@ __device__ __forceinline__ void state_step5(const DiscParams &Ph, const UHold<fa
 #define ACC(e) acc[(e) * BLOCK]
 // EM = 1 / 2 / 3: n_sub is kEmSteps / kEmSteps2 / kEmSteps3 and node n carries the weight kEmW[n] / kEmW2[n] / kEmW3[n]
 // instead of the trapezoid's 1/2, 1, ..., 1, 1/2.  EM = 3 takes the fifth-order steps (state_step5, column_step5).
-template <bool J2, int BLOCK, int NDST, bool GENU, int EM = 0>
+// RAG: a ragged batch -- K is the padded stride Kmax, the interval is (rs, rk) on a grid of rK nodes, gid = rs (K-1) + rk.
+template <bool J2, int BLOCK, int NDST, bool GENU, int EM = 0, bool RAG = false>
 __device__ __forceinline__ void discretize_thread(const double *__restrict__ x, const double *__restrict__ u,
                                                   const double *__restrict__ tf_arr, const DiscParams &P, int K, int Ku,
                                                   int n_sub, const DstTab &dst, long long pitch, long long offset,
-                                                  int32_t *__restrict__ status, long long gid, volatile double *acc)
+                                                  int32_t *__restrict__ status, long long gid, volatile double *acc,
+                                                  int rs = 0, int rk = 0, int rK = 0)
 {
 
-    const int s = (int)(gid / (K - 1));
-    const int k = (int)(gid - (long long)s * (K - 1));
+    const int s = RAG ? rs : (int)(gid / (K - 1));
+    const int k = RAG ? rk : (int)(gid - (long long)s * (K - 1));
+    const int Kg = RAG ? rK : K;                // nodes of this satellite's grid
     const double tf = tf_arr[s];
     const double *xs = x + ((long long)s * 7) * K + k;
     double rx = xs[0], ry = xs[K], rz = xs[2 * (long long)K];
@@ -730,10 +776,10 @@ __device__ __forceinline__ void discretize_thread(const double *__restrict__ x, 
     double m = xs[6 * (long long)K];
     UHold<GENU> hold;
     hold.init(u, s, k, K, Ku);
-    const double tau0 = (double)k / (double)(K - 1), dtau_k = 1.0 / (double)(K - 1);  // interval [tau_k, tau_k+1]
+    const double tau0 = (double)k / (double)(Kg - 1), dtau_k = 1.0 / (double)(Kg - 1);  // interval [tau_k, tau_k+1]
 
     const double inv_n = 1.0 / (double)n_sub;
-    const double h = inv_n / (double)(K - 1);  // step in tau
+    const double h = inv_n / (double)(Kg - 1);  // step in tau
     const double hs = tf * h;                  // step of the unscaled system
     // ---- step-normalised variables ------------------------------------------------------------------
     // With D = diag(I3, hs I3, 1) the kernel carries D x (velocity times the step) and D Phi D^-1, and integrates in
@@ -770,7 +816,13 @@ __device__ __forceinline__ void discretize_thread(const double *__restrict__ x, 
     // thrust at the current node and its norm
     double ux, uy, uz;
     if (GENU) hold.at(0.0, tau0, ux, uy, uz);
-    else {       // the two end nodes: as the reference looks them up; the far one waits in shared memory
+    else if (RAG) {
+        ref_node_input_ld(u + (long long)s * 3 * K, K, Kg, k + 1, hs2, ux, uy, uz);
+        ACC(kEndU) = ux;
+        ACC(kEndU + 1) = uy;
+        ACC(kEndU + 2) = uz;
+        ref_node_input_ld(u + (long long)s * 3 * K, K, Kg, k, hs2, ux, uy, uz);
+    } else {     // the two end nodes: as the reference looks them up; the far one waits in shared memory
         ref_node_input(u + (long long)s * 3 * K, K, k + 1, hs2, ux, uy, uz);
         ACC(kEndU) = ux;
         ACC(kEndU + 1) = uy;
@@ -839,7 +891,7 @@ __device__ __forceinline__ void discretize_thread(const double *__restrict__ x, 
         const double sm = ((double)n + 0.5) * inv_n, se = (double)(n + 1) * inv_n;
         double umx, umy, umz, uex, uey, uez;
         hold.at(sm, fma(sm, dtau_k, tau0), umx, umy, umz);
-        hold.at(se, (n + 1 == n_sub && k + 2 == K) ? 1.0 : fma(se, dtau_k, tau0), uex, uey, uez);
+        hold.at(se, (n + 1 == n_sub && k + 2 == Kg) ? 1.0 : fma(se, dtau_k, tau0), uex, uey, uez);
         const double uum = fma(umx, umx, fma(umy, umy, umz * umz));
         const double uue = fma(uex, uex, fma(uey, uey, uez * uez));
         const double iunm = inv_norm_guarded(uum, eps2);

@@ -119,18 +119,22 @@ __device__ __forceinline__ void node_accumulate_column(volatile double *acc, int
     ACC(ix) = fma(n.w, X, c.AX);
 }
 
-template <bool J2, int BLOCK, int MAXREG, int NDST>
+// RAG: a ragged batch: K is the padded stride Kmax, first[] the prefix sums of K_s - 1 (ragged_locate), and the launch
+// covers the live intervals of every satellite (k0 = 0, kc = K - 1, no k-major layout, one destination).  Satellite s has
+// K_s = first[s+1] - first[s] + 1 nodes, its results go to columns offset + s (Kmax-1) + k (k < K_s - 1); the padding
+// columns are never written.
+template <bool J2, int BLOCK, int MAXREG, int NDST, bool RAG = false>
 __global__ void __launch_bounds__(BLOCK) __maxnreg__(MAXREG)
 discretize_pair_kernel(const double *__restrict__ x, const double *__restrict__ u, const double *__restrict__ tf_arr,
                        DiscParams P, int n_sats, int K, int n_sub, DstTab dst, long long pitch, long long offset,
-                       int32_t *__restrict__ status, int k0, int kc)
+                       int32_t *__restrict__ status, int k0, int kc, const long long *__restrict__ first = nullptr)
 {
     // The launch covers the intervals k in [k0, k0 + kc) of every satellite (the whole batch: k0 = 0, kc = K - 1).  A
     // window of k is what the overlapped propagate -> discretize pass launches as soon as the propagation has produced
     // the samples up to k0 + kc (mpc_propagate_discretize).  gid is the interval's global index s (K-1) + k either way.
     extern __shared__ double acc_smem[];
     const long long tid = (long long)blockIdx.x * BLOCK + threadIdx.x;
-    if (tid >= (long long)n_sats * kc) return;
+    if (RAG ? tid >= first[n_sats] - first[0] : tid >= (long long)n_sats * kc) return;
     if (dst.stagger_phases > 1 && (int)blockIdx.x < dst.first_wave_ctas) {
         const long long wait = dst.stagger_cycles * (long long)(blockIdx.x % dst.stagger_phases) / dst.stagger_phases;
         const long long t0 = clock64();
@@ -140,8 +144,10 @@ discretize_pair_kernel(const double *__restrict__ x, const double *__restrict__ 
 
     // thread -> (satellite, interval): consecutive threads walk the direction in which the output columns are adjacent
     // (k for the satellite-major layout, the satellite for the k-major one), so that every store of a warp is one line
-    int s, k;
-    if (dst.km_ntot) {
+    int s, k, Kg = K;             // Kg: nodes of this satellite's grid
+    if (RAG) {
+        ragged_locate(first, n_sats, tid, s, k, Kg);
+    } else if (dst.km_ntot) {
         const int kk = (int)(tid / n_sats);
         s = (int)(tid - (long long)kk * n_sats);
         k = k0 + kk;
@@ -160,7 +166,7 @@ discretize_pair_kernel(const double *__restrict__ x, const double *__restrict__ 
 
     const int n_pairs = n_sub >> 1;
     const double inv_n = 1.0 / (double)n_sub;
-    const double h = inv_n / (double)(K - 1);  // node spacing in tau
+    const double h = inv_n / (double)(Kg - 1); // node spacing in tau
     const double hn = tf * h;                  // node spacing of the unscaled system
     const double H = 2.0 * hn;                 // integrator step = two nodes
     {
@@ -185,21 +191,21 @@ discretize_pair_kernel(const double *__restrict__ x, const double *__restrict__ 
                     // of its size: 10 fifth-order steps and the 11-node rule kEmW3 (its remainder grows like the eighth
                     // power of that change: 2.5e-13 of the 101-node sums at 1/8, 4e-11 at 1/4)
                     if (dst.em >= 2 && d2 <= 0.015625 * fmax(a2, b2)) {
-                        discretize_thread<J2, BLOCK, NDST, false, 3>(x, u, tf_arr, P, K, K, kEmSteps3, dst, pitch, offset, status, gid, acc);
+                        discretize_thread<J2, BLOCK, NDST, false, 3, RAG>(x, u, tf_arr, P, K, K, kEmSteps3, dst, pitch, offset, status, gid, acc, s, k, Kg);
                         return;
                     }
-                    discretize_thread<J2, BLOCK, NDST, false, 1>(x, u, tf_arr, P, K, K, kEmSteps, dst, pitch, offset, status, gid, acc);
+                    discretize_thread<J2, BLOCK, NDST, false, 1, RAG>(x, u, tf_arr, P, K, K, kEmSteps, dst, pitch, offset, status, gid, acc, s, k, Kg);
                     return;
                 }
                 // longer intervals (omega 2h <= 4.4e-3 rad: 0.035-orbit intervals): 50 steps and the 51-node rule kEmW2
                 if (w2H2 <= 1.94e-5) {
-                    discretize_thread<J2, BLOCK, NDST, false, 2>(x, u, tf_arr, P, K, K, kEmSteps2, dst, pitch, offset, status, gid, acc);
+                    discretize_thread<J2, BLOCK, NDST, false, 2, RAG>(x, u, tf_arr, P, K, K, kEmSteps2, dst, pitch, offset, status, gid, acc, s, k, Kg);
                     return;
                 }
             }
         }
         if ((n_sub & 1) || !(w2H2 <= 1.0e-5)) {
-            discretize_thread<J2, BLOCK, NDST, false>(x, u, tf_arr, P, K, K, n_sub, dst, pitch, offset, status, gid, acc);
+            discretize_thread<J2, BLOCK, NDST, false, 0, RAG>(x, u, tf_arr, P, K, K, n_sub, dst, pitch, offset, status, gid, acc, s, k, Kg);
             return;
         }
     }
@@ -230,11 +236,13 @@ discretize_pair_kernel(const double *__restrict__ x, const double *__restrict__ 
     int bad = 0;
     double ux, uy, uz;
     // the two end nodes: as the reference looks them up (ref_node_input); the far one waits in shared memory
-    ref_node_input(u + (long long)s * 3 * K, K, k + 1, H2, ux, uy, uz);
+    if (RAG) ref_node_input_ld(u + (long long)s * 3 * K, K, Kg, k + 1, H2, ux, uy, uz);
+    else ref_node_input(u + (long long)s * 3 * K, K, k + 1, H2, ux, uy, uz);
     ACC(kEndU) = ux;
     ACC(kEndU + 1) = uy;
     ACC(kEndU + 2) = uz;
-    ref_node_input(u + (long long)s * 3 * K, K, k, H2, ux, uy, uz);
+    if (RAG) ref_node_input_ld(u + (long long)s * 3 * K, K, Kg, k, H2, ux, uy, uz);
+    else ref_node_input(u + (long long)s * 3 * K, K, k, H2, ux, uy, uz);
     double uu = fma(ux, ux, fma(uy, uy, uz * uz));
     double iun = inv_norm_guarded(uu, eps2);
     double un = uu * iun;

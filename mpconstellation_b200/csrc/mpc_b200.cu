@@ -10,6 +10,7 @@
 #include <cstdarg>
 #include <cstdio>
 #include <cstring>
+#include <limits>
 #include <vector>
 
 #include <math_constants.h>
@@ -141,7 +142,7 @@ int launch_pair_cfg(const double *x, const double *u, const double *tf, const mp
     const unsigned grid = (unsigned)((n_int + BLOCK - 1) / BLOCK);
     mpc::DstTab tab = dst;
     tab.em = em_level();
-    kern<<<grid, BLOCK, smem, st>>>(x, u, tf, P, n_sats, K, n_sub, tab, pitch, offset, status, k0, kc);
+    kern<<<grid, BLOCK, smem, st>>>(x, u, tf, P, n_sats, K, n_sub, tab, pitch, offset, status, k0, kc, nullptr);
     g_launches.fetch_add(1, std::memory_order_relaxed);
     CUDA_TRY(cudaGetLastError());
     return MPC_SUCCESS;
@@ -498,6 +499,92 @@ int disc_device(const double *x, const double *u, const double *tf, const mpc_pa
                          : launch_disc<false>(x, u, tf, P, n_sats, K, n_sub, tab, n_dst, pitch, offset, status, st);
 }
 
+// ---- ragged batches: satellite s on K_s nodes, buffers padded to Kmax (mpc_discretize_batch_ragged) ----------------------
+int check_counts(const int32_t *cnt, int n, int cmax, const char *what)
+{
+    if (!cnt) return fail(MPC_E_INVALID, "null %s", what);
+    for (int s = 0; s < n; ++s)
+        if (cnt[s] < 2 || cnt[s] > cmax)
+            return fail(MPC_E_INVALID, "%s[%d] = %d: every count must be >= 2 and <= %d", what, s, (int)cnt[s], cmax);
+    return MPC_SUCCESS;
+}
+
+// first[s] = sum_{r < s} (K_r - 1): the kernels' map from a live interval to (s, k)
+std::vector<long long> ragged_first(const int32_t *K_sat, int n)
+{
+    std::vector<long long> f((size_t)n + 1, 0);
+    for (int s = 0; s < n; ++s) f[s + 1] = f[s] + (K_sat[s] - 1);
+    return f;
+}
+
+// One launch for the batch; the block size follows from the LIVE interval count, as launch_adaptive_k / launch_disc_n
+// choose it from n_sats (K-1) for a rectangular batch.  (The thread-group kernel of small rectangular batches has no
+// ragged form: small ragged batches take the pair kernel in one-warp CTAs.)
+template <bool J2, int BLOCK>
+int launch_ragged_default(const double *x, const double *u, const double *tf, const mpc::DiscParams &P, int n_sats, int K,
+                          long long n_live, const long long *first, const AdaptiveOpts &o, const mpc::DstTab &dst,
+                          long long pitch, long long offset, int32_t *status, cudaStream_t st)
+{
+    static thread_local int configured_dev = -1;
+    auto kern = mpc::discretize_default_ragged_kernel<J2, BLOCK>;
+    const size_t smem = (size_t)mpc::kDfSlots * BLOCK * sizeof(double);
+    int rc = configure_smem(kern, smem, configured_dev);
+    if (rc) return rc;
+    const unsigned grid = (unsigned)((n_live + BLOCK - 1) / BLOCK);
+    kern<<<grid, BLOCK, smem, st>>>(x, u, tf, P, n_sats, K, o.rtol, o.atol, o.max_step, dst, pitch, offset, status, o.n_nodes, first);
+    g_launches.fetch_add(1, std::memory_order_relaxed);
+    CUDA_TRY(cudaGetLastError());
+    return MPC_SUCCESS;
+}
+
+template <bool J2, int BLOCK>
+int launch_ragged_pair(const double *x, const double *u, const double *tf, const mpc::DiscParams &P, int n_sats, int K,
+                       long long n_live, const long long *first, int n_sub, const mpc::DstTab &dst, long long pitch,
+                       long long offset, int32_t *status, cudaStream_t st)
+{
+    static thread_local int configured_dev = -1;
+    auto kern = mpc::discretize_pair_kernel<J2, BLOCK, 255, 1, true>;
+    const size_t smem = (size_t)mpc::kDiscSlots * BLOCK * sizeof(double);
+    int rc = configure_smem(kern, smem, configured_dev);
+    if (rc) return rc;
+    const unsigned grid = (unsigned)((n_live + BLOCK - 1) / BLOCK);
+    mpc::DstTab tab = dst;
+    tab.em = em_level();
+    kern<<<grid, BLOCK, smem, st>>>(x, u, tf, P, n_sats, K, n_sub, tab, pitch, offset, status, 0, K - 1, first);
+    g_launches.fetch_add(1, std::memory_order_relaxed);
+    CUDA_TRY(cudaGetLastError());
+    return MPC_SUCCESS;
+}
+
+template <bool J2>
+int launch_ragged(const double *x, const double *u, const double *tf, const mpc::DiscParams &P, int n_sats, int K,
+                  long long n_live, const long long *first, const AdaptiveOpts *ad, int n_sub, const mpc::DstTab &dst,
+                  long long pitch, long long offset, int32_t *status, cudaStream_t st)
+{
+    if (ad) {
+        int block = g_default_block.load(std::memory_order_relaxed);
+        if (n_live < 148LL * 256) block = 32;
+        if (block == 256) return launch_ragged_default<J2, 256>(x, u, tf, P, n_sats, K, n_live, first, *ad, dst, pitch, offset, status, st);
+        if (block == 128) return launch_ragged_default<J2, 128>(x, u, tf, P, n_sats, K, n_live, first, *ad, dst, pitch, offset, status, st);
+        return launch_ragged_default<J2, 32>(x, u, tf, P, n_sats, K, n_live, first, *ad, dst, pitch, offset, status, st);
+    }
+    if (n_live > 148LL * 32 && n_live <= 148LL * 128)
+        return launch_ragged_pair<J2, kDiscBlock>(x, u, tf, P, n_sats, K, n_live, first, n_sub, dst, pitch, offset, status, st);
+    if (n_live < 148LL * 9 * 32 * 2)
+        return launch_ragged_pair<J2, 32>(x, u, tf, P, n_sats, K, n_live, first, n_sub, dst, pitch, offset, status, st);
+    return launch_ragged_pair<J2, kDiscBlock>(x, u, tf, P, n_sats, K, n_live, first, n_sub, dst, pitch, offset, status, st);
+}
+
+int check_ragged_disc(const double *x, const double *u, const double *tf, const mpc_params *p, int n_sats, int K_max,
+                      const int32_t *K_sat, int adaptive, int n_sub, double rtol, double atol, double max_step)
+{
+    int rc = check_disc_args(x, u, tf, p, n_sats, K_max, adaptive ? 1 : n_sub);
+    if (rc) return rc;
+    if (p->include_drag) return fail(MPC_E_UNSUPPORTED, "the drag linearisation is not implemented for ragged batches");
+    if (adaptive && (rc = check_adaptive(rtol, atol, max_step))) return rc;
+    return check_counts(K_sat, n_sats, K_max, "K_sat");
+}
+
 int check_ctrl(const mpc_controller *c)
 {
     if (!c) return fail(MPC_E_INVALID, "null controller");
@@ -559,14 +646,33 @@ void launch_rk45(bool overlap, bool spec, unsigned n_warps, cudaStream_t st, con
     }
 }
 
+// ragged batch (per-satellite sample counts and / or table lengths): one-warp CTAs, never beside the discretization
+template <int KIND, bool DRAG, bool J2>
+void launch_rk45_ragged(bool spec, unsigned n_warps, cudaStream_t st, const double *y0, const double *tf, const mpc::PropParams &PP,
+                        const mpc::CtrlParams &C, const mpc::Rk45Opts &O, int n_sats, int T, int lpw, double *y, double *u_out,
+                        int32_t *status, int32_t *n_steps, const int32_t *T_sat, const int32_t *ku)
+{
+    if (spec)
+        mpc::propagate_rk45_kernel<kPropBlock, KIND, DRAG, J2, true, true><<<n_warps, kPropBlock, 0, st>>>(
+            y0, tf, PP, C, O, n_sats, T, lpw, y, u_out, status, n_steps, nullptr, 0, T_sat, ku);
+    else
+        mpc::propagate_rk45_kernel<kPropBlock, KIND, DRAG, J2, false, true><<<n_warps, kPropBlock, 0, st>>>(
+            y0, tf, PP, C, O, n_sats, T, lpw, y, u_out, status, n_steps, nullptr, 0, T_sat, ku);
+}
+
 // progress / seg_len: see propagate_kernel (the overlapped pass); then the CTAs are 4 warps instead of 1, so that the
 // propagation occupies 32 SMs instead of 128 while the discretization runs beside it.  *progress_target receives the
 // value progress[b] reaches when window b may start (warps for the RK4 kernel, satellites for the RK45 one).
 int prop_device(const double *y0, const double *tf, const mpc_params *p, const mpc_controller *c,
                 const double *table_dev, const double *end_tau_dev, int n_sats, int T, const PropMode &mode, double *y, double *u_out, int32_t *status,
-                cudaStream_t st, unsigned int *progress = nullptr, int seg_len = 0, unsigned int *progress_target = nullptr)
+                cudaStream_t st, unsigned int *progress = nullptr, int seg_len = 0, unsigned int *progress_target = nullptr,
+                const int32_t *T_sat_dev = nullptr, const int32_t *ku_dev = nullptr)
 {
     if (!y0 || !tf || !p || !y) return fail(MPC_E_INVALID, "null pointer argument");
+    // per-satellite counts (device arrays here): the RK45 propagator on its own only
+    const bool ragged = T_sat_dev || ku_dev;
+    if (ragged && (!mode.rk45() || progress))
+        return fail(MPC_E_UNSUPPORTED, "per-satellite sample counts / table lengths need the RK45 propagator (n_sub = 0) outside the fused pass");
     const int n_sub = mode.n_sub;
     if (n_sats < 0 || T < 0 || n_sub < 0) return fail(MPC_E_INVALID, "need n_sats >= 0, T >= 0, n_sub >= 0");
     if (mode.rk45() && (!(mode.rk.rtol > 0.0) || !(mode.rk.atol > 0.0) || !(mode.rk.max_step > 0.0)))
@@ -585,6 +691,7 @@ int prop_device(const double *y0, const double *tf, const mpc_params *p, const m
     C.end_tau = c->end_tau;
     C.table = (c->kind == MPC_CTRL_SEQUENCE) ? table_dev : nullptr;
     C.end_tau_arr = (c->kind == MPC_CTRL_SEQUENCE) ? end_tau_dev : nullptr;
+    if (c->kind != MPC_CTRL_SEQUENCE) ku_dev = nullptr;
     const unsigned grid = (unsigned)((n_sats + kPropBlock - 1) / kPropBlock);
     const unsigned grid_ov = (unsigned)((n_sats + kPropBlockOverlap - 1) / kPropBlockOverlap);
     const mpc::PropParams PP = prop_params(p);
@@ -599,7 +706,10 @@ int prop_device(const double *y0, const double *tf, const mpc_params *p, const m
     // one straight-line kernel per (controller law, drag, J2)
 #define MPC_PROP(KIND, DRAG, J2)                                                                                          \
     do {                                                                                                                  \
-        if (mode.rk45())                                                                                                  \
+        if (ragged)                                                                                                       \
+            launch_rk45_ragged<KIND, DRAG, J2>(spec, n_warps, st, y0, tf, PP, C, mode.rk, n_sats, T, lpw, y, u_out, status,  \
+                                               mode.n_steps, T_sat_dev, ku_dev);                                           \
+        else if (mode.rk45())                                                                                             \
             launch_rk45<KIND, DRAG, J2>(progress != nullptr, spec, n_warps, st, y0, tf, PP, C, mode.rk, n_sats, T, lpw, y, \
                                         u_out, status, mode.n_steps, progress, seg_len);                                  \
         else if (progress)                                                                                                \
@@ -651,6 +761,9 @@ struct mpc_ctx {
     double *d_x = nullptr, *d_u = nullptr, *d_tf = nullptr, *d_out = nullptr, *d_y0 = nullptr, *d_tab = nullptr;
     int32_t *d_status = nullptr, *d_status2 = nullptr, *d_nodes = nullptr;
     double *d_endtau = nullptr;
+    long long *d_first = nullptr;            // ragged batches: prefix sums of K_s - 1
+    int32_t *d_cnt = nullptr;                // ragged batches: T_sat and table_len_sat
+    size_t cap_first = 0, cap_cnt = 0;
     cudaStream_t s_pushk = nullptr;          // high-priority stream of the copy kernels (push gather, SM-driven variant)
     cudaStream_t s_aux[3] = {};              // compute streams the chunk kernels of the push gather rotate over
     cudaStream_t s_push[MPC_MAX_DST] = {};   // one stream per peer for the copy-engine gather (mpc_discretize_batch_push)
@@ -887,6 +1000,30 @@ int mpc_discretize_batch_ugrid(const double *x, const double *u, int u_cols, con
     return mpc_discretize_batch(x, u, tf, p, n_sats, K, n_sub, out, out_pitch, out_offset, status, stream);
 }
 
+int mpc_discretize_batch_ragged(const double *x, const double *u, const double *tf, const mpc_params *p, int n_sats,
+                                int K_max, const int32_t *K_sat, int64_t *first, int adaptive, int n_sub, double rtol,
+                                double atol, double max_step, double *out, int64_t out_pitch, int64_t out_offset,
+                                int32_t *status, int32_t *n_nodes, void *stream)
+{
+    int rc = check_ragged_disc(x, u, tf, p, n_sats, K_max, K_sat, adaptive, n_sub, rtol, atol, max_step);
+    if (rc) return rc;
+    if (!out || !first) return fail(MPC_E_INVALID, "null output / first");
+    if (out_pitch < out_offset + (long long)n_sats * (K_max - 1) || out_offset < 0)
+        return fail(MPC_E_INVALID, "out_pitch/out_offset do not hold the batch");
+    if (n_sats == 0) return MPC_SUCCESS;
+    cudaStream_t st = (cudaStream_t)stream;
+    const std::vector<long long> f = ragged_first(K_sat, n_sats);
+    // (pageable source: cudaMemcpyAsync stages it before returning, the vector may go)
+    CUDA_TRY(cudaMemcpyAsync(first, f.data(), f.size() * sizeof(long long), cudaMemcpyHostToDevice, st));
+    mpc::DstTab tab{};
+    tab.p[0] = out;
+    const AdaptiveOpts o{rtol, atol, max_step, n_nodes};
+    const mpc::DiscParams P = disc_params(p);
+    const long long *fd = (const long long *)first;
+    return p->include_j2 ? launch_ragged<true>(x, u, tf, P, n_sats, K_max, f[n_sats], fd, adaptive ? &o : nullptr, n_sub, tab, out_pitch, out_offset, status, st)
+                         : launch_ragged<false>(x, u, tf, P, n_sats, K_max, f[n_sats], fd, adaptive ? &o : nullptr, n_sub, tab, out_pitch, out_offset, status, st);
+}
+
 int mpc_propagate_batch(const double *y0, const double *tf, const mpc_params *p, const mpc_controller *ctrl,
                         int n_sats, int T, int n_sub, double *y, double *u_out, int32_t *status, void *stream)
 {
@@ -904,6 +1041,20 @@ int mpc_propagate_batch_rk45(const double *y0, const double *tf, const mpc_param
     m.n_steps = n_steps;
     return prop_device(y0, tf, p, ctrl, ctrl ? ctrl->table : nullptr, ctrl ? ctrl->end_tau_per_sat : nullptr, n_sats, T, m,
                        y, u_out, status, (cudaStream_t)stream);
+}
+
+int mpc_propagate_batch_rk45_ragged(const double *y0, const double *tf, const mpc_params *p, const mpc_controller *ctrl,
+                                    int n_sats, int T_max, const int32_t *T_sat, const int32_t *table_len_sat, double rtol,
+                                    double atol, double max_step, double *y, double *u_out, int32_t *status,
+                                    int32_t *n_steps, void *stream)
+{
+    if (!T_sat) return fail(MPC_E_INVALID, "null T_sat");
+    if (T_max < 2) return fail(MPC_E_INVALID, "need T_max >= 2 (got %d)", T_max);
+    PropMode m;
+    m.rk = mpc::Rk45Opts{rtol, atol, max_step};
+    m.n_steps = n_steps;
+    return prop_device(y0, tf, p, ctrl, ctrl ? ctrl->table : nullptr, ctrl ? ctrl->end_tau_per_sat : nullptr, n_sats, T_max, m,
+                       y, u_out, status, (cudaStream_t)stream, nullptr, 0, nullptr, T_sat, table_len_sat);
 }
 
 int mpc_ctx_create(int device, mpc_ctx **out)
@@ -952,6 +1103,8 @@ int mpc_ctx_destroy(mpc_ctx *c)
     cudaFree(c->d_status2);
     cudaFree(c->d_nodes);
     cudaFree(c->d_endtau);
+    cudaFree(c->d_first);
+    cudaFree(c->d_cnt);
     if (c->h_stage) cudaFreeHost(c->h_stage);
     delete c;
     return MPC_SUCCESS;
@@ -974,12 +1127,15 @@ void mpc_host_free(void *p)
 }
 
 // shared body of the two host-buffer discretization entry points (ad == nullptr: fixed-step kernel)
+// K_sat != nullptr: a ragged batch (K = Kmax, mpc_discretize_batch_ragged_host)
 static int disc_host(mpc_ctx *ctx, const double *x, const double *u, const double *tf, const mpc_params *p, int n_sats,
                      int K, int n_sub, const AdaptiveOpts *ad, double *out_host, int32_t *status_host,
-                     int32_t *n_nodes_host)
+                     int32_t *n_nodes_host, const int32_t *K_sat = nullptr)
 {
     if (!ctx || !out_host) return fail(MPC_E_INVALID, "null ctx/out");
-    int rc = check_disc_args(x, u, tf, p, n_sats, K, n_sub);
+    int rc = K_sat ? check_ragged_disc(x, u, tf, p, n_sats, K, K_sat, ad != nullptr, n_sub, ad ? ad->rtol : 0.0, ad ? ad->atol : 0.0,
+                                       ad ? ad->max_step : 0.0)
+                   : check_disc_args(x, u, tf, p, n_sats, K, n_sub);
     if (rc) return rc;
     if (ad && (rc = check_adaptive(ad->rtol, ad->atol, ad->max_step))) return rc;
     const long long n_int = (long long)n_sats * (K - 1);
@@ -997,6 +1153,12 @@ static int disc_host(mpc_ctx *ctx, const double *x, const double *u, const doubl
     if ((rc = ensure_events(ctx, (size_t)n_chunks))) return rc;
     const mpc::DiscParams P = disc_params(p);
     CUDA_TRY(cudaMemcpyAsync(ctx->d_tf, tf, (size_t)n_sats * sizeof(double), cudaMemcpyHostToDevice, ctx->s_compute));
+    std::vector<long long> first;
+    if (K_sat) {
+        first = ragged_first(K_sat, n_sats);
+        if ((rc = ensure(ctx->d_first, ctx->cap_first, first.size()))) return rc;
+        CUDA_TRY(cudaMemcpyAsync(ctx->d_first, first.data(), first.size() * sizeof(long long), cudaMemcpyHostToDevice, ctx->s_compute));
+    }
     for (int c = 0; c < n_chunks; ++c) {
         const int s0 = c * cs, ns = std::min(cs, n_sats - s0);
         const double *dx = ctx->d_x + (size_t)s0 * 7 * K, *du = ctx->d_u + (size_t)s0 * 3 * Ku;
@@ -1007,7 +1169,20 @@ static int disc_host(mpc_ctx *ctx, const double *x, const double *u, const doubl
         mpc::DstTab tab{};
         tab.p[0] = ctx->d_out;
         const long long off = (long long)s0 * (K - 1);
-        if (ad) {
+        if (K_sat) {
+            // the kernel leaves the padding columns alone: they go back as NaN (all-ones bytes) / status 0 / 0 nodes
+            const long long nc = (long long)ns * (K - 1);
+            CUDA_TRY(cudaMemset2DAsync(ctx->d_out + off, (size_t)n_int * sizeof(double), 0xFF, (size_t)nc * sizeof(double),
+                                       MPC_OUT_ROWS, ctx->s_compute));
+            CUDA_TRY(cudaMemsetAsync(ctx->d_status + off, 0, (size_t)nc * sizeof(int32_t), ctx->s_compute));
+            if (ad && n_nodes_host) CUDA_TRY(cudaMemsetAsync(ctx->d_nodes + off, 0, (size_t)nc * sizeof(int32_t), ctx->s_compute));
+            AdaptiveOpts o = ad ? *ad : AdaptiveOpts{};
+            o.n_nodes = (ad && n_nodes_host) ? ctx->d_nodes + off : nullptr;
+            rc = p->include_j2 ? launch_ragged<true>(dx, du, ctx->d_tf + s0, P, ns, K, first[s0 + ns] - first[s0], ctx->d_first + s0,
+                                                     ad ? &o : nullptr, n_sub, tab, n_int, off, ctx->d_status + off, ctx->s_compute)
+                               : launch_ragged<false>(dx, du, ctx->d_tf + s0, P, ns, K, first[s0 + ns] - first[s0], ctx->d_first + s0,
+                                                      ad ? &o : nullptr, n_sub, tab, n_int, off, ctx->d_status + off, ctx->s_compute);
+        } else if (ad) {
             AdaptiveOpts o = *ad;
             with_drag(o, p);
             o.n_nodes = n_nodes_host ? ctx->d_nodes + off : nullptr;
@@ -1024,6 +1199,12 @@ static int disc_host(mpc_ctx *ctx, const double *x, const double *u, const doubl
     // The host writes the structural constants while the GPU / DMA engine work.  The int32 words go through
     // pinned staging: a copy into a pageable caller buffer would block this thread until the whole pipeline drains.
     fill_const_rows(out_host, n_int);
+    if (K_sat) {   // ... but not in the padding columns of a ragged batch
+        const double qnan = std::numeric_limits<double>::quiet_NaN();
+        for (int r = kConstRow0; r < kConstRow1; ++r)
+            for (int sv = 0; sv < n_sats; ++sv)
+                for (long long k = K_sat[sv] - 1; k < K - 1; ++k) out_host[(size_t)r * n_int + (size_t)sv * (K - 1) + k] = qnan;
+    }
     const bool want_nodes = ad && n_nodes_host;
     if ((rc = ensure_stage(ctx, (size_t)n_int * 2))) return rc;
     int32_t *st_dst = status_host ? (is_pinned(status_host) ? status_host : ctx->h_stage) : nullptr;
@@ -1044,6 +1225,17 @@ int mpc_discretize_batch_host(mpc_ctx *ctx, const double *x, const double *u, co
                               int32_t *status_host)
 {
     return disc_host(ctx, x, u, tf, p, n_sats, K, n_sub, nullptr, out_host, status_host, nullptr);
+}
+
+int mpc_discretize_batch_ragged_host(mpc_ctx *ctx, const double *x, const double *u, const double *tf, const mpc_params *p,
+                                     int n_sats, int K_max, const int32_t *K_sat, int adaptive, int n_sub, double rtol,
+                                     double atol, double max_step, double *out_host, int32_t *status_host,
+                                     int32_t *n_nodes_host)
+{
+    if (!K_sat) return fail(MPC_E_INVALID, "null K_sat");
+    const AdaptiveOpts o{rtol, atol, max_step, nullptr};
+    return disc_host(ctx, x, u, tf, p, n_sats, K_max, adaptive ? 1 : n_sub, adaptive ? &o : nullptr, out_host, status_host,
+                     adaptive ? n_nodes_host : nullptr, K_sat);
 }
 
 int mpc_discretize_batch_adaptive_host(mpc_ctx *ctx, const double *x, const double *u, const double *tf,
@@ -1081,14 +1273,19 @@ static int upload_table(mpc_ctx *ctx, const mpc_controller *ctrl, int n_sats, cu
     return MPC_SUCCESS;
 }
 
+// T_sat != nullptr: per-satellite sample counts (T = Tmax) and table lengths (ku, may be NULL), host arrays
+// (mpc_propagate_batch_rk45_ragged_host)
 static int prop_host(mpc_ctx *ctx, const double *y0, const double *tf, const mpc_params *p, const mpc_controller *ctrl,
                      int n_sats, int T, PropMode mode, double *y_host, double *u_host, int32_t *status_host,
-                     int32_t *n_steps_host)
+                     int32_t *n_steps_host, const int32_t *T_sat = nullptr, const int32_t *ku_in = nullptr)
 {
     if (!ctx || !y0 || !tf || !p || !y_host) return fail(MPC_E_INVALID, "null pointer argument");
     if (n_sats < 0 || T < 0 || mode.n_sub < 0) return fail(MPC_E_INVALID, "need n_sats >= 0, T >= 0, n_sub >= 0");
     int rc = check_ctrl(ctrl);
     if (rc) return rc;
+    const int32_t *ku = (ctrl->kind == MPC_CTRL_SEQUENCE) ? ku_in : nullptr;
+    if (T_sat && (rc = check_counts(T_sat, n_sats, T, "T_sat"))) return rc;
+    if (ku && (rc = check_counts(ku, n_sats, ctrl->table_len, "table_len_sat"))) return rc;
     if (n_sats == 0 || T == 0) return MPC_SUCCESS;
     CUDA_TRY(cudaSetDevice(ctx->device));
     if ((rc = ensure(ctx->d_y0, ctx->cap_y0, (size_t)n_sats * 7))) return rc;
@@ -1104,7 +1301,18 @@ static int prop_host(mpc_ctx *ctx, const double *y0, const double *tf, const mpc
         if ((rc = ensure(ctx->d_nodes, ctx->cap_nodes, (size_t)n_sats))) return rc;
         mode.n_steps = ctx->d_nodes;
     }
-    if ((rc = prop_device(ctx->d_y0, ctx->d_tf, p, ctrl, ctx->d_tab, ctrl->end_tau_per_sat ? ctx->d_endtau : nullptr, n_sats, T, mode, ctx->d_x, ctx->d_u, ctx->d_status2, st)))
+    if (T_sat || ku) {
+        if ((rc = ensure(ctx->d_cnt, ctx->cap_cnt, (size_t)n_sats * 2))) return rc;
+        if (T_sat) CUDA_TRY(cudaMemcpyAsync(ctx->d_cnt, T_sat, (size_t)n_sats * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+        if (ku) CUDA_TRY(cudaMemcpyAsync(ctx->d_cnt + n_sats, ku, (size_t)n_sats * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    }
+    if (T_sat) {   // the kernel leaves the padding columns alone: they go back as NaN (all-ones bytes)
+        CUDA_TRY(cudaMemsetAsync(ctx->d_x, 0xFF, (size_t)n_sats * 7 * T * sizeof(double), st));
+        if (u_host) CUDA_TRY(cudaMemsetAsync(ctx->d_u, 0xFF, (size_t)n_sats * 3 * T * sizeof(double), st));
+    }
+    if ((rc = prop_device(ctx->d_y0, ctx->d_tf, p, ctrl, ctx->d_tab, ctrl->end_tau_per_sat ? ctx->d_endtau : nullptr, n_sats, T, mode,
+                          ctx->d_x, ctx->d_u, ctx->d_status2, st, nullptr, 0, nullptr, T_sat ? ctx->d_cnt : nullptr,
+                          ku ? ctx->d_cnt + n_sats : nullptr)))
         return rc;
     CUDA_TRY(cudaMemcpyAsync(y_host, ctx->d_x, (size_t)n_sats * 7 * T * sizeof(double), cudaMemcpyDeviceToHost, st));
     if (u_host) CUDA_TRY(cudaMemcpyAsync(u_host, ctx->d_u, (size_t)n_sats * 3 * T * sizeof(double), cudaMemcpyDeviceToHost, st));
@@ -1114,6 +1322,17 @@ static int prop_host(mpc_ctx *ctx, const double *y0, const double *tf, const mpc
         CUDA_TRY(cudaMemcpyAsync(n_steps_host, ctx->d_nodes, (size_t)n_sats * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
     CUDA_TRY(cudaStreamSynchronize(st));
     return MPC_SUCCESS;
+}
+
+int mpc_propagate_batch_rk45_ragged_host(mpc_ctx *ctx, const double *y0, const double *tf, const mpc_params *p,
+                                         const mpc_controller *ctrl, int n_sats, int T_max, const int32_t *T_sat,
+                                         const int32_t *table_len_sat, double rtol, double atol, double max_step,
+                                         double *y_host, double *u_host, int32_t *status_host, int32_t *n_steps_host)
+{
+    if (!T_sat) return fail(MPC_E_INVALID, "null T_sat");
+    PropMode m;
+    m.rk = mpc::Rk45Opts{rtol, atol, max_step};
+    return prop_host(ctx, y0, tf, p, ctrl, n_sats, T_max, m, y_host, u_host, status_host, n_steps_host, T_sat, table_len_sat);
 }
 
 int mpc_propagate_batch_host(mpc_ctx *ctx, const double *y0, const double *tf, const mpc_params *p,

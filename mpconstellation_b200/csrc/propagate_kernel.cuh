@@ -31,10 +31,11 @@ struct CtrlParams {
 };
 
 // Controller law, compile-time kind (straight-line code per law); `ir` = 1/|r| of y, already needed by gravity.
+// ku > 0: the table law of a ragged batch -- this satellite's table has ku columns, stored with the stride C.table_len
 template <int KIND>
 __device__ __forceinline__ void ctrl_eval(const CtrlParams &C, const double *__restrict__ tab, double end_tau,
                                           const double (&y)[7], double ir, double tau, double &ux, double &uy,
-                                          double &uz)
+                                          double &uz, int ku = 0)
 {
     ux = uy = uz = 0.0;
     if (KIND == 1) {  // control.py:47-53
@@ -51,12 +52,12 @@ __device__ __forceinline__ void ctrl_eval(const CtrlParams &C, const double *__r
         uz = sc * fma(hx, y[1], -hy * y[0]);
     } else if (KIND == 3) {  // control.py:104-143: FOH table on tau/end_tau, zero after end_tau
         if (tau <= end_tau) {
-            const int Ku = C.table_len;
+            const int ld = C.table_len, Ku = (ku > 0) ? ku : ld;
             const double t = tau / end_tau;
             if (t == 1.0) {
                 ux = tab[Ku - 1];
-                uy = tab[2 * Ku - 1];
-                uz = tab[3 * Ku - 1];
+                uy = tab[ld + Ku - 1];
+                uz = tab[2 * ld + Ku - 1];
             } else {
                 const double km1 = (double)(Ku - 1);
                 int k = (int)floor(t * km1);
@@ -65,8 +66,8 @@ __device__ __forceinline__ void ctrl_eval(const CtrlParams &C, const double *__r
                 const double iw = 1.0 / (hi - lo);
                 const double ln = (hi - t) * iw, lp = (t - lo) * iw;
                 ux = fma(ln, tab[k], lp * tab[k + 1]);
-                uy = fma(ln, tab[Ku + k], lp * tab[Ku + k + 1]);
-                uz = fma(ln, tab[2 * Ku + k], lp * tab[2 * Ku + k + 1]);
+                uy = fma(ln, tab[ld + k], lp * tab[ld + k + 1]);
+                uz = fma(ln, tab[2 * ld + k], lp * tab[2 * ld + k + 1]);
             }
         }
     }
@@ -114,14 +115,14 @@ __device__ __noinline__ FohCache foh_cache_fill(const double *__restrict__ tab, 
 // cases), the end point t = 1 through the last interval (lambda- = 0 there) and the cut-off after end_tau by a select --
 // the branches and slow-path guards of the literal form kept ptxas from scheduling across the seven stage evaluations.
 __device__ __forceinline__ void ctrl_eval_foh_cached(const CtrlParams &C, const double *__restrict__ tab, double end_tau,
-                                                     double tau, FohCache &fc, double &ux, double &uy, double &uz)
+                                                     double tau, FohCache &fc, double &ux, double &uy, double &uz, int ku = 0)
 {
-    const int Ku = C.table_len;
+    const int Ku = (ku > 0) ? ku : C.table_len;
     double t = tau * fc.inv_et;
     t = fma(fma(-t, end_tau, tau), fc.inv_et, t);
     int k = (int)(t * fc.km1);
     k = min(max(k, 0), Ku - 2);
-    if (k != fc.k) fc = foh_cache_fill(tab, Ku, k, fc.km1, fc.inv_et);
+    if (k != fc.k) fc = foh_cache_fill(tab, C.table_len, k, fc.km1, fc.inv_et);
     const double ln = (fc.hi - t) * fc.iw, lp = (t - fc.lo) * fc.iw;
     const bool on = tau <= end_tau;
     const double vx = fma(ln, fc.a[0], lp * fc.b[0]), vy = fma(ln, fc.a[1], lp * fc.b[1]), vz = fma(ln, fc.a[2], lp * fc.b[2]);
@@ -131,11 +132,11 @@ __device__ __forceinline__ void ctrl_eval_foh_cached(const CtrlParams &C, const 
 }
 
 // f(y,u) without the tf factor (simulator.py:130-160); returns nonzero on non-positive mass.  fc: the knot-interval cache
-// of the table law (KIND 3 only; nullptr = evaluate the law from scratch)
+// of the table law (KIND 3 only; nullptr = evaluate the law from scratch); ku: see ctrl_eval
 template <int KIND, bool DRAG, bool J2>
 __device__ __forceinline__ int prop_rhs(const PropParams &P, const CtrlParams &C, const double *__restrict__ tab,
                                         double end_tau, const double (&y)[7], double tau, double (&dy)[7],
-                                        FohCache *fc = nullptr)
+                                        FohCache *fc = nullptr, int ku = 0)
 {
     const double m = y[6];
     const double r2 = fma(y[0], y[0], fma(y[1], y[1], y[2] * y[2]));
@@ -155,8 +156,8 @@ __device__ __forceinline__ int prop_rhs(const PropParams &P, const CtrlParams &C
         ay = fma(scm, fma(hz, y[0], -hx * y[2]), -mu3 * y[1]);
         az = fma(scm, fma(hx, y[1], -hy * y[0]), -mu3 * y[2]);
     } else {
-        if (KIND == 3 && fc) ctrl_eval_foh_cached(C, tab, end_tau, tau, *fc, ux, uy, uz);
-        else ctrl_eval<KIND>(C, tab, end_tau, y, ir, tau, ux, uy, uz);
+        if (KIND == 3 && fc) ctrl_eval_foh_cached(C, tab, end_tau, tau, *fc, ux, uy, uz, ku);
+        else ctrl_eval<KIND>(C, tab, end_tau, y, ir, tau, ux, uy, uz, ku);
         ax = fma(-mu3, y[0], ux * im);
         ay = fma(-mu3, y[1], uy * im);
         az = fma(-mu3, y[2], uz * im);

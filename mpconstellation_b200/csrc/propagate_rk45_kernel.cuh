@@ -42,11 +42,16 @@ __device__ __forceinline__ double rk45_min_step(double t)
 // 0.9 * err^-0.2 (rk.py SAFETY * error_norm ** error_exponent) from err^2
 __device__ __forceinline__ double rk45_factor(double err2) { return 0.9 * pow(err2, -0.1); }
 
-template <int BLOCK, int KIND, bool DRAG, bool J2, bool SPEC>
+// RAG: a ragged batch (launched without progress words): T is the padded stride Tmax of y_out / u_out, lane s samples
+// linspace(0, 1, T_sat[s]) and stores those T_sat[s] samples only (T_sat == nullptr: all T); its sequence table (stride
+// C.table_len) has Ku_sat[s] columns (Ku_sat == nullptr: all C.table_len).  The steps do not depend on the samples.  The
+// counts are clamped into the buffers (T_sat to [0, T], Ku_sat to [2, C.table_len]); the entry points validate them.
+template <int BLOCK, int KIND, bool DRAG, bool J2, bool SPEC, bool RAG = false>
 __global__ void __launch_bounds__(BLOCK)
 propagate_rk45_kernel(const double *__restrict__ y0, const double *__restrict__ tf_arr, PropParams P, CtrlParams C,
                       Rk45Opts O, int n_sats, int T, int lpw, double *__restrict__ y_out, double *__restrict__ u_out,
-                      int32_t *__restrict__ status, int32_t *__restrict__ n_steps, unsigned int *progress, int seg_len)
+                      int32_t *__restrict__ status, int32_t *__restrict__ n_steps, unsigned int *progress, int seg_len,
+                      const int32_t *__restrict__ T_sat = nullptr, const int32_t *__restrict__ Ku_sat = nullptr)
 {
     // progress != nullptr (the overlapped pass, see propagate_kernel): window b of the discretization needs the samples
     // up to e_b = min((b+1) seg_len, T-1).  Lanes may take different numbers of steps here, so every LANE that has stored
@@ -57,6 +62,9 @@ propagate_rk45_kernel(const double *__restrict__ y0, const double *__restrict__ 
     const int s = warp * lpw + lane;
     if (lane >= lpw || s >= n_sats) return;
     const double *tab = C.table ? C.table + (C.table_per_sat ? (long long)s * 3 * C.table_len : 0) : nullptr;
+    // samples of this lane (T: the stride) and columns of its table (0: C.table_len), held inside the buffers
+    const int Tn = (RAG && T_sat) ? min(max(T_sat[s], 0), T) : T;
+    const int ku = (RAG && Ku_sat) ? min(max(Ku_sat[s], 2), C.table_len) : 0;
     const double end_tau = C.end_tau_arr ? C.end_tau_arr[s] : C.end_tau;
     const double tf = tf_arr[s];
     const double rtol = O.rtol, atol = O.atol, max_step = O.max_step;
@@ -74,16 +82,16 @@ propagate_rk45_kernel(const double *__restrict__ y0, const double *__restrict__ 
     double *yo = y_out + (long long)s * 7 * T;
     double *uo = u_out ? u_out + (long long)s * 3 * T : nullptr;
     // t_eval = np.linspace(0, 1, T): arange(T) * step, the last point exactly 1
-    const double lstep = (T > 1) ? 1.0 / (double)(T - 1) : 0.0;
+    const double lstep = (Tn > 1) ? 1.0 / (double)(Tn - 1) : 0.0;
     int ti = 0;                   // next sample to write
     double te = 0.0;              // its time
     int bad = 0, fail = 0, steps = 0;
     double t = 0.0;
 
     FohCache foh;                 // KIND 3: knot interval of the table law shared by consecutive stage evaluations
-    foh_cache_init(foh, C.table_len, end_tau);
+    foh_cache_init(foh, RAG && ku > 0 ? ku : C.table_len, end_tau);
     FohCache *const fc = (KIND == 3) ? &foh : nullptr;
-    bad |= prop_rhs<KIND, DRAG, J2>(P, C, tab, end_tau, y, 0.0, K[0]);
+    bad |= prop_rhs<KIND, DRAG, J2>(P, C, tab, end_tau, y, 0.0, K[0], nullptr, ku);
     // ---- select_initial_step (common.py), f = tf * k ------------------------------------------------------------
     double h_abs;
     {
@@ -99,7 +107,7 @@ propagate_rk45_kernel(const double *__restrict__ y0, const double *__restrict__ 
         h0 = fmin(h0, 1.0);
 #pragma unroll
         for (int i = 0; i < 7; ++i) y1[i] = fma(h0 * tf, K[0][i], y[i]);
-        bad |= prop_rhs<KIND, DRAG, J2>(P, C, tab, end_tau, y1, h0, k1);
+        bad |= prop_rhs<KIND, DRAG, J2>(P, C, tab, end_tau, y1, h0, k1, nullptr, ku);
 #pragma unroll
         for (int i = 0; i < 7; ++i) {
             const double q = tf * (k1[i] - K[0][i]) / (atol + fabs(y[i]) * rtol);
@@ -138,7 +146,7 @@ propagate_rk45_kernel(const double *__restrict__ y0, const double *__restrict__ 
 #pragma unroll
                 for (int i = 0; i < NC; ++i) ys[i] = fma(K[0][i], a10, y[i]);
                 if (CM) ys[6] = fma(K[0][6], hs * (1.0 / 5), y[6]);
-                bad |= prop_rhs<KIND, DRAG, J2>(P, C, tab, end_tau, ys, t + (1.0 / 5) * h, K[1], fc);
+                bad |= prop_rhs<KIND, DRAG, J2>(P, C, tab, end_tau, ys, t + (1.0 / 5) * h, K[1], fc, ku);
             }
             have_k1 = false;
             {
@@ -147,7 +155,7 @@ propagate_rk45_kernel(const double *__restrict__ y0, const double *__restrict__ 
 #pragma unroll
                 for (int i = 0; i < NC; ++i) ys[i] = fma(K[1][i], a1, fma(K[0][i], a0, y[i]));
                 if (CM) ys[6] = fma(K[0][6], hs * (3.0 / 10), y[6]);
-                bad |= prop_rhs<KIND, DRAG, J2>(P, C, tab, end_tau, ys, t + (3.0 / 10) * h, K[2], fc);
+                bad |= prop_rhs<KIND, DRAG, J2>(P, C, tab, end_tau, ys, t + (3.0 / 10) * h, K[2], fc, ku);
             }
             {
                 double ys[7];
@@ -155,7 +163,7 @@ propagate_rk45_kernel(const double *__restrict__ y0, const double *__restrict__ 
 #pragma unroll
                 for (int i = 0; i < NC; ++i) ys[i] = fma(K[2][i], a2, fma(K[1][i], a1, fma(K[0][i], a0, y[i])));
                 if (CM) ys[6] = fma(K[0][6], hs * (4.0 / 5), y[6]);
-                bad |= prop_rhs<KIND, DRAG, J2>(P, C, tab, end_tau, ys, t + (4.0 / 5) * h, K[3], fc);
+                bad |= prop_rhs<KIND, DRAG, J2>(P, C, tab, end_tau, ys, t + (4.0 / 5) * h, K[3], fc, ku);
             }
             {
                 double ys[7];
@@ -165,7 +173,7 @@ propagate_rk45_kernel(const double *__restrict__ y0, const double *__restrict__ 
                 for (int i = 0; i < NC; ++i)
                     ys[i] = fma(K[3][i], a3, fma(K[2][i], a2, fma(K[1][i], a1, fma(K[0][i], a0, y[i]))));
                 if (CM) ys[6] = fma(K[0][6], hs * (8.0 / 9), y[6]);
-                bad |= prop_rhs<KIND, DRAG, J2>(P, C, tab, end_tau, ys, t + (8.0 / 9) * h, K[4], fc);
+                bad |= prop_rhs<KIND, DRAG, J2>(P, C, tab, end_tau, ys, t + (8.0 / 9) * h, K[4], fc, ku);
             }
             {
                 double ys[7];
@@ -175,7 +183,7 @@ propagate_rk45_kernel(const double *__restrict__ y0, const double *__restrict__ 
                 for (int i = 0; i < NC; ++i)
                     ys[i] = fma(K[4][i], a4, fma(K[3][i], a3, fma(K[2][i], a2, fma(K[1][i], a1, fma(K[0][i], a0, y[i])))));
                 if (CM) ys[6] = fma(K[0][6], hs, y[6]);
-                bad |= prop_rhs<KIND, DRAG, J2>(P, C, tab, end_tau, ys, t + h, K[5], fc);
+                bad |= prop_rhs<KIND, DRAG, J2>(P, C, tab, end_tau, ys, t + h, K[5], fc, ku);
             }
             {
                 const double b0 = hs * (35.0 / 384), b2 = hs * (500.0 / 1113), b3 = hs * (125.0 / 192),
@@ -184,7 +192,7 @@ propagate_rk45_kernel(const double *__restrict__ y0, const double *__restrict__ 
                 for (int i = 0; i < NC; ++i)
                     yn[i] = fma(K[5][i], b5, fma(K[4][i], b4, fma(K[3][i], b3, fma(K[2][i], b2, fma(K[0][i], b0, y[i])))));
                 if (CM) yn[6] = fma(K[0][6], hs, y[6]);
-                bad |= prop_rhs<KIND, DRAG, J2>(P, C, tab, end_tau, yn, t + h, K[6], fc);
+                bad |= prop_rhs<KIND, DRAG, J2>(P, C, tab, end_tau, yn, t + h, K[6], fc, ku);
             }
             double k1n[7];
             int bad_n = 0;
@@ -199,7 +207,7 @@ propagate_rk45_kernel(const double *__restrict__ y0, const double *__restrict__ 
 #pragma unroll
                 for (int i = 0; i < NC; ++i) ys[i] = fma(K[6][i], a10, yn[i]);
                 if (CM) ys[6] = fma(K[0][6], a10, yn[6]);
-                bad_n = prop_rhs<KIND, DRAG, J2>(P, C, tab, end_tau, ys, t_new + (1.0 / 5) * h_pred, k1n, fc);
+                bad_n = prop_rhs<KIND, DRAG, J2>(P, C, tab, end_tau, ys, t_new + (1.0 / 5) * h_pred, k1n, fc, ku);
             }
             // -- error norm (rk.py _estimate_error_norm) ---------------------------------------------------------------
             double eh[NC], esum0 = 0.0;
@@ -252,7 +260,7 @@ propagate_rk45_kernel(const double *__restrict__ y0, const double *__restrict__ 
         }
         if (bad || fail) break;
         // ---- samples with t_eval <= t_new off the dense output of this step (ivp.py:712-728, rk.py:723-737) ----------
-        if (ti < T && te <= t_new) {
+        if (ti < Tn && te <= t_new) {
             // Q = K^T P; column 0 of P is e_1 and its row 1 is zero
             double Q[7][4];
             const double hs = h * tf;
@@ -277,7 +285,7 @@ propagate_rk45_kernel(const double *__restrict__ y0, const double *__restrict__ 
             MPC_QROW(5, -282668133.0 / 205662961.0, 2019193451.0 / 616988883.0, -1453857185.0 / 822651844.0)
             MPC_QROW(6, 40617522.0 / 29380423.0, -110615467.0 / 29380423.0, 69997945.0 / 29380423.0)
 #undef MPC_QROW
-            while (ti < T && te <= t_new) {
+            while (ti < Tn && te <= t_new) {
                 const double xx = (te - t) / h;
                 const double x2 = xx * xx, x3 = x2 * xx, x4 = x3 * xx;
                 double ys[7];
@@ -294,7 +302,7 @@ propagate_rk45_kernel(const double *__restrict__ y0, const double *__restrict__ 
                 if (uo) {   // Discretizer.extract_uk (linearize_discretize.py:393-411) on the sample
                     double ux, uy, uz;
                     const double irs = fast_rsqrt(fma(ys[0], ys[0], fma(ys[1], ys[1], ys[2] * ys[2])));
-                    ctrl_eval<KIND>(C, tab, end_tau, ys, irs, te, ux, uy, uz);
+                    ctrl_eval<KIND>(C, tab, end_tau, ys, irs, te, ux, uy, uz, ku);
                     uo[ti] = ux;
                     uo[T + ti] = uy;
                     uo[2 * (long long)T + ti] = uz;
@@ -314,7 +322,7 @@ propagate_rk45_kernel(const double *__restrict__ y0, const double *__restrict__ 
                     if (lane == __ffs(peers) - 1) atomicAdd(progress + b, (unsigned)__popc(peers));
                 }
                 ++ti;
-                te = (ti == T - 1) ? 1.0 : (double)ti * lstep;
+                te = (ti == Tn - 1) ? 1.0 : (double)ti * lstep;
             }
         }
 #pragma unroll
@@ -328,7 +336,7 @@ propagate_rk45_kernel(const double *__restrict__ y0, const double *__restrict__ 
         // the reference raises here (simulator.py:135-136) or solve_ivp reports failure: nothing is handed on.  The
         // samples not yet written become NaN, and the windows waiting on them are released.
         const double qnan = __longlong_as_double(0x7ff8000000000000LL);
-        for (; ti < T; ++ti) {
+        for (; ti < Tn; ++ti) {
 #pragma unroll
             for (int c = 0; c < 7; ++c) yo[(long long)c * T + ti] = qnan;
             if (uo) {

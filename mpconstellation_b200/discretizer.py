@@ -140,8 +140,13 @@ class Discretizer:
 
     # -- batched form ------------------------------------------------------------------------------
     def discretize_batch(self, f, x, u, tf, out=None, check=True):
-        """x [N,7,K], u [N,3,K], tf scalar or [N] -> batch.DiscretizedBatch (SoA + reference-shaped views)."""
+        """x [N,7,K], u [N,3,K], tf scalar or [N] -> batch.DiscretizedBatch (SoA + reference-shaped views).
+        x, u may also be lists of the per-satellite (7,K_s) / (3,K_s) arrays Optimizer.solve_OPT holds (optimizer.py:
+        243-249): they are packed into one ragged batch (padded to max K_s) and discretized in one launch."""
         self._check_options(f)
+        K_sat = None
+        if isinstance(x, (list, tuple)):
+            x, u, K_sat = pack_ragged(x, u)
         x = np.asarray(x, dtype=np.float64)
         u = np.asarray(u, dtype=np.float64)
         K = x.shape[2]
@@ -156,7 +161,7 @@ class Discretizer:
         return batch.discretize_batch(x, u, tf, self.const, include_J2=self.include_J2,
                                       include_drag=bool(self.include_drag), disc_drag=self._disc_drag(x),
                                       n_sub=max(1, int(self.integrator_steps) - 1), out=out, device=self.device,
-                                      check=check, adaptive=adaptive)
+                                      check=check, adaptive=adaptive, K=K_sat)
 
     @staticmethod
     def extract_uk(x_k, tau_k, controller):
@@ -165,3 +170,19 @@ class Discretizer:
         u_func = spec_from(controller).host_u_func() if not callable(controller) or hasattr(controller, "device_spec") \
             else controller
         return np.column_stack([u_func(x_k[:, i], tau_k[i]) for i in range(x_k.shape[1])])
+
+
+def pack_ragged(xs, us):
+    """Per-satellite arrays (7,K_s) / (3,K_s) -> x [N,7,Kmax], u [N,3,Kmax] (NaN past K_s), K_sat int32 [N]."""
+    if len(xs) != len(us) or not xs:
+        raise ValueError("need one (7,K_s) and one (3,K_s) array per satellite")
+    K_sat = np.array([np.shape(a)[1] for a in xs], dtype=np.int32)
+    if any(np.shape(a) != (7, k) for a, k in zip(xs, K_sat)) or any(np.shape(b) != (3, k) for b, k in zip(us, K_sat)):
+        raise ValueError("satellite s needs x (7,K_s) and u (3,K_s) on the same K_s nodes")
+    Kmax = int(K_sat.max())
+    x = np.full((len(xs), 7, Kmax), np.nan)
+    u = np.full((len(us), 3, Kmax), np.nan)
+    for s, (a, b) in enumerate(zip(xs, us)):
+        x[s, :, :K_sat[s]] = a
+        u[s, :, :K_sat[s]] = b
+    return x, u, K_sat

@@ -7,8 +7,10 @@ and Simulator.run_segments (simulator.py:79-94) advances the satellites segment 
 
 `BatchedSCP` keeps that control flow but evaluates both hot-path legs for ALL satellites at once on the GPU.  The
 convex subproblem itself (pyomo + ipopt, optimizer.py:251-613) is out of scope and is injected as a callable:
-    solver(hand_off) -> (u_new [N,3,K], tf_new [N])
-where `hand_off.sat(s)` yields exactly the five arrays optimizer.py:327-339 indexes.  With pyomo/ipopt installed one
+    solver(hand_off) -> (u_new [N,3,Kmax] padded, or a list of (3,K_s) arrays; tf_new [N])
+where `hand_off.sat(s)` yields exactly the five arrays optimizer.py:327-339 indexes.  Every satellite is linearized on
+its own K_s = int(base_res * tf_s) nodes, as the reference's per-satellite controllers do (control.py:221,227,
+simulator.py:38); batches whose K_s differ run as one ragged launch per leg.  With pyomo/ipopt installed one
 wraps the reference's Optimizer in such a callable; `hold_reference_solver` is a deterministic stand-in (it returns the
 reference input unchanged) for boxes without a solver, clearly NOT an optimizer.
 """
@@ -24,10 +26,11 @@ from . import _lib
 @dataclass
 class Linearization:
     """Result of one batched linearization pass (the hand-off to the subproblem)."""
-    x_bar: np.ndarray        # [N,7,K] reference trajectories
-    u_bar: np.ndarray        # [N,3,K] reference inputs (extract_uk)
+    x_bar: np.ndarray        # [N,7,Kmax] reference trajectories (NaN past K_s)
+    u_bar: np.ndarray        # [N,3,Kmax] reference inputs (extract_uk)
     tf: np.ndarray           # [N]
     matrices: "batch.DiscretizedBatch"
+    K: np.ndarray = None     # [N] nodes of every satellite, int(base_res * tf_s)
 
     def sat(self, s):
         """(A_k, B_kp, B_kn, Sigma_k, xi_k) of satellite s -- what Optimizer.solve_OPT appends at optimizer.py:243-249."""
@@ -37,7 +40,7 @@ class Linearization:
         """Residual of the reference's dynamics constraint (optimizer.py:327-339) for a candidate (x [7,K], u [3,K], tf),
         indexed exactly as the pyomo rule does: one value per (i, k)."""
         A_k, B_kp, B_kn, Sigma_k, xi_k = self.sat(s)
-        K = x.shape[1]
+        K = int(self.K[s]) if self.K is not None else x.shape[1]
         res = np.zeros((7, K - 1))
         for k in range(K - 1):
             for i in range(7):
@@ -52,6 +55,32 @@ class Linearization:
 def hold_reference_solver(lin):
     """Stand-in for the pyomo/ipopt subproblem: keeps the reference input and final time (NOT an optimizer)."""
     return np.array(lin.u_bar), np.array(lin.tf)
+
+
+def node_counts(base_res, tf):
+    """K_s = int(base_res * tf_s) per satellite, the reference's own expression (simulator.py:38); K_s < 2 raises."""
+    K = np.array([int(base_res * float(t)) for t in np.atleast_1d(tf)], dtype=np.int32)
+    if K.size and K.min() < 2:
+        raise ValueError(f"int(base_res * tf) < 2 nodes for satellite {int(np.argmin(K))} (tf = "
+                         f"{float(np.atleast_1d(tf)[np.argmin(K)])}, base_res = {base_res})")
+    return K
+
+
+def sequence_table(u_new, K):
+    """The solver's inputs as a sequence table: (table [N,3,Ku], per-satellite lengths or None when all are equal).
+    u_new: [N,3,Kmax] padded (satellite s has K[s] columns) or a list of (3,K_s) arrays."""
+    if isinstance(u_new, (list, tuple)):
+        lens = np.array([np.shape(a)[1] for a in u_new], dtype=np.int32)
+        tab = np.zeros((len(u_new), 3, int(lens.max())))
+        for s, a in enumerate(u_new):
+            tab[s, :, :lens[s]] = a
+    else:
+        tab = np.ascontiguousarray(u_new, dtype=np.float64)
+        lens = np.minimum(np.asarray(K, dtype=np.int32), tab.shape[2])
+    if (lens == lens[0]).all():
+        return np.ascontiguousarray(tab[:, :, :lens[0]]), None
+    tab = np.ascontiguousarray(np.nan_to_num(tab, nan=0.0))   # (padding is never read; keep it finite)
+    return tab, lens
 
 
 class BatchedSCP:
@@ -74,7 +103,20 @@ class BatchedSCP:
         y0 = np.ascontiguousarray(y0, dtype=np.float64)
         N = y0.shape[0]
         tfv = np.ascontiguousarray(np.broadcast_to(np.asarray(tf, dtype=np.float64), (N,)))
-        K = int(self.base_res * float(np.max(tfv)))
+        K_sat = node_counts(self.base_res, tfv)
+        ragged_law = getattr(spec_from(controller), "table_len", None) is not None
+        if (K_sat != K_sat[0]).any() or ragged_law:
+            # one ragged launch per leg: every satellite on its own grid (the fused pass is rectangular only)
+            x, u, _, _ = batch.propagate_batch(y0, tfv, controller, self.const, include_drag=False, include_J2=False,
+                                               T=K_sat, device=self.device)
+            if self.use_uniform_steps:
+                res = batch.discretize_batch(x, u, tfv, self.const, include_J2=self.include_J2, device=self.device,
+                                             n_sub=self.integrator_steps - 1, K=K_sat)
+            else:
+                res = batch.discretize_batch(x, u, tfv, self.const, include_J2=self.include_J2, device=self.device,
+                                             adaptive=dict(rtol=1e-3, atol=1e-6, max_step=1e-2), K=K_sat)
+            return Linearization(np.asarray(x), np.asarray(u), tfv, res, K_sat)
+        K = int(K_sat[0])
         if self.use_uniform_steps:
             # (k-major layout: the streamed host pass; the per-satellite views of the result hide it)
             res, x, u = batch.propagate_discretize(y0, tfv, controller, self.const, T=K, disc_J2=self.include_J2,
@@ -85,11 +127,16 @@ class BatchedSCP:
                                                T=K, device=self.device)
             res = batch.discretize_batch(x, u, tfv, self.const, include_J2=self.include_J2, device=self.device,
                                          adaptive=dict(rtol=1e-3, atol=1e-6, max_step=1e-2))
-        return Linearization(np.asarray(x), np.asarray(u), tfv, res)
+        return Linearization(np.asarray(x), np.asarray(u), tfv, res, K_sat)
 
     def plan(self, y0, solver=hold_reference_solver):
         """OptimalController.update for N satellites: seed trajectory, then n_iterations of (linearize, solve,
-        re-propagate with the solved inputs).  Returns the per-satellite input tables [N,3,K] and their tf_u."""
+        re-propagate with the solved inputs).  Returns the per-satellite input tables [N,3,Ku] (satellite s: the K_s
+        columns of its last solve, zero-padded) and their tf_u."""
+        tab, _, tf_u, history = self._plan(y0, solver)
+        return tab, tf_u, history
+
+    def _plan(self, y0, solver):
         N = y0.shape[0]
         ctrl = ConstantTangentialThrustController(tangential_thrust=self.seed_thrust)
         tf_u = np.full(N, self.horizon)
@@ -97,11 +144,12 @@ class BatchedSCP:
         for _ in range(self.n_iterations):
             lin = self.linearize(y0, tf_u, ctrl)
             u_new, tf_u = solver(lin)
-            u_new = np.ascontiguousarray(u_new, dtype=np.float64)
+            tab, lens = sequence_table(u_new, lin.K)
             history.append(lin)
-            # SequenceController(u=u_opt, tf_u=tf_u, tf_sim=tf_u) -> end_tau = 1 (control.py:221)
-            ctrl = ControllerSpec(_lib.CTRL_SEQUENCE, (0.0, 0.0, 0.0), u_new, 1.0)
-        return u_new, tf_u, history
+            # SequenceController(u=u_opt, tf_u=tf_u, tf_sim=tf_u) -> end_tau = 1 (control.py:221); satellite s's table
+            # has the K_s columns of its own solve
+            ctrl = ControllerSpec(_lib.CTRL_SEQUENCE, (0.0, 0.0, 0.0), tab, 1.0, lens)
+        return tab, lens, tf_u, history
 
     def run_segments(self, y0, n_segments, solver=hold_reference_solver, include_drag=True, include_J2=True,
                      sim_base_res=100):
@@ -112,10 +160,10 @@ class BatchedSCP:
         N = y.shape[0]
         traj, plans = [], []
         for _ in range(n_segments):
-            u_tab, tf_u, hist = self.plan(y, solver)
+            u_tab, lens, tf_u, hist = self._plan(y, solver)
             plans.append(hist)
             end_tau = np.asarray(tf_u, dtype=np.float64) / self.interval     # one end_tau per satellite
-            ctrl = ControllerSpec(_lib.CTRL_SEQUENCE, (0.0, 0.0, 0.0), u_tab, end_tau)
+            ctrl = ControllerSpec(_lib.CTRL_SEQUENCE, (0.0, 0.0, 0.0), u_tab, end_tau, lens)
             T = int(sim_base_res * self.interval)
             ys, _, _, _ = batch.propagate_batch(y, self.interval, ctrl, self.const, include_drag=include_drag,
                                                 include_J2=include_J2, T=T, device=self.device)
