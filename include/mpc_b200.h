@@ -438,6 +438,40 @@ int mpc_constraint_terms_host(mpc_ctx *ctx, const double *x, const double *u, in
 int mpc_dynamics_jacobian(const double *soa, int64_t pitch, int64_t offset, int n_sats, int K, double *values,
                           int64_t *indices, double *rhs, void *stream);
 
+/*
+ * Ragged batches (satellite s on its own K_s = K_sat[s] nodes, 2 <= K_s <= K_max; the hand-off of
+ * mpc_discretize_batch_ragged).  Buffers stay padded to K_max and the padding is never written; one launch for the
+ * batch, the threads mapped to the live intervals only.
+ *   K_sat   HOST array [n_sats] (validated; it also sizes the launch)
+ *   first   DEVICE scratch of n_sats + 1 int64, filled by the call (prefix sums first[s] = sum_{r<s} (K_r - 1))
+ *
+ * mpc_constraint_terms_ragged: x [n_sats][7][K_max], u [n_sats][3][K_max] on the nodes of x.  Satellite s gets
+ * rbar_hat [n_sats][3][K_max-1] columns k < K_s - 1, ubar_hat [n_sats][3][K_max] columns k < K_s and final_terms
+ * [n_sats][MPC_FINAL_TERMS] from node K_s - 1: bit for bit what mpc_constraint_terms gives for that satellite alone at
+ * K = u_cols = K_s.
+ */
+int mpc_constraint_terms_ragged(const double *x, const double *u, int n_sats, int K_max, const int32_t *K_sat, int64_t *first,
+                                double mu, double *rbar_hat, double *ubar_hat, double *final_terms, void *stream);
+/* Host-buffer form: x, u, K_sat and the outputs are host arrays; the padding columns of rbar_hat / ubar_hat are NaN. */
+int mpc_constraint_terms_ragged_host(mpc_ctx *ctx, const double *x, const double *u, int n_sats, int K_max,
+                                     const int32_t *K_sat, double mu, double *rbar_hat, double *ubar_hat, double *final_terms);
+
+/*
+ * mpc_dynamics_jacobian_ragged: the dynamics constraint of a ragged batch as a block-diagonal CSR of n_sats independent
+ * single-satellite systems, each with its own final time tf_s (every satellite's Optimizer has its own tf variable,
+ * optimizer.py:281).  Block s is the numbering of mpc_dynamics_jacobian with n_sats = 1, K = K_s, shifted:
+ *   rows       R_s = 7 first[s];   row = R_s + i (K_s-1) + k                       (7 first[n_sats] rows)
+ *   variables  V_s = sum_{r<s} (17 K_r + 1) = 17 (first[s] + s) + s                (17 (first[n_sats] + n_sats) + n_sats)
+ *              x[i,k] -> V_s + i K_s + k          u[j,k] -> V_s + 7 K_s + j K_s + k
+ *              nu[i,k] -> V_s + 10 K_s + i K_s + k   tf_s -> V_s + 17 K_s
+ * Still MPC_JAC_NNZ_PER_ROW non-zeros per row in ascending column order (indptr[r] = 16 r).  soa holds the ragged
+ * result of mpc_discretize_batch_ragged: satellite s, interval k at column offset + s (K_max-1) + k, pitch >= offset +
+ * n_sats (K_max-1).  indices may be NULL (only the values change between SCP iterations).  Device pointers except K_sat.
+ */
+int mpc_dynamics_jacobian_ragged(const double *soa, int64_t pitch, int64_t offset, int n_sats, int K_max,
+                                 const int32_t *K_sat, int64_t *first, double *values, int64_t *indices, double *rhs,
+                                 void *stream);
+
 /* ---------------------------------------------------------------- measurement helpers */
 
 /* FP64 FMA-chain microbenchmark: measured DFMA peak of `device` in TFLOP/s (2 flop per FMA). */

@@ -157,6 +157,9 @@ def lib():
     L.mpc_dynamics_jacobian.argtypes = [_DP, i64, i64, i, i, _DP, _DP, _DP, vp]
     L.mpc_constraint_terms.argtypes = [_DP, _DP, i, i, i, d, _DP, _DP, _DP, vp]
     L.mpc_constraint_terms_host.argtypes = [vp, _DP, _DP, i, i, i, d, _DP, _DP, _DP]
+    L.mpc_constraint_terms_ragged.argtypes = [_DP, _DP, i, i, _DP, _DP, d, _DP, _DP, _DP, vp]
+    L.mpc_constraint_terms_ragged_host.argtypes = [vp, _DP, _DP, i, i, _DP, d, _DP, _DP, _DP]
+    L.mpc_dynamics_jacobian_ragged.argtypes = [_DP, i64, i64, i, i, _DP, _DP, _DP, _DP, _DP, vp]
     L.mpc_fp64_peak_probe.argtypes = [i, i, ctypes.POINTER(ctypes.c_double), ctypes.POINTER(ctypes.c_double)]
     L.mpc_set_gather_tuning.argtypes = [i, i]
     L.mpc_set_gather_tuning.restype = i
@@ -167,7 +170,8 @@ def lib():
                  "mpc_discretize_batch_ugrid", "mpc_discretize_batch_ugrid_host",
                  "mpc_ctx_create", "mpc_ctx_destroy", "mpc_discretize_batch_host", "mpc_propagate_batch_host",
                  "mpc_propagate_discretize_host", "mpc_propagate_discretize", "mpc_propagate_discretize_multi", "mpc_fp64_peak_probe", "mpc_constraint_terms",
-                 "mpc_constraint_terms_host", "mpc_discretize_batch_push", "mpc_fill_const_rows", "mpc_dynamics_jacobian"):
+                 "mpc_constraint_terms_host", "mpc_discretize_batch_push", "mpc_fill_const_rows", "mpc_dynamics_jacobian",
+                 "mpc_constraint_terms_ragged", "mpc_constraint_terms_ragged_host", "mpc_dynamics_jacobian_ragged"):
         getattr(L, name).restype = i
     _lib = L
     return L
@@ -184,6 +188,7 @@ EXPORTED_SYMBOLS = [
     "mpc_discretize_batch_host", "mpc_discretize_batch_adaptive_host", "mpc_discretize_batch_ugrid_host", "mpc_propagate_batch_host", "mpc_propagate_discretize_host", "mpc_propagate_discretize", "mpc_propagate_discretize_multi",
     "mpc_constraint_terms", "mpc_constraint_terms_host", "mpc_discretize_batch_push", "mpc_fill_const_rows",
     "mpc_dynamics_jacobian",
+    "mpc_constraint_terms_ragged", "mpc_constraint_terms_ragged_host", "mpc_dynamics_jacobian_ragged",
     "mpc_fp64_peak_probe", "mpc_set_tuning", "mpc_set_gather_tuning",
 ]
 

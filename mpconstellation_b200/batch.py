@@ -356,36 +356,53 @@ def _torch():
 
 
 def discretize_batch_device(x, u, tf, const, include_J2=False, n_sub=100, out=None, out_pitch=None, out_offset=0,
-                            status=None, extra_dst=None, adaptive=None, n_nodes=None):
+                            status=None, extra_dst=None, adaptive=None, n_nodes=None, K=None, first=None):
     """Device form: x [N,7,K], u [N,3,K], tf [N] are float64 CUDA tensors; work is enqueued on torch's
     current stream, nothing synchronises.  `out` is [105, pitch]; `extra_dst` is an optional list of
-    further [105, pitch] buffers (e.g. peer-mapped) every result is also stored to (total 1,2,4 or 8)."""
+    further [105, pitch] buffers (e.g. peer-mapped) every result is also stored to (total 1,2,4 or 8).
+    K = int array [N] (host): a ragged batch as in discretize_batch (x, u [N,.,Kmax]); `first` is an int64 CUDA tensor
+    [N+1] the call fills with the prefix sums of K_s - 1 (allocated when None).  The padding columns of `out` are not
+    written; status (zeroed when allocated here) and n_nodes keep the [N*(Kmax-1)] layout."""
     torch = _torch()
-    N, _, K = x.shape
-    n_int = N * (K - 1)
+    N, _, K_ = x.shape
+    n_int = N * (K_ - 1)
     assert x.is_cuda and x.dtype == torch.float64 and x.is_contiguous()
-    assert u.shape == (N, 3, K) and u.is_contiguous() and tf.shape == (N,)
+    assert u.shape == (N, 3, K_) and u.is_contiguous() and tf.shape == (N,)
+    K_sat = None
+    if K is not None:
+        K_sat = _counts(K, N, K_, "K")
+        if extra_dst:
+            raise ValueError("a ragged batch has one destination")
+        if first is None:
+            first = torch.empty(N + 1, dtype=torch.int64, device=x.device)
     if out is None:
         out = torch.empty((_lib.MPC_OUT_ROWS, n_int), dtype=torch.float64, device=x.device)
     pitch = out.shape[1] if out_pitch is None else int(out_pitch)
     if status is None:
-        status = torch.empty(n_int, dtype=torch.int32, device=x.device)
+        status = (torch.zeros if K_sat is not None else torch.empty)(n_int, dtype=torch.int32, device=x.device)
     p = _lib.make_params(const, include_J2, False)
     stream = torch.cuda.current_stream(x.device).cuda_stream
     L = _lib.lib()
-    if adaptive is not None:
+    if K_sat is not None:
+        ad = adaptive or {}
+        _lib.check(L.mpc_discretize_batch_ragged(
+            x.data_ptr(), u.data_ptr(), tf.data_ptr(), ctypes.byref(p), N, K_, _lib.addr(K_sat), first.data_ptr(),
+            int(adaptive is not None), int(n_sub), float(ad.get("rtol", 1e-3)), float(ad.get("atol", 1e-6)),
+            float(ad.get("max_step", 1e-2)), out.data_ptr(), pitch, int(out_offset), status.data_ptr(),
+            n_nodes.data_ptr() if n_nodes is not None else None, stream))
+    elif adaptive is not None:
         _lib.check(L.mpc_discretize_batch_adaptive(
-            x.data_ptr(), u.data_ptr(), tf.data_ptr(), ctypes.byref(p), N, K, float(adaptive.get("rtol", 1e-3)),
+            x.data_ptr(), u.data_ptr(), tf.data_ptr(), ctypes.byref(p), N, K_, float(adaptive.get("rtol", 1e-3)),
             float(adaptive.get("atol", 1e-6)), float(adaptive.get("max_step", 1e-2)), out.data_ptr(), pitch,
             int(out_offset), status.data_ptr(), n_nodes.data_ptr() if n_nodes is not None else None, stream))
     elif extra_dst:
         ptrs = [out.data_ptr()] + [int(d if isinstance(d, int) else d.data_ptr()) for d in extra_dst]
         arr = (ctypes.c_void_p * len(ptrs))(*ptrs)
-        _lib.check(L.mpc_discretize_batch_multi(x.data_ptr(), u.data_ptr(), tf.data_ptr(), ctypes.byref(p), N, K,
+        _lib.check(L.mpc_discretize_batch_multi(x.data_ptr(), u.data_ptr(), tf.data_ptr(), ctypes.byref(p), N, K_,
                                                 int(n_sub), arr, len(ptrs), pitch, int(out_offset),
                                                 status.data_ptr(), stream))
     else:
-        _lib.check(L.mpc_discretize_batch(x.data_ptr(), u.data_ptr(), tf.data_ptr(), ctypes.byref(p), N, K,
+        _lib.check(L.mpc_discretize_batch(x.data_ptr(), u.data_ptr(), tf.data_ptr(), ctypes.byref(p), N, K_,
                                           int(n_sub), out.data_ptr(), pitch, int(out_offset), status.data_ptr(),
                                           stream))
     return out, status
@@ -393,10 +410,22 @@ def discretize_batch_device(x, u, tf, const, include_J2=False, n_sub=100, out=No
 
 def propagate_batch_device(y0, tf, controller, const, include_drag=True, include_J2=True, T=100, n_sub=None,
                            y=None, u_out=None, status=None):
-    """Device form of propagate_batch: y0 [N,7], tf [N] float64 CUDA tensors -> y [N,7,T], u [N,3,T], status [N]."""
+    """Device form of propagate_batch: y0 [N,7], tf [N] float64 CUDA tensors -> y [N,7,T], u [N,3,T], status [N].
+    T = int array [N] (host): satellite s sampled at linspace(0, 1, T_s) into the first T_s columns of y / u [.,.,Tmax]
+    (the padding columns are not written), the reference integrator only, as propagate_batch; so is a sequence law
+    with per-satellite table lengths (ControllerSpec.table_len)."""
     torch = _torch()
     N = y0.shape[0]
     spec = spec_from(controller)
+    T_sat = tab_len = None
+    if spec.kind == _lib.CTRL_SEQUENCE and spec.table_len is not None:
+        tab_len = _counts(spec.table_len, N, np.shape(spec.table)[-1], "table_len")
+    if np.ndim(T) != 0:
+        T_sat = _counts(T, N, int(np.max(T)) if N else 2, "T")
+        T = int(T_sat.max()) if N else 2
+    T = int(T)
+    if (T_sat is not None or tab_len is not None) and n_sub not in (None, 0):
+        raise ValueError("per-satellite sample counts / table lengths need the reference integrator (n_sub=None)")
     if n_sub is None:
         n_sub = 0                         # the reference's RK45, replayed (see propagate_batch)
     if y is None:
@@ -405,8 +434,7 @@ def propagate_batch_device(y0, tf, controller, const, include_drag=True, include
         u_out = torch.empty((N, 3, T), dtype=torch.float64, device=y0.device)
     if status is None:
         status = torch.empty(N, dtype=torch.int32, device=y0.device)
-    _rectangular_law(spec)
-    tab_dev = et_dev = None
+    tab_dev = et_dev = cnt_dev = len_dev = None
     if spec.kind == _lib.CTRL_SEQUENCE:
         tab_dev = torch.as_tensor(spec.table, dtype=torch.float64).to(y0.device).contiguous()
         if np.ndim(spec.end_tau) != 0:
@@ -415,10 +443,19 @@ def propagate_batch_device(y0, tf, controller, const, include_drag=True, include
                             end_tau_addr=et_dev.data_ptr() if et_dev is not None else None)
     p = _lib.make_params(const, include_J2, include_drag)
     stream = torch.cuda.current_stream(y0.device).cuda_stream
-    _lib.check(_lib.lib().mpc_propagate_batch(y0.data_ptr(), tf.data_ptr(), ctypes.byref(p), ctypes.byref(c), N,
-                                              int(T), int(n_sub), y.data_ptr(), u_out.data_ptr(),
-                                              status.data_ptr(), stream))
-    for t_ in (tab_dev, et_dev):
+    if T_sat is not None or tab_len is not None:
+        # the ragged entry point reads the counts on the device
+        cnt_dev = torch.as_tensor(T_sat if T_sat is not None else np.full(N, T, dtype=np.int32)).to(y0.device)
+        len_dev = torch.as_tensor(tab_len).to(y0.device) if tab_len is not None else None
+        _lib.check(_lib.lib().mpc_propagate_batch_rk45_ragged(
+            y0.data_ptr(), tf.data_ptr(), ctypes.byref(p), ctypes.byref(c), N, T, cnt_dev.data_ptr(),
+            len_dev.data_ptr() if len_dev is not None else None, 1e-3, 1e-6, 1e-3, y.data_ptr(), u_out.data_ptr(),
+            status.data_ptr(), None, stream))
+    else:
+        _lib.check(_lib.lib().mpc_propagate_batch(y0.data_ptr(), tf.data_ptr(), ctypes.byref(p), ctypes.byref(c), N,
+                                                  int(T), int(n_sub), y.data_ptr(), u_out.data_ptr(),
+                                                  status.data_ptr(), stream))
+    for t_ in (tab_dev, et_dev, cnt_dev, len_dev):
         if t_ is not None:
             t_.record_stream(torch.cuda.current_stream(y0.device))
     return y, u_out, status

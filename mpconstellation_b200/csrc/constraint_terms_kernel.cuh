@@ -14,6 +14,8 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include "discretize_kernel.cuh"   // ragged_locate
+
 namespace mpc {
 
 constexpr int kFinalTerms = 32;
@@ -160,37 +162,72 @@ __device__ inline void terminal_terms(const double (&r)[3], const double (&v)[3]
     o[kOffDVnB] = g[0] * r[0] + g[1] * r[1] + g[2] * r[2] + g[3] * v[0] + g[4] * v[1] + g[5] * v[2];
 }
 
+// The per-column pieces of optimizer.py:128-168, shared by the rectangular and the ragged launch.  Satellite s's blocks:
+// x [7][ld], rbar_hat [3][ld-1], u and ubar_hat [3][ldu].
+__device__ __forceinline__ void rbar_column(const double *__restrict__ xs, int ld, int c, double *__restrict__ rbar_hat, int s)
+{   // :128-129  r_bar / ||r_bar||  (columns 0..K-2); no contraction, bit-identical to numpy
+    const double r0 = xs[c], r1 = xs[ld + c], r2 = xs[2 * ld + c];
+    const double n = __dsqrt_rn(__dadd_rn(__dadd_rn(__dmul_rn(r0, r0), __dmul_rn(r1, r1)), __dmul_rn(r2, r2)));
+    double *o = rbar_hat + (size_t)s * 3 * (ld - 1);
+    o[c] = __ddiv_rn(r0, n);
+    o[(ld - 1) + c] = __ddiv_rn(r1, n);
+    o[2 * (ld - 1) + c] = __ddiv_rn(r2, n);
+}
+
+__device__ __forceinline__ void ubar_column(const double *__restrict__ u, int ldu, int c, double eps, double *__restrict__ ubar_hat,
+                                            int s)
+{   // :132-139  (mask as written: filled where the norm is <= eps, zero elsewhere)
+    const double *us = u + (size_t)s * 3 * ldu;
+    const double u0 = us[c], u1 = us[ldu + c], u2 = us[2 * ldu + c];
+    const double n = __dsqrt_rn(__dadd_rn(__dadd_rn(__dmul_rn(u0, u0), __dmul_rn(u1, u1)), __dmul_rn(u2, u2)));
+    const bool fill = n <= eps;
+    double *o = ubar_hat + (size_t)s * 3 * ldu;
+    o[c] = fill ? __ddiv_rn(u0, n) : 0.0;
+    o[ldu + c] = fill ? __ddiv_rn(u1, n) : 0.0;
+    o[2 * ldu + c] = fill ? __ddiv_rn(u2, n) : 0.0;
+}
+
 // x [N][7][K], u [N][3][Ku] -> rbar_hat [N][3][K-1], ubar_hat [N][3][Ku], fin [N][32].
 // Thread i covers column c = i % C of satellite s = i / C, C = max(K, Ku): consecutive threads touch
 // consecutive addresses of every row.
+//
+// RAG: a ragged batch.  K = Ku = Kmax is the padded stride and first[] the prefix sums of K_s - 1 (ragged_locate); the
+// launch covers the live intervals of every satellite.  The thread of interval k writes column k of rbar_hat and
+// ubar_hat; the thread of the last interval (k = K_s - 2) also writes ubar_hat column K_s - 1 and the terminal terms of
+// node K_s - 1.  Satellite s gets exactly the bits of a rectangular launch of that satellite at K = Ku = K_s; the padding
+// columns are never written.
+template <bool RAG = false>
 __global__ void __launch_bounds__(256)
 constraint_terms_kernel(const double *__restrict__ x, const double *__restrict__ u, int n_sats, int K, int Ku,
                         double mu, double eps, double *__restrict__ rbar_hat, double *__restrict__ ubar_hat,
-                        double *__restrict__ fin)
+                        double *__restrict__ fin, const long long *__restrict__ first = nullptr)
 {
-    const int C = K > Ku ? K : Ku;
     const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (RAG) {
+        if (i >= first[n_sats] - first[0]) return;
+        int s, k, Ks;
+        ragged_locate(first, n_sats, i, s, k, Ks);
+        const double *xs = x + (size_t)s * 7 * K;
+        rbar_column(xs, K, k, rbar_hat, s);
+        ubar_column(u, K, k, eps, ubar_hat, s);
+        if (k == Ks - 2) {
+            ubar_column(u, K, Ks - 1, eps, ubar_hat, s);
+            const double r[3] = {xs[Ks - 1], xs[K + Ks - 1], xs[2 * K + Ks - 1]};
+            const double v[3] = {xs[3 * K + Ks - 1], xs[4 * K + Ks - 1], xs[5 * K + Ks - 1]};
+            double o[kFinalTerms];
+            terminal_terms(r, v, mu, o);
+            double *dst = fin + (size_t)s * kFinalTerms;
+#pragma unroll
+            for (int j = 0; j < kFinalTerms; ++j) dst[j] = o[j];
+        }
+        return;
+    }
+    const int C = K > Ku ? K : Ku;
     if (i >= (long long)n_sats * C) return;
     const int s = (int)(i / C), c = (int)(i % C);
     const double *xs = x + (size_t)s * 7 * K;
-    if (c < K - 1) {   // :128-129  r_bar / ||r_bar||  (columns 0..K-2); no contraction, bit-identical to numpy
-        const double r0 = xs[c], r1 = xs[K + c], r2 = xs[2 * K + c];
-        const double n = __dsqrt_rn(__dadd_rn(__dadd_rn(__dmul_rn(r0, r0), __dmul_rn(r1, r1)), __dmul_rn(r2, r2)));
-        double *o = rbar_hat + (size_t)s * 3 * (K - 1);
-        o[c] = __ddiv_rn(r0, n);
-        o[(K - 1) + c] = __ddiv_rn(r1, n);
-        o[2 * (K - 1) + c] = __ddiv_rn(r2, n);
-    }
-    if (c < Ku) {   // :132-139  (mask as written: filled where the norm is <= eps, zero elsewhere)
-        const double *us = u + (size_t)s * 3 * Ku;
-        const double u0 = us[c], u1 = us[Ku + c], u2 = us[2 * Ku + c];
-        const double n = __dsqrt_rn(__dadd_rn(__dadd_rn(__dmul_rn(u0, u0), __dmul_rn(u1, u1)), __dmul_rn(u2, u2)));
-        const bool fill = n <= eps;
-        double *o = ubar_hat + (size_t)s * 3 * Ku;
-        o[c] = fill ? __ddiv_rn(u0, n) : 0.0;
-        o[Ku + c] = fill ? __ddiv_rn(u1, n) : 0.0;
-        o[2 * Ku + c] = fill ? __ddiv_rn(u2, n) : 0.0;
-    }
+    if (c < K - 1) rbar_column(xs, K, c, rbar_hat, s);
+    if (c < Ku) ubar_column(u, Ku, c, eps, ubar_hat, s);
     if (c == K - 1) {
         const double r[3] = {xs[K - 1], xs[2 * K - 1], xs[3 * K - 1]};
         const double v[3] = {xs[4 * K - 1], xs[5 * K - 1], xs[6 * K - 1]};
@@ -201,7 +238,6 @@ constraint_terms_kernel(const double *__restrict__ x, const double *__restrict__
         for (int j = 0; j < kFinalTerms; ++j) dst[j] = o[j];
     }
 }
-
 
 // ---------------------------------------------------------------------------------------------------------------
 // Sparse assembly of the dynamics constraint (optimizer.py:327-339) from the SoA discretization result.
@@ -217,22 +253,24 @@ constraint_terms_kernel(const double *__restrict__ x, const double *__restrict__
 //   [ -A[i,0..6] with +1 at x[s,i,k+1] merged in order ] ... see the column list in the kernel.
 // CSR: indptr[r] = 16 r (implicit), indices [rows*16], values [rows*16], rhs [rows].
 // One thread per row; consecutive threads = consecutive k, so the SoA reads are coalesced.
+//
+// RAG: a ragged batch, assembled as N independent single-satellite systems (block-diagonal J), each with its own final
+// time tf_s.  K is the padded stride Kmax of the SoA result (column offset + s (Kmax-1) + k), first[] the prefix sums of
+// K_s - 1 (ragged_locate).  Satellite s's rows start at R_s = 7 first[s], row = R_s + i (K_s-1) + k; its variables at
+// V_s = sum_{r<s} (17 K_r + 1) = 17 (first[s] + s) + s:
+//   x[i,k] -> V_s + i K_s + k | u[j,k] -> V_s + 7K_s + j K_s + k | nu[i,k] -> V_s + 10K_s + i K_s + k | tf_s -> V_s + 17K_s
+// i.e. the rectangular numbering of n_sats = 1, K = K_s shifted by V_s.  One thread per live interval writes its 7 rows
+// (one index search per interval instead of one per row); consecutive threads still walk k, so every SoA read and every
+// row store of a warp covers consecutive columns / rows as in the rectangular kernel.
 constexpr int kJacNnzPerRow = 16;
 
-__global__ void __launch_bounds__(256)
-dynamics_jacobian_kernel(const double *__restrict__ soa, long long pitch, long long offset, int n_sats, int K,
-                         double *__restrict__ values, int64_t *__restrict__ indices, double *__restrict__ rhs)
+// Row r of the system: state row i of interval k, read from SoA column col; x0 / u0 / nu0 / tfc: the columns of x[s,0,0],
+// u[s,0,0], nu[s,i,0] and tf; Kc: nodes of the satellite's grid.
+__device__ __forceinline__ void jacobian_row(const double *__restrict__ soa, long long pitch, long long col, int i, int k,
+                                             int Kc, long long r, long long x0, long long u0, long long nu0, long long tfc,
+                                             double *__restrict__ values, int64_t *__restrict__ indices,
+                                             double *__restrict__ rhs)
 {
-    const long long rows = (long long)n_sats * 7 * (K - 1);
-    const long long r = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (r >= rows) return;
-    const int k = (int)(r % (K - 1));
-    const long long si = r / (K - 1);
-    const int i = (int)(si % 7);
-    const long long s = si / 7;
-    const long long col = offset + s * (K - 1) + k;   // column of this interval in the SoA result
-    const long long NK = (long long)n_sats * K;
-    const long long x0 = s * 7 * K, u0 = 7 * NK + s * 3 * K, nu0 = 10 * NK + (s * 7 + i) * (long long)K, tfc = 17 * NK;
     double *vo = values + r * kJacNnzPerRow;
     int64_t *co = indices ? indices + r * kJacNnzPerRow : nullptr;
     auto put = [&](int pos, double val, long long column) {
@@ -242,16 +280,49 @@ dynamics_jacobian_kernel(const double *__restrict__ soa, long long pitch, long l
     // ascending column order: x[s,0..i,k] | x[s,i,k+1] | x[s,i+1..6,k] | u[s,j,k], u[s,j,k+1] per j | nu | tf
 #pragma unroll
     for (int j = 0; j < 7; ++j)                                                          // -A_k[k,i,j] * x[s,j,k]
-        put(j + (j > i ? 1 : 0), -soa[(long long)(i * 7 + j) * pitch + col], x0 + (long long)j * K + k);
-    put(i + 1, 1.0, x0 + (long long)i * K + k + 1);                                      // +x[s,i,k+1]
+        put(j + (j > i ? 1 : 0), -soa[(long long)(i * 7 + j) * pitch + col], x0 + (long long)j * Kc + k);
+    put(i + 1, 1.0, x0 + (long long)i * Kc + k + 1);                                     // +x[s,i,k+1]
 #pragma unroll
     for (int j = 0; j < 3; ++j) {
-        put(8 + 2 * j, -soa[(long long)(70 + i * 3 + j) * pitch + col], u0 + (long long)j * K + k);       // -B_kn u[s,j,k]
-        put(9 + 2 * j, -soa[(long long)(49 + i * 3 + j) * pitch + col], u0 + (long long)j * K + k + 1);   // -B_kp u[s,j,k+1]
+        put(8 + 2 * j, -soa[(long long)(70 + i * 3 + j) * pitch + col], u0 + (long long)j * Kc + k);       // -B_kn u[s,j,k]
+        put(9 + 2 * j, -soa[(long long)(49 + i * 3 + j) * pitch + col], u0 + (long long)j * Kc + k + 1);   // -B_kp u[s,j,k+1]
     }
     put(14, -1.0, nu0 + k);                                                               // -nu[s,i,k]
     put(15, -soa[(long long)(91 + i) * pitch + col], tfc);                                // -Sigma_k[i,k] * tf
     rhs[r] = soa[(long long)(98 + i) * pitch + col];                     // xi_k[i,k]
+}
+
+template <bool RAG = false>
+__global__ void __launch_bounds__(256)
+dynamics_jacobian_kernel(const double *__restrict__ soa, long long pitch, long long offset, int n_sats, int K,
+                         double *__restrict__ values, int64_t *__restrict__ indices, double *__restrict__ rhs,
+                         const long long *__restrict__ first = nullptr)
+{
+    if (RAG) {
+        const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+        if (t >= first[n_sats] - first[0]) return;
+        int s, k, Ks;
+        ragged_locate(first, n_sats, t, s, k, Ks);
+        const long long f = first[s] - first[0];
+        const long long V = 17 * (f + s) + s;
+        const long long col = offset + (long long)s * (K - 1) + k;
+#pragma unroll
+        for (int i = 0; i < 7; ++i)
+            jacobian_row(soa, pitch, col, i, k, Ks, 7 * f + (long long)i * (Ks - 1) + k, V, V + 7LL * Ks,
+                         V + 10LL * Ks + (long long)i * Ks, V + 17LL * Ks, values, indices, rhs);
+        return;
+    }
+    const long long rows = (long long)n_sats * 7 * (K - 1);
+    const long long r = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (r >= rows) return;
+    const int k = (int)(r % (K - 1));
+    const long long si = r / (K - 1);
+    const int i = (int)(si % 7);
+    const long long s = si / 7;
+    const long long col = offset + s * (K - 1) + k;   // column of this interval in the SoA result
+    const long long NK = (long long)n_sats * K;
+    jacobian_row(soa, pitch, col, i, k, K, r, s * 7 * K, 7 * NK + s * 3 * K, 10 * NK + (s * 7 + i) * (long long)K, 17 * NK,
+                 values, indices, rhs);
 }
 
 }  // namespace mpc

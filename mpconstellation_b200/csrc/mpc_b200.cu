@@ -1912,6 +1912,80 @@ int mpc_dynamics_jacobian(const double *soa, int64_t pitch, int64_t offset, int 
     return MPC_SUCCESS;
 }
 
+// ---- ragged batches (satellite s on K_s nodes, buffers padded to K_max): one launch over the live intervals ----------
+static int cterms_ragged_launch(const double *x, const double *u, int n_sats, int K_max, long long n_live,
+                                const long long *first, double mu, double *rbar, double *ubar, double *fin, cudaStream_t st)
+{
+    const unsigned grid = (unsigned)((n_live + 255) / 256);
+    mpc::constraint_terms_kernel<true><<<grid, 256, 0, st>>>(x, u, n_sats, K_max, K_max, mu, 2.220446049250313e-16, rbar, ubar,
+                                                             fin, first);
+    g_launches.fetch_add(1, std::memory_order_relaxed);
+    CUDA_TRY(cudaGetLastError());
+    return MPC_SUCCESS;
+}
+
+int mpc_constraint_terms_ragged(const double *x, const double *u, int n_sats, int K_max, const int32_t *K_sat, int64_t *first,
+                                double mu, double *rbar_hat, double *ubar_hat, double *final_terms, void *stream)
+{
+    int rc = cterms_check(x, u, n_sats, K_max, K_max, rbar_hat, ubar_hat, final_terms);
+    if (rc || (rc = check_counts(K_sat, n_sats, K_max, "K_sat"))) return rc;
+    if (!first) return fail(MPC_E_INVALID, "null first");
+    if (n_sats == 0) return MPC_SUCCESS;
+    cudaStream_t st = (cudaStream_t)stream;
+    const std::vector<long long> f = ragged_first(K_sat, n_sats);
+    CUDA_TRY(cudaMemcpyAsync(first, f.data(), f.size() * sizeof(long long), cudaMemcpyHostToDevice, st));
+    return cterms_ragged_launch(x, u, n_sats, K_max, f[n_sats], (const long long *)first, mu, rbar_hat, ubar_hat, final_terms, st);
+}
+
+int mpc_constraint_terms_ragged_host(mpc_ctx *ctx, const double *x, const double *u, int n_sats, int K_max,
+                                     const int32_t *K_sat, double mu, double *rbar_hat, double *ubar_hat, double *final_terms)
+{
+    if (!ctx) return fail(MPC_E_INVALID, "null ctx");
+    int rc = cterms_check(x, u, n_sats, K_max, K_max, rbar_hat, ubar_hat, final_terms);
+    if (rc || (rc = check_counts(K_sat, n_sats, K_max, "K_sat")) || n_sats == 0) return rc;
+    CUDA_TRY(cudaSetDevice(ctx->device));
+    const size_t nx = (size_t)n_sats * 7 * K_max, nu = (size_t)n_sats * 3 * K_max, nr = (size_t)n_sats * 3 * (K_max - 1),
+                 nf = (size_t)n_sats * MPC_FINAL_TERMS;
+    const std::vector<long long> f = ragged_first(K_sat, n_sats);
+    if ((rc = ensure(ctx->d_x, ctx->cap_x, nx))) return rc;
+    if ((rc = ensure(ctx->d_u, ctx->cap_u, nu))) return rc;
+    if ((rc = ensure(ctx->d_out, ctx->cap_out, nr + nu + nf))) return rc;
+    if ((rc = ensure(ctx->d_first, ctx->cap_first, f.size()))) return rc;
+    cudaStream_t st = ctx->s_compute;
+    double *d_r = ctx->d_out, *d_ub = d_r + nr, *d_f = d_ub + nu;
+    CUDA_TRY(cudaMemcpyAsync(ctx->d_x, x, nx * sizeof(double), cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(ctx->d_u, u, nu * sizeof(double), cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(ctx->d_first, f.data(), f.size() * sizeof(long long), cudaMemcpyHostToDevice, st));
+    // the kernel leaves the padding columns alone: they go back as NaN (all-ones bytes)
+    CUDA_TRY(cudaMemsetAsync(d_r, 0xFF, (nr + nu) * sizeof(double), st));
+    if ((rc = cterms_ragged_launch(ctx->d_x, ctx->d_u, n_sats, K_max, f[n_sats], ctx->d_first, mu, d_r, d_ub, d_f, st))) return rc;
+    CUDA_TRY(cudaMemcpyAsync(rbar_hat, d_r, nr * sizeof(double), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaMemcpyAsync(ubar_hat, d_ub, nu * sizeof(double), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaMemcpyAsync(final_terms, d_f, nf * sizeof(double), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    return MPC_SUCCESS;
+}
+
+int mpc_dynamics_jacobian_ragged(const double *soa, int64_t pitch, int64_t offset, int n_sats, int K_max,
+                                 const int32_t *K_sat, int64_t *first, double *values, int64_t *indices, double *rhs,
+                                 void *stream)
+{
+    if (!soa || !values || !rhs || !first) return fail(MPC_E_INVALID, "null pointer argument");
+    if (n_sats < 0 || K_max < 2) return fail(MPC_E_INVALID, "need n_sats >= 0, K_max >= 2 (got %d, %d)", n_sats, K_max);
+    if (pitch < offset + (long long)n_sats * (K_max - 1) || offset < 0) return fail(MPC_E_INVALID, "pitch/offset do not hold the batch");
+    int rc = check_counts(K_sat, n_sats, K_max, "K_sat");
+    if (rc || n_sats == 0) return rc;
+    cudaStream_t st = (cudaStream_t)stream;
+    const std::vector<long long> f = ragged_first(K_sat, n_sats);
+    CUDA_TRY(cudaMemcpyAsync(first, f.data(), f.size() * sizeof(long long), cudaMemcpyHostToDevice, st));
+    const unsigned grid = (unsigned)((f[n_sats] + 255) / 256);
+    mpc::dynamics_jacobian_kernel<true><<<grid, 256, 0, st>>>(soa, pitch, offset, n_sats, K_max, values, indices, rhs,
+                                                              (const long long *)first);
+    g_launches.fetch_add(1, std::memory_order_relaxed);
+    CUDA_TRY(cudaGetLastError());
+    return MPC_SUCCESS;
+}
+
 int mpc_fp64_peak_probe(int device, int repeats, double *tflops, double *ms)
 {
     if (!tflops) return fail(MPC_E_INVALID, "null output");
