@@ -472,6 +472,79 @@ int mpc_dynamics_jacobian_ragged(const double *soa, int64_t pitch, int64_t offse
                                  const int32_t *K_sat, int64_t *first, double *values, int64_t *indices, double *rhs,
                                  void *stream);
 
+/* ---------------------------------------------------------------- per-satellite designer units */
+
+/*
+ * The per-scale fields of one satellite's normalized Constants (SatelliteScale.get_normalized_constants of THAT
+ * satellite, satellite_scale.py:36-44): what the kernels read.  A constellation that mixes altitudes and masses is
+ * linearized satellite by satellite in these units, as N separate controllers of the reference do (control.py:164,187).
+ * Everything else stays launch-wide in mpc_params: include_j2, include_drag, c_d, rho_atm (its mu .. rho are not read).
+ */
+typedef struct mpc_sat_consts {
+    double mu, r_e, j2, g0, isp, s_area, rho;
+} mpc_sat_consts;
+
+/* doubles of device scratch per satellite the *_units device entry points fill with the derived kernel constants */
+#define MPC_SAT_SCRATCH_DOUBLES 8
+
+/*
+ * *_units: the computation of the single-constant entry point for every satellite s in the units of consts[s], one
+ * launch for the batch; satellite s comes out bit for bit as a launch of the same kernel under consts[s] alone.
+ *   consts          HOST array [n_sats], validated (every value finite, mu > 0, g0 * isp > 0; otherwise MPC_E_INVALID
+ *                   naming the satellite).  The kernel constants are derived on the host with the expressions of the
+ *                   single-constant path and copied (cudaMemcpyAsync on `stream`) into
+ *   consts_scratch  DEVICE scratch of n_sats * MPC_SAT_SCRATCH_DOUBLES doubles, which the call fills.
+ * Not available (MPC_E_UNSUPPORTED): the drag linearisation (include_drag in the discretization), the fixed-step RK4
+ * propagator, u on its own grid, the round-1 default-mode kernel (mpc_set_tuning(9)), the fused overlapped pass and the
+ * multi-GPU gather entry points.
+ *
+ * mpc_discretize_batch_units: mpc_discretize_batch_ragged with per-satellite constants; K_sat == NULL means a rectangular
+ * batch (K = K_max nodes for every satellite; `first` is then not used and may be NULL).  The fixed-step form always
+ * takes the two-node-step kernel (small batches in one-warp CTAs, no thread-group kernel), in its ragged form: a
+ * rectangular batch runs as one with K_max nodes everywhere, its prefix sums written into consts_scratch.
+ */
+int mpc_discretize_batch_units(const double *x, const double *u, const double *tf, const mpc_params *p,
+                               const mpc_sat_consts *consts, int n_sats, int K_max, const int32_t *K_sat, int64_t *first,
+                               double *consts_scratch, int adaptive, int n_sub, double rtol, double atol, double max_step,
+                               double *out, int64_t out_pitch, int64_t out_offset, int32_t *status, int32_t *n_nodes,
+                               void *stream);
+/* Host-buffer form (context-owned scratch): as mpc_discretize_batch_ragged_host, K_sat == NULL: rectangular. */
+int mpc_discretize_batch_units_host(mpc_ctx *ctx, const double *x, const double *u, const double *tf, const mpc_params *p,
+                                    const mpc_sat_consts *consts, int n_sats, int K_max, const int32_t *K_sat, int adaptive,
+                                    int n_sub, double rtol, double atol, double max_step, double *out_host,
+                                    int32_t *status_host, int32_t *n_nodes_host);
+
+/*
+ * mpc_propagate_batch_rk45_units: mpc_propagate_batch_rk45_ragged with per-satellite constants (mu, kj2, 1/(g0 isp) and,
+ * with include_drag, the drag coefficient 0.5 c_d s_area rho_atm / rho of each satellite).  T_sat == NULL (and
+ * table_len_sat == NULL): every satellite on T_max samples, the rectangular run.  T_sat / table_len_sat are DEVICE
+ * arrays as in the ragged entry point.
+ */
+int mpc_propagate_batch_rk45_units(const double *y0, const double *tf, const mpc_params *p, const mpc_sat_consts *consts,
+                                   const mpc_controller *ctrl, int n_sats, int T_max, const int32_t *T_sat,
+                                   const int32_t *table_len_sat, double *consts_scratch, double rtol, double atol,
+                                   double max_step, double *y, double *u_out, int32_t *status, int32_t *n_steps,
+                                   void *stream);
+/* Host-buffer form: T_sat / table_len_sat are host arrays or NULL, as in mpc_propagate_batch_rk45_ragged_host. */
+int mpc_propagate_batch_rk45_units_host(mpc_ctx *ctx, const double *y0, const double *tf, const mpc_params *p,
+                                        const mpc_sat_consts *consts, const mpc_controller *ctrl, int n_sats, int T_max,
+                                        const int32_t *T_sat, const int32_t *table_len_sat, double rtol, double atol,
+                                        double max_step, double *y_host, double *u_host, int32_t *status_host,
+                                        int32_t *n_steps_host);
+
+/*
+ * mpc_constraint_terms_units: the terminal terms of satellite s with consts[s].mu (the only constant the constraint terms
+ * read).  K_sat == NULL: rectangular, u on the nodes of x (u_cols = K_max; `first` may be NULL); otherwise as
+ * mpc_constraint_terms_ragged (K_sat a host array, `first` its device scratch).
+ */
+int mpc_constraint_terms_units(const double *x, const double *u, int n_sats, int K_max, const int32_t *K_sat, int64_t *first,
+                               const mpc_sat_consts *consts, double *consts_scratch, double *rbar_hat, double *ubar_hat,
+                               double *final_terms, void *stream);
+/* Host-buffer form; the padding columns of a ragged batch come back NaN. */
+int mpc_constraint_terms_units_host(mpc_ctx *ctx, const double *x, const double *u, int n_sats, int K_max,
+                                    const int32_t *K_sat, const mpc_sat_consts *consts, double *rbar_hat, double *ubar_hat,
+                                    double *final_terms);
+
 /* ---------------------------------------------------------------- measurement helpers */
 
 /* FP64 FMA-chain microbenchmark: measured DFMA peak of `device` in TFLOP/s (2 flop per FMA). */

@@ -14,8 +14,9 @@ import numpy as np
 _HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(_HERE, "csrc")
 SO_PATH = os.path.join(CSRC, "libmpc_b200.so")
-SOURCES = ["mpc_b200.cu", "mpc_b200_drag.cu"]    # the drag-branch kernels have a translation unit of their own
-HEADERS = ["discretize_kernel.cuh", "discretize_adaptive_kernel.cuh", "discretize_default_kernel.cuh", "propagate_kernel.cuh", "propagate_rk45_kernel.cuh", "discretize_group_kernel.cuh", "constraint_terms_kernel.cuh", "discretize_drag_kernel.cuh", "discretize_pair_kernel.cuh", "mpc_b200_drag.h", os.path.join("..", "..", "include", "mpc_b200.h")]
+# the drag-branch kernels and the per-satellite-constants kernels have a translation unit each
+SOURCES = ["mpc_b200.cu", "mpc_b200_drag.cu", "mpc_b200_units.cu"]
+HEADERS = ["discretize_kernel.cuh", "discretize_adaptive_kernel.cuh", "discretize_default_kernel.cuh", "propagate_kernel.cuh", "propagate_rk45_kernel.cuh", "discretize_group_kernel.cuh", "constraint_terms_kernel.cuh", "discretize_drag_kernel.cuh", "discretize_pair_kernel.cuh", "mpc_b200_drag.h", "mpc_b200_units.h", os.path.join("..", "..", "include", "mpc_b200.h")]
 # No -split-compile: with it nvcc partitions the module for parallel compilation and the register allocation of the
 # 250-register kernels comes out differently from build to build (the same source gave discretize_default_kernel 253
 # registers / 296 B of stack in one build and 255 / 536 B in the next: 1.366 vs 1.390 ms on BASELINE configs[2];
@@ -46,6 +47,14 @@ class MpcParams(ctypes.Structure):
 
 
 RHO_CHEB = 32
+
+
+class MpcSatConsts(ctypes.Structure):
+    """mpc_sat_consts: the per-scale fields of one satellite's normalized Constants"""
+    _fields_ = [(n, ctypes.c_double) for n in ("mu", "r_e", "j2", "g0", "isp", "s_area", "rho")]
+
+
+SAT_SCRATCH_DOUBLES = 8    # MPC_SAT_SCRATCH_DOUBLES
 
 
 class MpcController(ctypes.Structure):
@@ -160,6 +169,12 @@ def lib():
     L.mpc_constraint_terms_ragged.argtypes = [_DP, _DP, i, i, _DP, _DP, d, _DP, _DP, _DP, vp]
     L.mpc_constraint_terms_ragged_host.argtypes = [vp, _DP, _DP, i, i, _DP, d, _DP, _DP, _DP]
     L.mpc_dynamics_jacobian_ragged.argtypes = [_DP, i64, i64, i, i, _DP, _DP, _DP, _DP, _DP, vp]
+    L.mpc_discretize_batch_units.argtypes = [_DP, _DP, _DP, pp, _DP, i, i, _DP, _DP, _DP, i, i, d, d, d, _DP, i64, i64, _DP, _DP, vp]
+    L.mpc_discretize_batch_units_host.argtypes = [vp, _DP, _DP, _DP, pp, _DP, i, i, _DP, i, i, d, d, d, _DP, _DP, _DP]
+    L.mpc_propagate_batch_rk45_units.argtypes = [_DP, _DP, pp, _DP, pc, i, i, _DP, _DP, _DP, d, d, d, _DP, _DP, _DP, _DP, vp]
+    L.mpc_propagate_batch_rk45_units_host.argtypes = [vp, _DP, _DP, pp, _DP, pc, i, i, _DP, _DP, d, d, d, _DP, _DP, _DP, _DP]
+    L.mpc_constraint_terms_units.argtypes = [_DP, _DP, i, i, _DP, _DP, _DP, _DP, _DP, _DP, _DP, vp]
+    L.mpc_constraint_terms_units_host.argtypes = [vp, _DP, _DP, i, i, _DP, _DP, _DP, _DP, _DP]
     L.mpc_fp64_peak_probe.argtypes = [i, i, ctypes.POINTER(ctypes.c_double), ctypes.POINTER(ctypes.c_double)]
     L.mpc_set_gather_tuning.argtypes = [i, i]
     L.mpc_set_gather_tuning.restype = i
@@ -171,7 +186,9 @@ def lib():
                  "mpc_ctx_create", "mpc_ctx_destroy", "mpc_discretize_batch_host", "mpc_propagate_batch_host",
                  "mpc_propagate_discretize_host", "mpc_propagate_discretize", "mpc_propagate_discretize_multi", "mpc_fp64_peak_probe", "mpc_constraint_terms",
                  "mpc_constraint_terms_host", "mpc_discretize_batch_push", "mpc_fill_const_rows", "mpc_dynamics_jacobian",
-                 "mpc_constraint_terms_ragged", "mpc_constraint_terms_ragged_host", "mpc_dynamics_jacobian_ragged"):
+                 "mpc_constraint_terms_ragged", "mpc_constraint_terms_ragged_host", "mpc_dynamics_jacobian_ragged",
+                 "mpc_discretize_batch_units", "mpc_discretize_batch_units_host", "mpc_propagate_batch_rk45_units",
+                 "mpc_propagate_batch_rk45_units_host", "mpc_constraint_terms_units", "mpc_constraint_terms_units_host"):
         getattr(L, name).restype = i
     _lib = L
     return L
@@ -189,8 +206,37 @@ EXPORTED_SYMBOLS = [
     "mpc_constraint_terms", "mpc_constraint_terms_host", "mpc_discretize_batch_push", "mpc_fill_const_rows",
     "mpc_dynamics_jacobian",
     "mpc_constraint_terms_ragged", "mpc_constraint_terms_ragged_host", "mpc_dynamics_jacobian_ragged",
+    "mpc_discretize_batch_units", "mpc_discretize_batch_units_host", "mpc_propagate_batch_rk45_units",
+    "mpc_propagate_batch_rk45_units_host", "mpc_constraint_terms_units", "mpc_constraint_terms_units_host",
     "mpc_fp64_peak_probe", "mpc_set_tuning", "mpc_set_gather_tuning",
 ]
+
+
+SAT_CONST_FIELDS = ("MU", "R_E", "J2", "G0", "ISP", "S", "RHO")   # what mpc_sat_consts carries, in its order
+
+
+def sat_consts(const, n):
+    """const: one Constants bag or a sequence of n of them -> (None, one bag) when every satellite has the same seven
+    per-scale values bit for bit (the single-constant launches apply), else (mpc_sat_consts [n], None).  A length other
+    than n, or a bag without one of the seven attributes, raises ValueError."""
+    if hasattr(const, "MU"):             # one bag
+        return None, const
+    try:
+        const = list(const)              # any sequence of bags: list, tuple, numpy object array, ...
+    except TypeError:
+        raise ValueError(f"const must be a Constants bag or a sequence of {n} of them, got {type(const).__name__}") from None
+    if len(const) != n:
+        raise ValueError(f"per-satellite constants: expected {n} Constants, got {len(const)}")
+    rows = []
+    for s, c in enumerate(const):
+        try:
+            rows.append([float(getattr(c, f)) for f in SAT_CONST_FIELDS])
+        except AttributeError as e:
+            raise ValueError(f"per-satellite constants: const[{s}] has no attribute {e.name!r}") from None
+    vals = np.array(rows, dtype=np.float64).reshape(n, 7)
+    if n == 0 or (vals.view(np.uint64) == vals[0].view(np.uint64)).all():
+        return None, (const[0] if n else None)
+    return (MpcSatConsts * n).from_buffer_copy(np.ascontiguousarray(vals)), None
 
 
 def check(rc):

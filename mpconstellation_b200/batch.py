@@ -135,6 +135,11 @@ def discretize_batch(x, u, tf, const, include_J2=False, include_drag=False, n_su
     K_s <= x.shape[2] nodes (the first K_s columns of x[s], u[s]), one launch for all; the result keeps the layout of
     Kmax = x.shape[2] with NaN in the padding columns (DiscretizedBatch.sat(s) returns K_s - 1 intervals).  u must be on
     the nodes of x, and the drag linearisation is not available for ragged batches.
+
+    const: one Constants bag, or a sequence of N -- satellite s linearized in the units of its own scale (model.
+    sat_units), one launch for the batch, as N single-satellite calls would give it.  N bags that agree bit for bit in
+    the seven per-scale fields take the single-constant launches.  Per-satellite constants need u on the nodes of x and
+    are not available with include_drag.
     """
     ctx = _ctx(device)
     counts, K = K, None
@@ -154,6 +159,7 @@ def discretize_batch(x, u, tf, const, include_J2=False, include_drag=False, n_su
         raise ValueError("out must be C-contiguous float64 [105, N*(K-1)]")
     if status is None:
         status = np.zeros(n_int, dtype=np.int32)
+    psc, const = _units_of(const, N, Ku != K, include_drag)
     p = _lib.make_params(const, include_J2, include_drag, disc_drag=disc_drag)
     n_nodes = None
     K_sat = None
@@ -162,7 +168,14 @@ def discretize_batch(x, u, tf, const, include_J2=False, include_drag=False, n_su
         if Ku != K:
             raise ValueError("a ragged batch needs u on the nodes of x ([N,3,Kmax])")
     with _lock(device):
-        if K_sat is not None:
+        if psc is not None:
+            ad = adaptive or {}
+            n_nodes = np.zeros(n_int, dtype=np.int32) if adaptive is not None else None
+            _lib.check(_lib.lib().mpc_discretize_batch_units_host(
+                ctx, _lib.addr(x), _lib.addr(u), _lib.addr(tfv), ctypes.byref(p), psc, N, K, _lib.addr(K_sat),
+                int(adaptive is not None), int(n_sub), float(ad.get("rtol", 1e-3)), float(ad.get("atol", 1e-6)),
+                float(ad.get("max_step", 1e-2)), _lib.addr(out), _lib.addr(status), _lib.addr(n_nodes)))
+        elif K_sat is not None:
             ad = adaptive or {}
             n_nodes = np.zeros(n_int, dtype=np.int32) if adaptive is not None else None
             _lib.check(_lib.lib().mpc_discretize_batch_ragged_host(
@@ -191,6 +204,25 @@ def discretize_batch(x, u, tf, const, include_J2=False, include_drag=False, n_su
     if check:
         res.raise_on_error()
     return res
+
+
+def _units_of(const, n, ugrid=False, drag=False):
+    """(mpc_sat_consts [n] or None, the bag for mpc_params): see _lib.sat_consts; rejects what has no per-satellite form"""
+    psc, one = _lib.sat_consts(const, n)
+    if psc is None:
+        return None, one
+    if ugrid:
+        raise ValueError("per-satellite constants need u on the nodes of x (no u on its own grid)")
+    if drag:
+        raise ValueError("the drag linearisation (include_drag=True) is not available with per-satellite constants")
+    return psc, list(const)[0]
+
+
+def _rk4_units(const, n, n_sub):
+    """per-satellite constants need the reference integrator: raise before any device work when n_sub asks for RK4"""
+    if n_sub not in (None, 0) and _lib.sat_consts(const, n)[0] is not None:
+        raise ValueError("per-satellite constants need the reference integrator (n_sub=None); the fixed-step RK4 "
+                         "propagator has no per-satellite form")
 
 
 def _ctrl_struct(spec, n_sats, table_addr=None, end_tau_addr=None):
@@ -246,12 +278,16 @@ def propagate_batch(y0, tf, controller, const, include_drag=True, include_J2=Tru
     controller exactly as simulator.py:185-187 calls it (max_step=0.001, rtol 1e-3, atol 1e-6, dense-output samples);
     `rk45=dict(rtol=, atol=, max_step=)` overrides those numbers, `n_steps` (int32 [N]) receives the steps attempted.
     n_sub >= 1: fixed-step RK4 with n_sub steps between samples (default_n_sub(T) mirrors max_step=0.001).
+
+    const: one Constants bag, or a sequence of N (satellite s integrated in the units of its own scale, one launch; N bags
+    that agree bit for bit take the single-constant launch).  Per-satellite constants need the reference integrator.
     """
-    ctx = _ctx(device)
     y0 = _f64(y0)
     if y0.ndim != 2 or y0.shape[1] != 7:
         raise ValueError(f"y0 must be [N,7], got {y0.shape}")
     N = y0.shape[0]
+    _rk4_units(const, N, n_sub)
+    ctx = _ctx(device)
     spec = spec_from(controller)
     T_sat = tab_len = None
     if spec.kind == _lib.CTRL_SEQUENCE and spec.table_len is not None:
@@ -278,6 +314,7 @@ def propagate_batch(y0, tf, controller, const, include_drag=True, include_J2=Tru
             t[s_, :ts] = np.linspace(0, 1, ts)
     if N == 0 or T == 0:
         return y, uo, t, status
+    psc, const = _units_of(const, N)
     p = _lib.make_params(const, include_J2, include_drag)
     c, _keep = _ctrl_struct(spec, N)
     if n_sub == 0:
@@ -285,7 +322,12 @@ def propagate_batch(y0, tf, controller, const, include_drag=True, include_J2=Tru
         if n_steps is not None and (n_steps.shape != (N,) or n_steps.dtype != np.int32):
             raise ValueError("n_steps must be int32 [N]")
         with _lock(device):
-            if T_sat is not None or tab_len is not None:
+            if psc is not None:
+                _lib.check(_lib.lib().mpc_propagate_batch_rk45_units_host(
+                    ctx, _lib.addr(y0), _lib.addr(tfv), ctypes.byref(p), psc, ctypes.byref(c), N, T, _lib.addr(T_sat),
+                    _lib.addr(tab_len), float(o.get("rtol", 1e-3)), float(o.get("atol", 1e-6)), float(o.get("max_step", 1e-3)),
+                    _lib.addr(y), _lib.addr(uo), _lib.addr(status), _lib.addr(n_steps)))
+            elif T_sat is not None or tab_len is not None:
                 counts = T_sat if T_sat is not None else np.full(N, T, dtype=np.int32)
                 _lib.check(_lib.lib().mpc_propagate_batch_rk45_ragged_host(
                     ctx, _lib.addr(y0), _lib.addr(tfv), ctypes.byref(p), ctypes.byref(c), N, T, _lib.addr(counts),
@@ -362,7 +404,8 @@ def discretize_batch_device(x, u, tf, const, include_J2=False, n_sub=100, out=No
     further [105, pitch] buffers (e.g. peer-mapped) every result is also stored to (total 1,2,4 or 8).
     K = int array [N] (host): a ragged batch as in discretize_batch (x, u [N,.,Kmax]); `first` is an int64 CUDA tensor
     [N+1] the call fills with the prefix sums of K_s - 1 (allocated when None).  The padding columns of `out` are not
-    written; status (zeroed when allocated here) and n_nodes keep the [N*(Kmax-1)] layout."""
+    written; status (zeroed when allocated here) and n_nodes keep the [N*(Kmax-1)] layout.
+    const: one Constants bag or a sequence of N, as in discretize_batch (no extra_dst with per-satellite constants)."""
     torch = _torch()
     N, _, K_ = x.shape
     n_int = N * (K_ - 1)
@@ -380,10 +423,22 @@ def discretize_batch_device(x, u, tf, const, include_J2=False, n_sub=100, out=No
     pitch = out.shape[1] if out_pitch is None else int(out_pitch)
     if status is None:
         status = (torch.zeros if K_sat is not None else torch.empty)(n_int, dtype=torch.int32, device=x.device)
+    psc, const = _units_of(const, N)
+    if psc is not None and extra_dst:
+        raise ValueError("per-satellite constants have one destination")
     p = _lib.make_params(const, include_J2, False)
     stream = torch.cuda.current_stream(x.device).cuda_stream
     L = _lib.lib()
-    if K_sat is not None:
+    if psc is not None:
+        ad = adaptive or {}
+        scratch = torch.empty(N * _lib.SAT_SCRATCH_DOUBLES, dtype=torch.float64, device=x.device)
+        _lib.check(L.mpc_discretize_batch_units(
+            x.data_ptr(), u.data_ptr(), tf.data_ptr(), ctypes.byref(p), psc, N, K_, _lib.addr(K_sat),
+            first.data_ptr() if first is not None else None, scratch.data_ptr(), int(adaptive is not None), int(n_sub),
+            float(ad.get("rtol", 1e-3)), float(ad.get("atol", 1e-6)), float(ad.get("max_step", 1e-2)), out.data_ptr(), pitch,
+            int(out_offset), status.data_ptr(), n_nodes.data_ptr() if n_nodes is not None else None, stream))
+        scratch.record_stream(torch.cuda.current_stream(x.device))
+    elif K_sat is not None:
         ad = adaptive or {}
         _lib.check(L.mpc_discretize_batch_ragged(
             x.data_ptr(), u.data_ptr(), tf.data_ptr(), ctypes.byref(p), N, K_, _lib.addr(K_sat), first.data_ptr(),
@@ -413,9 +468,11 @@ def propagate_batch_device(y0, tf, controller, const, include_drag=True, include
     """Device form of propagate_batch: y0 [N,7], tf [N] float64 CUDA tensors -> y [N,7,T], u [N,3,T], status [N].
     T = int array [N] (host): satellite s sampled at linspace(0, 1, T_s) into the first T_s columns of y / u [.,.,Tmax]
     (the padding columns are not written), the reference integrator only, as propagate_batch; so is a sequence law
-    with per-satellite table lengths (ControllerSpec.table_len)."""
+    with per-satellite table lengths (ControllerSpec.table_len).
+    const: one Constants bag or a sequence of N, as in propagate_batch."""
     torch = _torch()
     N = y0.shape[0]
+    _rk4_units(const, N, n_sub)
     spec = spec_from(controller)
     T_sat = tab_len = None
     if spec.kind == _lib.CTRL_SEQUENCE and spec.table_len is not None:
@@ -441,9 +498,19 @@ def propagate_batch_device(y0, tf, controller, const, include_drag=True, include
             et_dev = torch.as_tensor(np.asarray(spec.end_tau, dtype=np.float64)).to(y0.device).contiguous()
     c, _keep = _ctrl_struct(spec, N, table_addr=tab_dev.data_ptr() if tab_dev is not None else None,
                             end_tau_addr=et_dev.data_ptr() if et_dev is not None else None)
+    psc, const = _units_of(const, N)
     p = _lib.make_params(const, include_J2, include_drag)
     stream = torch.cuda.current_stream(y0.device).cuda_stream
-    if T_sat is not None or tab_len is not None:
+    if psc is not None:
+        cnt_dev = torch.as_tensor(T_sat).to(y0.device) if T_sat is not None else None
+        len_dev = torch.as_tensor(tab_len).to(y0.device) if tab_len is not None else None
+        scratch = torch.empty(N * _lib.SAT_SCRATCH_DOUBLES, dtype=torch.float64, device=y0.device)
+        _lib.check(_lib.lib().mpc_propagate_batch_rk45_units(
+            y0.data_ptr(), tf.data_ptr(), ctypes.byref(p), psc, ctypes.byref(c), N, T,
+            cnt_dev.data_ptr() if cnt_dev is not None else None, len_dev.data_ptr() if len_dev is not None else None,
+            scratch.data_ptr(), 1e-3, 1e-6, 1e-3, y.data_ptr(), u_out.data_ptr(), status.data_ptr(), None, stream))
+        scratch.record_stream(torch.cuda.current_stream(y0.device))
+    elif T_sat is not None or tab_len is not None:
         # the ragged entry point reads the counts on the device
         cnt_dev = torch.as_tensor(T_sat if T_sat is not None else np.full(N, T, dtype=np.int32)).to(y0.device)
         len_dev = torch.as_tensor(tab_len).to(y0.device) if tab_len is not None else None

@@ -30,7 +30,10 @@ def constraint_terms_batch(x, u, const, device=0, K=None):
 
     K = int array [N]: a ragged batch (Linearization.K) -- satellite s on its own K_s <= x.shape[2] nodes (the first K_s
     columns of x[s], u[s]; u must be on the nodes of x), one launch for all.  rbar_hat / ubar_hat keep the padded shapes
-    with NaN past K_s - 1 / K_s, and the terminal terms come from node K_s - 1."""
+    with NaN past K_s - 1 / K_s, and the terminal terms come from node K_s - 1.
+
+    const: one Constants bag, or a sequence of N (satellite s in the units of its own scale; the terminal terms read its
+    MU).  N bags that agree bit for bit take the single-constant launch; otherwise u must be on the nodes of x."""
     ctx = _ctx(device)
     x = _f64(x)
     u = _f64(u)
@@ -45,11 +48,17 @@ def constraint_terms_batch(x, u, const, device=0, K=None):
         K_sat = _counts(K, N, Kx, "K")
         if Ku != Kx:
             raise ValueError("a ragged batch needs u on the nodes of x ([N,3,Kmax])")
+    psc, const = _lib.sat_consts(const, N)
+    if psc is not None and Ku != Kx:
+        raise ValueError("per-satellite constants need u on the nodes of x ([N,3,K])")
     rbar = np.empty((N, 3, Kx - 1))
     ubar = np.empty((N, 3, Ku))
     fin = np.empty((N, _lib.FINAL_TERMS))
     with _lock(device):
-        if K_sat is not None:
+        if psc is not None:
+            _lib.check(_lib.lib().mpc_constraint_terms_units_host(ctx, _lib.addr(x), _lib.addr(u), N, Kx, _lib.addr(K_sat), psc,
+                                                                  _lib.addr(rbar), _lib.addr(ubar), _lib.addr(fin)))
+        elif K_sat is not None:
             _lib.check(_lib.lib().mpc_constraint_terms_ragged_host(ctx, _lib.addr(x), _lib.addr(u), N, Kx, _lib.addr(K_sat),
                                                                    float(const.MU), _lib.addr(rbar), _lib.addr(ubar),
                                                                    _lib.addr(fin)))
@@ -65,7 +74,8 @@ def constraint_terms_device(x, u, const, rbar_hat=None, ubar_hat=None, final_ter
     """Device form: x [N,7,K], u [N,3,Ku] float64 CUDA tensors; enqueued on torch's current stream.
     Returns (rbar_hat [N,3,K-1], ubar_hat [N,3,Ku], final_terms [N,32]).
     K = int array [N] (host): a ragged batch as in constraint_terms_batch; `first` is an int64 CUDA tensor [N+1] the call
-    fills with the prefix sums of K_s - 1 (allocated when None).  The padding columns of the outputs are not written."""
+    fills with the prefix sums of K_s - 1 (allocated when None).  The padding columns of the outputs are not written.
+    const: one Constants bag or a sequence of N, as in constraint_terms_batch."""
     import torch
     N, _, Kx = x.shape
     Ku = u.shape[2]
@@ -75,8 +85,11 @@ def constraint_terms_device(x, u, const, rbar_hat=None, ubar_hat=None, final_ter
         K_sat = _counts(K, N, Kx, "K")
         if Ku != Kx:
             raise ValueError("a ragged batch needs u on the nodes of x ([N,3,Kmax])")
-        if first is None:
-            first = torch.empty(N + 1, dtype=torch.int64, device=x.device)
+    psc, const = _lib.sat_consts(const, N)
+    if psc is not None and Ku != Kx:
+        raise ValueError("per-satellite constants need u on the nodes of x ([N,3,K])")
+    if K_sat is not None and first is None:
+        first = torch.empty(N + 1, dtype=torch.int64, device=x.device)
     if rbar_hat is None:
         rbar_hat = torch.empty((N, 3, Kx - 1), dtype=torch.float64, device=x.device)
     if ubar_hat is None:
@@ -84,7 +97,14 @@ def constraint_terms_device(x, u, const, rbar_hat=None, ubar_hat=None, final_ter
     if final_terms is None:
         final_terms = torch.empty((N, _lib.FINAL_TERMS), dtype=torch.float64, device=x.device)
     stream = torch.cuda.current_stream(x.device).cuda_stream
-    if K_sat is not None:
+    if psc is not None:
+        scratch = torch.empty(N * _lib.SAT_SCRATCH_DOUBLES, dtype=torch.float64, device=x.device)
+        _lib.check(_lib.lib().mpc_constraint_terms_units(x.data_ptr(), u.data_ptr(), N, Kx, _lib.addr(K_sat),
+                                                         first.data_ptr() if first is not None else None, psc,
+                                                         scratch.data_ptr(), rbar_hat.data_ptr(), ubar_hat.data_ptr(),
+                                                         final_terms.data_ptr(), stream))
+        scratch.record_stream(torch.cuda.current_stream(x.device))
+    elif K_sat is not None:
         _lib.check(_lib.lib().mpc_constraint_terms_ragged(x.data_ptr(), u.data_ptr(), N, Kx, _lib.addr(K_sat),
                                                           first.data_ptr(), float(const.MU), rbar_hat.data_ptr(),
                                                           ubar_hat.data_ptr(), final_terms.data_ptr(), stream))

@@ -239,6 +239,40 @@ constraint_terms_kernel(const double *__restrict__ x, const double *__restrict__
     }
 }
 
+// Per-satellite constants (mpc_constraint_terms_units): constraint_terms_kernel with satellite s's MU read from mu_sat[s],
+// rectangular (first == nullptr, u on the nodes of x: Ku = K) or ragged.  A kernel of its own rather than a template flag
+// on the one above, whose instantiations keep their names and code.
+template <bool RAG>
+__global__ void __launch_bounds__(256)
+constraint_terms_units_kernel(const double *__restrict__ x, const double *__restrict__ u, int n_sats, int K,
+                              const double *__restrict__ mu_sat, double eps, double *__restrict__ rbar_hat,
+                              double *__restrict__ ubar_hat, double *__restrict__ fin, const long long *__restrict__ first)
+{
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    int s, c, Ks = K;             // c: interval (ragged) or column (rectangular)
+    if (RAG) {
+        if (i >= first[n_sats] - first[0]) return;
+        ragged_locate(first, n_sats, i, s, c, Ks);
+    } else {
+        if (i >= (long long)n_sats * K) return;
+        s = (int)(i / K);
+        c = (int)(i % K);
+    }
+    const double *xs = x + (size_t)s * 7 * K;
+    if (c < Ks - 1) rbar_column(xs, K, c, rbar_hat, s);
+    ubar_column(u, K, c, eps, ubar_hat, s);
+    if (c == Ks - 1 || (RAG && c == Ks - 2)) {
+        if (RAG) ubar_column(u, K, Ks - 1, eps, ubar_hat, s);
+        const double r[3] = {xs[Ks - 1], xs[K + Ks - 1], xs[2 * K + Ks - 1]};
+        const double v[3] = {xs[3 * K + Ks - 1], xs[4 * K + Ks - 1], xs[5 * K + Ks - 1]};
+        double o[kFinalTerms];
+        terminal_terms(r, v, mu_sat[s], o);
+        double *dst = fin + (size_t)s * kFinalTerms;
+#pragma unroll
+        for (int j = 0; j < kFinalTerms; ++j) dst[j] = o[j];
+    }
+}
+
 // ---------------------------------------------------------------------------------------------------------------
 // Sparse assembly of the dynamics constraint (optimizer.py:327-339) from the SoA discretization result.
 //

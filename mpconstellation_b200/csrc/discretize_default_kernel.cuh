@@ -92,12 +92,16 @@ __device__ __forceinline__ void df_store_stage(volatile double *sm, int s, const
 
 // RAG: a ragged batch (discretize_default_ragged_kernel): K is the padded stride Kmax, first[] the prefix sums of K_s - 1
 // (ragged_locate); threads map to live intervals only, gid below is the interval's output column s (Kmax-1) + k.
-template <bool J2, int BLOCK, bool GENU, bool DRAG, bool RAG = false>
+// PSC: per-satellite constants (discretize_default_units_kernel): the thread of satellite `sat` reads psc[sat] where the
+// others read P.  The table is read where the constants are used, inside the step loop (it is not __restrict__: the
+// stores to the output buffer keep the loads where they are), so that this 254-register body keeps no more values live.
+template <bool J2, int BLOCK, bool GENU, bool DRAG, bool RAG = false, bool PSC = false>
 __device__ __forceinline__ void
 discretize_default_body(const double *__restrict__ x_in, const double *__restrict__ u_in,
-                        const double *__restrict__ tf_arr, const DiscParams &P, int n_sats, int K, int Ku, double rtol, double atol,
+                        const double *__restrict__ tf_arr, const DiscParams &P0, int n_sats, int K, int Ku, double rtol, double atol,
                         double max_step, const DstTab &dst, long long pitch, long long offset, int32_t *__restrict__ status,
-                        int32_t *__restrict__ n_nodes, double kf, const DragLin *L, const long long *__restrict__ first = nullptr)
+                        int32_t *__restrict__ n_nodes, double kf, const DragLin *L, const long long *__restrict__ first = nullptr,
+                        const DiscParams *psc = nullptr)
 {
     constexpr int kStage = DRAG ? 18 : 9;
     extern __shared__ double acc_smem[];
@@ -115,6 +119,7 @@ discretize_default_body(const double *__restrict__ x_in, const double *__restric
         sat = (int)(gid / (K - 1));
         k = (int)(gid - (long long)sat * (K - 1));
     }
+    const DiscParams &P = PSC ? psc[sat] : P0;
     volatile double *sm = acc_smem + threadIdx.x;
     const double tf = tf_arr[sat];
     const double *xs = x_in + ((long long)sat * 7) * K + k;
@@ -508,6 +513,19 @@ discretize_default_ragged_kernel(const double *__restrict__ x_in, const double *
 {
     discretize_default_body<J2, BLOCK, false, false, true>(x_in, u_in, tf_arr, P, n_sats, K, K, rtol, atol, max_step, dst, pitch,
                                                            offset, status, n_nodes, 0.0, nullptr, first);
+}
+
+// per-satellite constants (mpc_discretize_batch_units): satellite s runs with psc[s] in place of the launch-wide
+// DiscParams; RAG as discretize_default_ragged_kernel (first == nullptr otherwise)
+template <bool J2, int BLOCK, bool RAG>
+__global__ void __launch_bounds__(BLOCK)
+discretize_default_units_kernel(const double *__restrict__ x_in, const double *__restrict__ u_in,
+                                const double *__restrict__ tf_arr, const DiscParams *psc, int n_sats, int K, double rtol,
+                                double atol, double max_step, DstTab dst, long long pitch, long long offset,
+                                int32_t *__restrict__ status, int32_t *__restrict__ n_nodes, const long long *__restrict__ first)
+{
+    discretize_default_body<J2, BLOCK, false, false, RAG, true>(x_in, u_in, tf_arr, psc[0], n_sats, K, K, rtol, atol, max_step,
+                                                                dst, pitch, offset, status, n_nodes, 0.0, nullptr, first, psc);
 }
 
 }  // namespace mpc

@@ -758,7 +758,9 @@ __device__ __forceinline__ void state_step5(const DiscParams &Ph, const UHold<fa
 // EM = 1 / 2 / 3: n_sub is kEmSteps / kEmSteps2 / kEmSteps3 and node n carries the weight kEmW[n] / kEmW2[n] / kEmW3[n]
 // instead of the trapezoid's 1/2, 1, ..., 1, 1/2.  EM = 3 takes the fifth-order steps (state_step5, column_step5).
 // RAG: a ragged batch -- K is the padded stride Kmax, the interval is (rs, rk) on a grid of rK nodes, gid = rs (K-1) + rk.
-template <bool J2, int BLOCK, int NDST, bool GENU, int EM = 0, bool RAG = false>
+// PSC: per-satellite constants (discretize_pair_kernel): P is this satellite's, and the node terms read 1/(G0 ISP) from
+// the thread's extra shared-memory slot kDiscSlots instead of keeping it live through the step loop.
+template <bool J2, int BLOCK, int NDST, bool GENU, int EM = 0, bool RAG = false, bool PSC = false>
 __device__ __forceinline__ void discretize_thread(const double *__restrict__ x, const double *__restrict__ u,
                                                   const double *__restrict__ tf_arr, const DiscParams &P, int K, int Ku,
                                                   int n_sub, const DstTab &dst, long long pitch, long long offset,
@@ -864,7 +866,9 @@ __device__ __forceinline__ void discretize_thread(const double *__restrict__ x, 
                              ((n == 0 || n == n_sub) ? 0.5 : 1.0)));   // trapezoid end weights (:77-80)
             const double ws = w * sfrac;
             // D Duf = [0; hs I/m; b^T];  hs D Sigma = [v~; a~; mdot~];  hs D xi' = -[v~; G~ r; mdot~_B]
-            node_accumulate<BLOCK>(acc, pr, pv, P, im * hs, ux, uy, uz, iun, md1, vx, vy, vz, a1x, a1y, a1z, grx, gry, grz, w, ws);
+            DiscParams Pn = P;
+            if constexpr (PSC) Pn.inv_ve = ACC(kDiscSlots);
+            node_accumulate<BLOCK>(acc, pr, pv, Pn, im * hs, ux, uy, uz, iun, md1, vx, vy, vz, a1x, a1y, a1z, grx, gry, grz, w, ws);
         }
         if (n == n_sub) break;
 

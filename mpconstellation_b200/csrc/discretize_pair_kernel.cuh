@@ -123,11 +123,17 @@ __device__ __forceinline__ void node_accumulate_column(volatile double *acc, int
 // covers the live intervals of every satellite (k0 = 0, kc = K - 1, no k-major layout, one destination).  Satellite s has
 // K_s = first[s+1] - first[s] + 1 nodes, its results go to columns offset + s (Kmax-1) + k (k < K_s - 1); the padding
 // columns are never written.
-template <bool J2, int BLOCK, int MAXREG, int NDST, bool RAG = false>
+// PSC: per-satellite constants -- the thread of satellite s runs with psc[s] in place of P (the units of that satellite's
+// own scale: mpc_discretize_batch_units); everything else is the launch's.  P is folded into the step-normalised Ph at
+// thread start; the one value the step loop still reads, 1/(G0 ISP) of the node terms, is parked in an extra shared-memory
+// slot per thread (kDiscSlots; the launch adds it) and re-read where it is used, so that the loop keeps no more registers
+// live than with the launch-wide P (kept live, it made this 255-register kernel spill).
+template <bool J2, int BLOCK, int MAXREG, int NDST, bool RAG = false, bool PSC = false>
 __global__ void __launch_bounds__(BLOCK) __maxnreg__(MAXREG)
 discretize_pair_kernel(const double *__restrict__ x, const double *__restrict__ u, const double *__restrict__ tf_arr,
                        DiscParams P, int n_sats, int K, int n_sub, DstTab dst, long long pitch, long long offset,
-                       int32_t *__restrict__ status, int k0, int kc, const long long *__restrict__ first = nullptr)
+                       int32_t *__restrict__ status, int k0, int kc, const long long *__restrict__ first = nullptr,
+                       const DiscParams *__restrict__ psc = nullptr)
 {
     // The launch covers the intervals k in [k0, k0 + kc) of every satellite (the whole batch: k0 = 0, kc = K - 1).  A
     // window of k is what the overlapped propagate -> discretize pass launches as soon as the propagation has produced
@@ -154,6 +160,10 @@ discretize_pair_kernel(const double *__restrict__ x, const double *__restrict__ 
     } else {
         s = (int)(tid / kc);
         k = k0 + (int)(tid - (long long)s * kc);
+    }
+    if constexpr (PSC) {
+        P = psc[s];
+        ACC(kDiscSlots) = P.inv_ve;
     }
     const long long gid = (long long)s * (K - 1) + k;
     const double tf = tf_arr[s];
@@ -191,21 +201,21 @@ discretize_pair_kernel(const double *__restrict__ x, const double *__restrict__ 
                     // of its size: 10 fifth-order steps and the 11-node rule kEmW3 (its remainder grows like the eighth
                     // power of that change: 2.5e-13 of the 101-node sums at 1/8, 4e-11 at 1/4)
                     if (dst.em >= 2 && d2 <= 0.015625 * fmax(a2, b2)) {
-                        discretize_thread<J2, BLOCK, NDST, false, 3, RAG>(x, u, tf_arr, P, K, K, kEmSteps3, dst, pitch, offset, status, gid, acc, s, k, Kg);
+                        discretize_thread<J2, BLOCK, NDST, false, 3, RAG, PSC>(x, u, tf_arr, P, K, K, kEmSteps3, dst, pitch, offset, status, gid, acc, s, k, Kg);
                         return;
                     }
-                    discretize_thread<J2, BLOCK, NDST, false, 1, RAG>(x, u, tf_arr, P, K, K, kEmSteps, dst, pitch, offset, status, gid, acc, s, k, Kg);
+                    discretize_thread<J2, BLOCK, NDST, false, 1, RAG, PSC>(x, u, tf_arr, P, K, K, kEmSteps, dst, pitch, offset, status, gid, acc, s, k, Kg);
                     return;
                 }
                 // longer intervals (omega 2h <= 4.4e-3 rad: 0.035-orbit intervals): 50 steps and the 51-node rule kEmW2
                 if (w2H2 <= 1.94e-5) {
-                    discretize_thread<J2, BLOCK, NDST, false, 2, RAG>(x, u, tf_arr, P, K, K, kEmSteps2, dst, pitch, offset, status, gid, acc, s, k, Kg);
+                    discretize_thread<J2, BLOCK, NDST, false, 2, RAG, PSC>(x, u, tf_arr, P, K, K, kEmSteps2, dst, pitch, offset, status, gid, acc, s, k, Kg);
                     return;
                 }
             }
         }
         if ((n_sub & 1) || !(w2H2 <= 1.0e-5)) {
-            discretize_thread<J2, BLOCK, NDST, false, 0, RAG>(x, u, tf_arr, P, K, K, n_sub, dst, pitch, offset, status, gid, acc, s, k, Kg);
+            discretize_thread<J2, BLOCK, NDST, false, 0, RAG, PSC>(x, u, tf_arr, P, K, K, n_sub, dst, pitch, offset, status, gid, acc, s, k, Kg);
             return;
         }
     }
@@ -274,7 +284,9 @@ discretize_pair_kernel(const double *__restrict__ x, const double *__restrict__ 
         {
             const double sfrac = (double)(2 * j) * inv_n;
             const double w = (j == 0 || j == n_pairs) ? 0.5 : 1.0;
-            node_accumulate<BLOCK>(acc, pr, pv, P, im * H, ux, uy, uz, iun, md1, vx, vy, vz, a1x, a1y, a1z, gr[0], gr[1], gr[2],
+            DiscParams Pn = P;
+            if constexpr (PSC) Pn.inv_ve = ACC(kDiscSlots);
+            node_accumulate<BLOCK>(acc, pr, pv, Pn, im * H, ux, uy, uz, iun, md1, vx, vy, vz, a1x, a1y, a1z, gr[0], gr[1], gr[2],
                                    w, w * sfrac);
         }
         if (j == n_pairs) break;
@@ -357,7 +369,7 @@ discretize_pair_kernel(const double *__restrict__ x, const double *__restrict__ 
             nv.aa[2] = fma(umz, i2, amz);
         }
         {
-            const double bs = -P.inv_ve * iunm;
+            const double bs = -(PSC ? (double)ACC(kDiscSlots) : P.inv_ve) * iunm;
             nv.b[0] = bs * umx;
             nv.b[1] = bs * umy;
             nv.b[2] = bs * umz;

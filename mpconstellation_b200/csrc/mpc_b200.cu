@@ -6,6 +6,7 @@
 #include <cuda_runtime.h>
 
 #include <algorithm>
+#include <cmath>
 #include <atomic>
 #include <cstdarg>
 #include <cstdio>
@@ -21,6 +22,7 @@
 #include "propagate_kernel.cuh"
 #include "propagate_rk45_kernel.cuh"
 #include "mpc_b200_drag.h"
+#include "mpc_b200_units.h"
 #include "constraint_terms_kernel.cuh"
 #include "discretize_drag_kernel.cuh"
 #include "discretize_pair_kernel.cuh"
@@ -70,6 +72,56 @@ mpc::PropParams prop_params(const mpc_params *p)
     d.include_j2 = p->include_j2;
     d.include_drag = p->include_drag;
     return d;
+}
+
+// ---- per-satellite designer units (the *_units entry points) ---------------------------------------------------------
+static_assert(sizeof(mpc::PropParams) <= MPC_SAT_SCRATCH_DOUBLES * sizeof(double) &&
+              sizeof(mpc::DiscParams) <= MPC_SAT_SCRATCH_DOUBLES * sizeof(double), "per-satellite scratch too small");
+
+int check_sat_consts(const mpc_sat_consts *c, int n)
+{
+    if (!c) return fail(MPC_E_INVALID, "null consts");
+    for (int s = 0; s < n; ++s) {
+        const double v[7] = {c[s].mu, c[s].r_e, c[s].j2, c[s].g0, c[s].isp, c[s].s_area, c[s].rho};
+        for (double x : v)
+            if (!std::isfinite(x)) return fail(MPC_E_INVALID, "consts[%d]: every value must be finite", s);
+        if (!(c[s].mu > 0.0) || !(c[s].g0 * c[s].isp > 0.0))
+            return fail(MPC_E_INVALID, "consts[%d]: need mu > 0 and g0 * isp > 0 (got %g, %g)", s, c[s].mu, c[s].g0 * c[s].isp);
+    }
+    return MPC_SUCCESS;
+}
+
+// q (a copy of the launch's mpc_params) with satellite s's per-scale fields: its kernel constants come out of
+// disc_params / prop_params themselves, the expressions (and so the bits) of a single-constant launch under consts[s]
+void with_consts(mpc_params &q, const mpc_sat_consts &c)
+{
+    q.mu = c.mu;
+    q.r_e = c.r_e;
+    q.j2 = c.j2;
+    q.g0 = c.g0;
+    q.isp = c.isp;
+    q.s_area = c.s_area;
+    q.rho = c.rho;
+}
+
+// derive the kernel constants of every satellite and copy them into the device scratch (the vector is pageable:
+// cudaMemcpyAsync has staged it when it returns)
+template <typename T, typename F>
+int upload_sat_table(const mpc_params *p, const mpc_sat_consts *c, int n, void *scratch, cudaStream_t st, F derive)
+{
+    if (!scratch) return fail(MPC_E_INVALID, "null consts_scratch");
+    if (mpc_units_sizeof(0) != sizeof(mpc::DiscParams) || mpc_units_sizeof(1) != sizeof(mpc::DstTab) ||
+        mpc_units_sizeof(2) != sizeof(mpc::PropParams) || mpc_units_sizeof(3) != sizeof(mpc::CtrlParams) ||
+        mpc_units_sizeof(4) != sizeof(mpc::Rk45Opts))
+        return fail(MPC_E_CUDA, "mpc_b200_units.cu was built against different parameter structs");
+    std::vector<T> v((size_t)n);
+    mpc_params q = *p;
+    for (int s = 0; s < n; ++s) {
+        with_consts(q, c[s]);
+        v[s] = derive(&q);
+    }
+    CUDA_TRY(cudaMemcpyAsync(scratch, v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice, st));
+    return MPC_SUCCESS;
 }
 
 std::atomic<int> g_tuning{0};
@@ -142,7 +194,7 @@ int launch_pair_cfg(const double *x, const double *u, const double *tf, const mp
     const unsigned grid = (unsigned)((n_int + BLOCK - 1) / BLOCK);
     mpc::DstTab tab = dst;
     tab.em = em_level();
-    kern<<<grid, BLOCK, smem, st>>>(x, u, tf, P, n_sats, K, n_sub, tab, pitch, offset, status, k0, kc, nullptr);
+    kern<<<grid, BLOCK, smem, st>>>(x, u, tf, P, n_sats, K, n_sub, tab, pitch, offset, status, k0, kc, nullptr, nullptr);
     g_launches.fetch_add(1, std::memory_order_relaxed);
     CUDA_TRY(cudaGetLastError());
     return MPC_SUCCESS;
@@ -550,7 +602,7 @@ int launch_ragged_pair(const double *x, const double *u, const double *tf, const
     const unsigned grid = (unsigned)((n_live + BLOCK - 1) / BLOCK);
     mpc::DstTab tab = dst;
     tab.em = em_level();
-    kern<<<grid, BLOCK, smem, st>>>(x, u, tf, P, n_sats, K, n_sub, tab, pitch, offset, status, 0, K - 1, first);
+    kern<<<grid, BLOCK, smem, st>>>(x, u, tf, P, n_sats, K, n_sub, tab, pitch, offset, status, 0, K - 1, first, nullptr);
     g_launches.fetch_add(1, std::memory_order_relaxed);
     CUDA_TRY(cudaGetLastError());
     return MPC_SUCCESS;
@@ -573,6 +625,63 @@ int launch_ragged(const double *x, const double *u, const double *tf, const mpc:
     if (n_live < 148LL * 9 * 32 * 2)
         return launch_ragged_pair<J2, 32>(x, u, tf, P, n_sats, K, n_live, first, n_sub, dst, pitch, offset, status, st);
     return launch_ragged_pair<J2, kDiscBlock>(x, u, tf, P, n_sats, K, n_live, first, n_sub, dst, pitch, offset, status, st);
+}
+
+// Per-satellite constants (psc: device DiscParams [n_sats]): one launch for the batch, rectangular (first == nullptr,
+// n_units = n_sats (K-1); default mode only) or ragged (n_units live intervals).  The fixed-step form is ragged only: a
+// rectangular batch takes it with equal counts, because the rectangular pair kernel with the table spilled where its
+// single-constant twin does not (the J2 build: 20 / 56 B against 4 / 40 B), and the ragged one matches its twin.  The block sizes are those launch_disc_n / launch_adaptive_k
+// and launch_ragged choose from the same count; the thread-group kernel of small rectangular batches has no such form:
+// small batches take the pair kernel in one-warp CTAs, as small ragged batches do.
+int launch_units_disc(const double *x, const double *u, const double *tf, const mpc::DiscParams *psc, bool j2, int n_sats,
+                      int K, long long n_units, const long long *first, const AdaptiveOpts *ad, int n_sub, const mpc::DstTab &dst,
+                      long long pitch, long long offset, int32_t *status, cudaStream_t st)
+{
+    MpcUnitsDisc a{};
+    mpc::DstTab tab = dst;
+    tab.em = em_level();
+    a.x = x;
+    a.u = u;
+    a.tf = tf;
+    a.psc = psc;
+    a.dst_tab = &tab;
+    a.first = first;
+    a.n_units = n_units;
+    a.include_j2 = j2;
+    a.n_sats = n_sats;
+    a.K = K;
+    a.n_sub = n_sub;
+    a.adaptive = ad != nullptr;
+    if (ad) {
+        a.block = g_default_block.load(std::memory_order_relaxed);
+        if (n_units < 148LL * 256) a.block = 32;
+        a.rtol = ad->rtol;
+        a.atol = ad->atol;
+        a.max_step = ad->max_step;
+        a.n_nodes = ad->n_nodes;
+    } else {
+        a.block = (n_units > 148LL * 32 && n_units <= 148LL * 128) || n_units >= 148LL * 9 * 32 * 2 ? kDiscBlock : 32;
+    }
+    a.pitch = pitch;
+    a.offset = offset;
+    a.status = status;
+    a.stream = st;
+    CUDA_TRY(mpc_units_launch_disc(&a));
+    g_launches.fetch_add(1, std::memory_order_relaxed);
+    return MPC_SUCCESS;
+}
+
+int check_units_disc(const double *x, const double *u, const double *tf, const mpc_params *p, const mpc_sat_consts *consts,
+                     int n_sats, int K_max, const int32_t *K_sat, int adaptive, int n_sub, double rtol, double atol, double max_step)
+{
+    int rc = check_disc_args(x, u, tf, p, n_sats, K_max, adaptive ? 1 : n_sub);
+    if (rc) return rc;
+    if (p->include_drag) return fail(MPC_E_UNSUPPORTED, "the drag linearisation is not implemented with per-satellite constants");
+    if (adaptive && g_default_v1.load(std::memory_order_relaxed))
+        return fail(MPC_E_UNSUPPORTED, "the round-1 default-mode kernel (mpc_set_tuning(9)) has no per-satellite-constants form");
+    if (adaptive && (rc = check_adaptive(rtol, atol, max_step))) return rc;
+    if (K_sat && (rc = check_counts(K_sat, n_sats, K_max, "K_sat"))) return rc;
+    return check_sat_consts(consts, n_sats);
 }
 
 int check_ragged_disc(const double *x, const double *u, const double *tf, const mpc_params *p, int n_sats, int K_max,
@@ -666,9 +775,11 @@ void launch_rk45_ragged(bool spec, unsigned n_warps, cudaStream_t st, const doub
 int prop_device(const double *y0, const double *tf, const mpc_params *p, const mpc_controller *c,
                 const double *table_dev, const double *end_tau_dev, int n_sats, int T, const PropMode &mode, double *y, double *u_out, int32_t *status,
                 cudaStream_t st, unsigned int *progress = nullptr, int seg_len = 0, unsigned int *progress_target = nullptr,
-                const int32_t *T_sat_dev = nullptr, const int32_t *ku_dev = nullptr)
+                const int32_t *T_sat_dev = nullptr, const int32_t *ku_dev = nullptr, const mpc::PropParams *psc_dev = nullptr)
 {
     if (!y0 || !tf || !p || !y) return fail(MPC_E_INVALID, "null pointer argument");
+    if (psc_dev && (!mode.rk45() || progress))
+        return fail(MPC_E_UNSUPPORTED, "per-satellite constants need the RK45 propagator (n_sub = 0) outside the fused pass");
     // per-satellite counts (device arrays here): the RK45 propagator on its own only
     const bool ragged = T_sat_dev || ku_dev;
     if (ragged && (!mode.rk45() || progress))
@@ -703,6 +814,31 @@ int prop_device(const double *y0, const double *tf, const mpc_params *p, const m
     const unsigned n_warps = (unsigned)((n_sats + lpw - 1) / lpw);
     const bool spec = g_rk45_spec.load(std::memory_order_relaxed) != 0;
     if (progress_target) *progress_target = mode.rk45() ? (unsigned)n_sats : (unsigned)((n_sats + 31) / 32);
+    if (psc_dev) {   // per-satellite constants: one-warp CTAs, mpc_b200_units.cu
+        MpcUnitsProp a{};
+        a.y0 = y0;
+        a.tf = tf;
+        a.psc = psc_dev;
+        a.ctrl = &C;
+        a.opts = &mode.rk;
+        a.kind = c->kind;
+        a.include_drag = p->include_drag;
+        a.include_j2 = p->include_j2;
+        a.n_sats = n_sats;
+        a.T = T;
+        a.lpw = lpw;
+        a.n_warps = n_warps;
+        a.y = y;
+        a.u_out = u_out;
+        a.status = status;
+        a.n_steps = mode.n_steps;
+        a.T_sat = T_sat_dev;
+        a.ku = ku_dev;
+        a.stream = st;
+        CUDA_TRY(mpc_units_launch_rk45(&a));
+        g_launches.fetch_add(1, std::memory_order_relaxed);
+        return MPC_SUCCESS;
+    }
     // one straight-line kernel per (controller law, drag, J2)
 #define MPC_PROP(KIND, DRAG, J2)                                                                                          \
     do {                                                                                                                  \
@@ -764,6 +900,8 @@ struct mpc_ctx {
     long long *d_first = nullptr;            // ragged batches: prefix sums of K_s - 1
     int32_t *d_cnt = nullptr;                // ragged batches: T_sat and table_len_sat
     size_t cap_first = 0, cap_cnt = 0;
+    double *d_psc = nullptr;                 // per-satellite constants: the derived kernel constants (*_units_host)
+    size_t cap_psc = 0;
     cudaStream_t s_pushk = nullptr;          // high-priority stream of the copy kernels (push gather, SM-driven variant)
     cudaStream_t s_aux[3] = {};              // compute streams the chunk kernels of the push gather rotate over
     cudaStream_t s_push[MPC_MAX_DST] = {};   // one stream per peer for the copy-engine gather (mpc_discretize_batch_push)
@@ -1105,6 +1243,7 @@ int mpc_ctx_destroy(mpc_ctx *c)
     cudaFree(c->d_endtau);
     cudaFree(c->d_first);
     cudaFree(c->d_cnt);
+    cudaFree(c->d_psc);
     if (c->h_stage) cudaFreeHost(c->h_stage);
     delete c;
     return MPC_SUCCESS;
@@ -1128,12 +1267,15 @@ void mpc_host_free(void *p)
 
 // shared body of the two host-buffer discretization entry points (ad == nullptr: fixed-step kernel)
 // K_sat != nullptr: a ragged batch (K = Kmax, mpc_discretize_batch_ragged_host)
+// consts != nullptr: per-satellite constants (mpc_discretize_batch_units_host), rectangular or ragged
 static int disc_host(mpc_ctx *ctx, const double *x, const double *u, const double *tf, const mpc_params *p, int n_sats,
                      int K, int n_sub, const AdaptiveOpts *ad, double *out_host, int32_t *status_host,
-                     int32_t *n_nodes_host, const int32_t *K_sat = nullptr)
+                     int32_t *n_nodes_host, const int32_t *K_sat = nullptr, const mpc_sat_consts *consts = nullptr)
 {
     if (!ctx || !out_host) return fail(MPC_E_INVALID, "null ctx/out");
-    int rc = K_sat ? check_ragged_disc(x, u, tf, p, n_sats, K, K_sat, ad != nullptr, n_sub, ad ? ad->rtol : 0.0, ad ? ad->atol : 0.0,
+    int rc = consts ? check_units_disc(x, u, tf, p, consts, n_sats, K, K_sat, ad != nullptr, n_sub, ad ? ad->rtol : 0.0,
+                                       ad ? ad->atol : 0.0, ad ? ad->max_step : 0.0)
+           : K_sat ? check_ragged_disc(x, u, tf, p, n_sats, K, K_sat, ad != nullptr, n_sub, ad ? ad->rtol : 0.0, ad ? ad->atol : 0.0,
                                        ad ? ad->max_step : 0.0)
                    : check_disc_args(x, u, tf, p, n_sats, K, n_sub);
     if (rc) return rc;
@@ -1159,6 +1301,11 @@ static int disc_host(mpc_ctx *ctx, const double *x, const double *u, const doubl
         if ((rc = ensure(ctx->d_first, ctx->cap_first, first.size()))) return rc;
         CUDA_TRY(cudaMemcpyAsync(ctx->d_first, first.data(), first.size() * sizeof(long long), cudaMemcpyHostToDevice, ctx->s_compute));
     }
+    if (consts) {
+        if ((rc = ensure(ctx->d_psc, ctx->cap_psc, (size_t)n_sats * MPC_SAT_SCRATCH_DOUBLES))) return rc;
+        if ((rc = upload_sat_table<mpc::DiscParams>(p, consts, n_sats, ctx->d_psc, ctx->s_compute, disc_params))) return rc;
+    }
+    const mpc::DiscParams *psc = (const mpc::DiscParams *)ctx->d_psc;
     for (int c = 0; c < n_chunks; ++c) {
         const int s0 = c * cs, ns = std::min(cs, n_sats - s0);
         const double *dx = ctx->d_x + (size_t)s0 * 7 * K, *du = ctx->d_u + (size_t)s0 * 3 * Ku;
@@ -1169,7 +1316,12 @@ static int disc_host(mpc_ctx *ctx, const double *x, const double *u, const doubl
         mpc::DstTab tab{};
         tab.p[0] = ctx->d_out;
         const long long off = (long long)s0 * (K - 1);
-        if (K_sat) {
+        if (consts && !K_sat) {
+            AdaptiveOpts o = ad ? *ad : AdaptiveOpts{};
+            o.n_nodes = (ad && n_nodes_host) ? ctx->d_nodes + off : nullptr;
+            rc = launch_units_disc(dx, du, ctx->d_tf + s0, psc + s0, p->include_j2, ns, K, (long long)ns * (K - 1), nullptr,
+                                   ad ? &o : nullptr, n_sub, tab, n_int, off, ctx->d_status + off, ctx->s_compute);
+        } else if (K_sat) {
             // the kernel leaves the padding columns alone: they go back as NaN (all-ones bytes) / status 0 / 0 nodes
             const long long nc = (long long)ns * (K - 1);
             CUDA_TRY(cudaMemset2DAsync(ctx->d_out + off, (size_t)n_int * sizeof(double), 0xFF, (size_t)nc * sizeof(double),
@@ -1178,10 +1330,14 @@ static int disc_host(mpc_ctx *ctx, const double *x, const double *u, const doubl
             if (ad && n_nodes_host) CUDA_TRY(cudaMemsetAsync(ctx->d_nodes + off, 0, (size_t)nc * sizeof(int32_t), ctx->s_compute));
             AdaptiveOpts o = ad ? *ad : AdaptiveOpts{};
             o.n_nodes = (ad && n_nodes_host) ? ctx->d_nodes + off : nullptr;
-            rc = p->include_j2 ? launch_ragged<true>(dx, du, ctx->d_tf + s0, P, ns, K, first[s0 + ns] - first[s0], ctx->d_first + s0,
-                                                     ad ? &o : nullptr, n_sub, tab, n_int, off, ctx->d_status + off, ctx->s_compute)
-                               : launch_ragged<false>(dx, du, ctx->d_tf + s0, P, ns, K, first[s0 + ns] - first[s0], ctx->d_first + s0,
-                                                      ad ? &o : nullptr, n_sub, tab, n_int, off, ctx->d_status + off, ctx->s_compute);
+            if (consts)
+                rc = launch_units_disc(dx, du, ctx->d_tf + s0, psc + s0, p->include_j2, ns, K, first[s0 + ns] - first[s0],
+                                       ctx->d_first + s0, ad ? &o : nullptr, n_sub, tab, n_int, off, ctx->d_status + off, ctx->s_compute);
+            else
+                rc = p->include_j2 ? launch_ragged<true>(dx, du, ctx->d_tf + s0, P, ns, K, first[s0 + ns] - first[s0], ctx->d_first + s0,
+                                                         ad ? &o : nullptr, n_sub, tab, n_int, off, ctx->d_status + off, ctx->s_compute)
+                                   : launch_ragged<false>(dx, du, ctx->d_tf + s0, P, ns, K, first[s0 + ns] - first[s0], ctx->d_first + s0,
+                                                          ad ? &o : nullptr, n_sub, tab, n_int, off, ctx->d_status + off, ctx->s_compute);
         } else if (ad) {
             AdaptiveOpts o = *ad;
             with_drag(o, p);
@@ -1275,9 +1431,11 @@ static int upload_table(mpc_ctx *ctx, const mpc_controller *ctrl, int n_sats, cu
 
 // T_sat != nullptr: per-satellite sample counts (T = Tmax) and table lengths (ku, may be NULL), host arrays
 // (mpc_propagate_batch_rk45_ragged_host)
+// consts != nullptr: per-satellite constants (mpc_propagate_batch_rk45_units_host)
 static int prop_host(mpc_ctx *ctx, const double *y0, const double *tf, const mpc_params *p, const mpc_controller *ctrl,
                      int n_sats, int T, PropMode mode, double *y_host, double *u_host, int32_t *status_host,
-                     int32_t *n_steps_host, const int32_t *T_sat = nullptr, const int32_t *ku_in = nullptr)
+                     int32_t *n_steps_host, const int32_t *T_sat = nullptr, const int32_t *ku_in = nullptr,
+                     const mpc_sat_consts *consts = nullptr)
 {
     if (!ctx || !y0 || !tf || !p || !y_host) return fail(MPC_E_INVALID, "null pointer argument");
     if (n_sats < 0 || T < 0 || mode.n_sub < 0) return fail(MPC_E_INVALID, "need n_sats >= 0, T >= 0, n_sub >= 0");
@@ -1286,6 +1444,7 @@ static int prop_host(mpc_ctx *ctx, const double *y0, const double *tf, const mpc
     const int32_t *ku = (ctrl->kind == MPC_CTRL_SEQUENCE) ? ku_in : nullptr;
     if (T_sat && (rc = check_counts(T_sat, n_sats, T, "T_sat"))) return rc;
     if (ku && (rc = check_counts(ku, n_sats, ctrl->table_len, "table_len_sat"))) return rc;
+    if (consts && (rc = check_sat_consts(consts, n_sats))) return rc;
     if (n_sats == 0 || T == 0) return MPC_SUCCESS;
     CUDA_TRY(cudaSetDevice(ctx->device));
     if ((rc = ensure(ctx->d_y0, ctx->cap_y0, (size_t)n_sats * 7))) return rc;
@@ -1310,9 +1469,13 @@ static int prop_host(mpc_ctx *ctx, const double *y0, const double *tf, const mpc
         CUDA_TRY(cudaMemsetAsync(ctx->d_x, 0xFF, (size_t)n_sats * 7 * T * sizeof(double), st));
         if (u_host) CUDA_TRY(cudaMemsetAsync(ctx->d_u, 0xFF, (size_t)n_sats * 3 * T * sizeof(double), st));
     }
+    if (consts) {
+        if ((rc = ensure(ctx->d_psc, ctx->cap_psc, (size_t)n_sats * MPC_SAT_SCRATCH_DOUBLES))) return rc;
+        if ((rc = upload_sat_table<mpc::PropParams>(p, consts, n_sats, ctx->d_psc, st, prop_params))) return rc;
+    }
     if ((rc = prop_device(ctx->d_y0, ctx->d_tf, p, ctrl, ctx->d_tab, ctrl->end_tau_per_sat ? ctx->d_endtau : nullptr, n_sats, T, mode,
                           ctx->d_x, ctx->d_u, ctx->d_status2, st, nullptr, 0, nullptr, T_sat ? ctx->d_cnt : nullptr,
-                          ku ? ctx->d_cnt + n_sats : nullptr)))
+                          ku ? ctx->d_cnt + n_sats : nullptr, consts ? (const mpc::PropParams *)ctx->d_psc : nullptr)))
         return rc;
     CUDA_TRY(cudaMemcpyAsync(y_host, ctx->d_x, (size_t)n_sats * 7 * T * sizeof(double), cudaMemcpyDeviceToHost, st));
     if (u_host) CUDA_TRY(cudaMemcpyAsync(u_host, ctx->d_u, (size_t)n_sats * 3 * T * sizeof(double), cudaMemcpyDeviceToHost, st));
@@ -1333,6 +1496,93 @@ int mpc_propagate_batch_rk45_ragged_host(mpc_ctx *ctx, const double *y0, const d
     PropMode m;
     m.rk = mpc::Rk45Opts{rtol, atol, max_step};
     return prop_host(ctx, y0, tf, p, ctrl, n_sats, T_max, m, y_host, u_host, status_host, n_steps_host, T_sat, table_len_sat);
+}
+
+// ---- per-satellite designer units --------------------------------------------------------------------------------------
+int mpc_discretize_batch_units(const double *x, const double *u, const double *tf, const mpc_params *p,
+                               const mpc_sat_consts *consts, int n_sats, int K_max, const int32_t *K_sat, int64_t *first,
+                               double *consts_scratch, int adaptive, int n_sub, double rtol, double atol, double max_step,
+                               double *out, int64_t out_pitch, int64_t out_offset, int32_t *status, int32_t *n_nodes,
+                               void *stream)
+{
+    int rc = check_units_disc(x, u, tf, p, consts, n_sats, K_max, K_sat, adaptive, n_sub, rtol, atol, max_step);
+    if (rc) return rc;
+    if (!out || (K_sat && !first)) return fail(MPC_E_INVALID, "null output / first");
+    if (out_pitch < out_offset + (long long)n_sats * (K_max - 1) || out_offset < 0)
+        return fail(MPC_E_INVALID, "out_pitch/out_offset do not hold the batch");
+    if (n_sats == 0) return MPC_SUCCESS;
+    cudaStream_t st = (cudaStream_t)stream;
+    if ((rc = upload_sat_table<mpc::DiscParams>(p, consts, n_sats, consts_scratch, st, disc_params))) return rc;
+    long long n_units = (long long)n_sats * (K_max - 1);
+    // the fixed-step form of a rectangular batch is the ragged launch with equal counts (launch_units_disc); its prefix
+    // sums go behind the table in the scratch (3 + 1 of the MPC_SAT_SCRATCH_DOUBLES per satellite, plus one)
+    std::vector<int32_t> equal;
+    if (!K_sat && !adaptive) {
+        equal.assign((size_t)n_sats, K_max);
+        K_sat = equal.data();
+        first = (int64_t *)(consts_scratch + (size_t)n_sats * (sizeof(mpc::DiscParams) / sizeof(double)));
+    }
+    if (K_sat) {
+        const std::vector<long long> f = ragged_first(K_sat, n_sats);
+        CUDA_TRY(cudaMemcpyAsync(first, f.data(), f.size() * sizeof(long long), cudaMemcpyHostToDevice, st));
+        n_units = f[n_sats];
+    }
+    mpc::DstTab tab{};
+    tab.p[0] = out;
+    const AdaptiveOpts o{rtol, atol, max_step, n_nodes};
+    return launch_units_disc(x, u, tf, (const mpc::DiscParams *)consts_scratch, p->include_j2, n_sats, K_max, n_units,
+                             K_sat ? (const long long *)first : nullptr, adaptive ? &o : nullptr, n_sub, tab, out_pitch,
+                             out_offset, status, st);
+}
+
+int mpc_discretize_batch_units_host(mpc_ctx *ctx, const double *x, const double *u, const double *tf, const mpc_params *p,
+                                    const mpc_sat_consts *consts, int n_sats, int K_max, const int32_t *K_sat, int adaptive,
+                                    int n_sub, double rtol, double atol, double max_step, double *out_host,
+                                    int32_t *status_host, int32_t *n_nodes_host)
+{
+    if (!consts) return fail(MPC_E_INVALID, "null consts");
+    const AdaptiveOpts o{rtol, atol, max_step, nullptr};
+    std::vector<int32_t> equal;   // a rectangular fixed-step batch: the ragged launch with equal counts (launch_units_disc)
+    if (!K_sat && !adaptive && n_sats > 0) {
+        equal.assign((size_t)n_sats, K_max);
+        K_sat = equal.data();
+    }
+    return disc_host(ctx, x, u, tf, p, n_sats, K_max, adaptive ? 1 : n_sub, adaptive ? &o : nullptr, out_host, status_host,
+                     adaptive ? n_nodes_host : nullptr, K_sat, consts);
+}
+
+int mpc_propagate_batch_rk45_units(const double *y0, const double *tf, const mpc_params *p, const mpc_sat_consts *consts,
+                                   const mpc_controller *ctrl, int n_sats, int T_max, const int32_t *T_sat,
+                                   const int32_t *table_len_sat, double *consts_scratch, double rtol, double atol,
+                                   double max_step, double *y, double *u_out, int32_t *status, int32_t *n_steps,
+                                   void *stream)
+{
+    if (!p) return fail(MPC_E_INVALID, "null pointer argument");
+    if (T_sat && T_max < 2) return fail(MPC_E_INVALID, "need T_max >= 2 (got %d)", T_max);
+    int rc = check_sat_consts(consts, n_sats);
+    if (rc) return rc;
+    if (n_sats > 0 && T_max > 0 &&
+        (rc = upload_sat_table<mpc::PropParams>(p, consts, n_sats, consts_scratch, (cudaStream_t)stream, prop_params)))
+        return rc;
+    PropMode m;
+    m.rk = mpc::Rk45Opts{rtol, atol, max_step};
+    m.n_steps = n_steps;
+    return prop_device(y0, tf, p, ctrl, ctrl ? ctrl->table : nullptr, ctrl ? ctrl->end_tau_per_sat : nullptr, n_sats, T_max, m,
+                       y, u_out, status, (cudaStream_t)stream, nullptr, 0, nullptr, T_sat, table_len_sat,
+                       (const mpc::PropParams *)consts_scratch);
+}
+
+int mpc_propagate_batch_rk45_units_host(mpc_ctx *ctx, const double *y0, const double *tf, const mpc_params *p,
+                                        const mpc_sat_consts *consts, const mpc_controller *ctrl, int n_sats, int T_max,
+                                        const int32_t *T_sat, const int32_t *table_len_sat, double rtol, double atol,
+                                        double max_step, double *y_host, double *u_host, int32_t *status_host,
+                                        int32_t *n_steps_host)
+{
+    if (!consts) return fail(MPC_E_INVALID, "null consts");
+    PropMode m;
+    m.rk = mpc::Rk45Opts{rtol, atol, max_step};
+    return prop_host(ctx, y0, tf, p, ctrl, n_sats, T_max, m, y_host, u_host, status_host, n_steps_host, T_sat, table_len_sat,
+                     consts);
 }
 
 int mpc_propagate_batch_host(mpc_ctx *ctx, const double *y0, const double *tf, const mpc_params *p,
@@ -1983,6 +2233,84 @@ int mpc_dynamics_jacobian_ragged(const double *soa, int64_t pitch, int64_t offse
                                                               (const long long *)first);
     g_launches.fetch_add(1, std::memory_order_relaxed);
     CUDA_TRY(cudaGetLastError());
+    return MPC_SUCCESS;
+}
+
+// ---- per-satellite designer units: MU of every satellite from its own constants ----------------------------------------
+static int cterms_units_launch(const double *x, const double *u, int n_sats, int K_max, long long n_units, const long long *first,
+                               const double *mu_sat, double *rbar, double *ubar, double *fin, cudaStream_t st)
+{
+    if (mpc_units_sizeof(0) != sizeof(mpc::DiscParams)) return fail(MPC_E_CUDA, "mpc_b200_units.cu was built against different parameter structs");
+    CUDA_TRY(mpc_units_launch_cterms(x, u, n_sats, K_max, n_units, first, mu_sat, rbar, ubar, fin, st));
+    g_launches.fetch_add(1, std::memory_order_relaxed);
+    return MPC_SUCCESS;
+}
+
+static std::vector<double> mu_table(const mpc_sat_consts *c, int n)
+{
+    std::vector<double> v((size_t)n);
+    for (int s = 0; s < n; ++s) v[s] = c[s].mu;
+    return v;
+}
+
+int mpc_constraint_terms_units(const double *x, const double *u, int n_sats, int K_max, const int32_t *K_sat, int64_t *first,
+                               const mpc_sat_consts *consts, double *consts_scratch, double *rbar_hat, double *ubar_hat,
+                               double *final_terms, void *stream)
+{
+    int rc = cterms_check(x, u, n_sats, K_max, K_max, rbar_hat, ubar_hat, final_terms);
+    if (rc || (K_sat && (rc = check_counts(K_sat, n_sats, K_max, "K_sat"))) || (rc = check_sat_consts(consts, n_sats))) return rc;
+    if ((K_sat && !first) || !consts_scratch) return fail(MPC_E_INVALID, "null first / consts_scratch");
+    if (n_sats == 0) return MPC_SUCCESS;
+    cudaStream_t st = (cudaStream_t)stream;
+    const std::vector<double> mu = mu_table(consts, n_sats);
+    CUDA_TRY(cudaMemcpyAsync(consts_scratch, mu.data(), mu.size() * sizeof(double), cudaMemcpyHostToDevice, st));
+    long long n_units = (long long)n_sats * K_max;
+    if (K_sat) {
+        const std::vector<long long> f = ragged_first(K_sat, n_sats);
+        CUDA_TRY(cudaMemcpyAsync(first, f.data(), f.size() * sizeof(long long), cudaMemcpyHostToDevice, st));
+        n_units = f[n_sats];
+    }
+    return cterms_units_launch(x, u, n_sats, K_max, n_units, K_sat ? (const long long *)first : nullptr, consts_scratch, rbar_hat,
+                               ubar_hat, final_terms, st);
+}
+
+int mpc_constraint_terms_units_host(mpc_ctx *ctx, const double *x, const double *u, int n_sats, int K_max,
+                                    const int32_t *K_sat, const mpc_sat_consts *consts, double *rbar_hat, double *ubar_hat,
+                                    double *final_terms)
+{
+    if (!ctx) return fail(MPC_E_INVALID, "null ctx");
+    int rc = cterms_check(x, u, n_sats, K_max, K_max, rbar_hat, ubar_hat, final_terms);
+    if (rc || (K_sat && (rc = check_counts(K_sat, n_sats, K_max, "K_sat"))) || (rc = check_sat_consts(consts, n_sats)) || n_sats == 0)
+        return rc;
+    CUDA_TRY(cudaSetDevice(ctx->device));
+    const size_t nx = (size_t)n_sats * 7 * K_max, nu = (size_t)n_sats * 3 * K_max, nr = (size_t)n_sats * 3 * (K_max - 1),
+                 nf = (size_t)n_sats * MPC_FINAL_TERMS;
+    if ((rc = ensure(ctx->d_x, ctx->cap_x, nx))) return rc;
+    if ((rc = ensure(ctx->d_u, ctx->cap_u, nu))) return rc;
+    if ((rc = ensure(ctx->d_out, ctx->cap_out, nr + nu + nf))) return rc;
+    if ((rc = ensure(ctx->d_psc, ctx->cap_psc, (size_t)n_sats * MPC_SAT_SCRATCH_DOUBLES))) return rc;
+    cudaStream_t st = ctx->s_compute;
+    double *d_r = ctx->d_out, *d_ub = d_r + nr, *d_f = d_ub + nu;
+    CUDA_TRY(cudaMemcpyAsync(ctx->d_x, x, nx * sizeof(double), cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(ctx->d_u, u, nu * sizeof(double), cudaMemcpyHostToDevice, st));
+    const std::vector<double> mu = mu_table(consts, n_sats);
+    CUDA_TRY(cudaMemcpyAsync(ctx->d_psc, mu.data(), mu.size() * sizeof(double), cudaMemcpyHostToDevice, st));
+    long long n_units = (long long)n_sats * K_max;
+    if (K_sat) {
+        const std::vector<long long> f = ragged_first(K_sat, n_sats);
+        if ((rc = ensure(ctx->d_first, ctx->cap_first, f.size()))) return rc;
+        CUDA_TRY(cudaMemcpyAsync(ctx->d_first, f.data(), f.size() * sizeof(long long), cudaMemcpyHostToDevice, st));
+        n_units = f[n_sats];
+        // the kernel leaves the padding columns alone: they go back as NaN (all-ones bytes)
+        CUDA_TRY(cudaMemsetAsync(d_r, 0xFF, (nr + nu) * sizeof(double), st));
+    }
+    if ((rc = cterms_units_launch(ctx->d_x, ctx->d_u, n_sats, K_max, n_units, K_sat ? ctx->d_first : nullptr, ctx->d_psc, d_r, d_ub,
+                                  d_f, st)))
+        return rc;
+    CUDA_TRY(cudaMemcpyAsync(rbar_hat, d_r, nr * sizeof(double), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaMemcpyAsync(ubar_hat, d_ub, nu * sizeof(double), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaMemcpyAsync(final_terms, d_f, nf * sizeof(double), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
     return MPC_SUCCESS;
 }
 

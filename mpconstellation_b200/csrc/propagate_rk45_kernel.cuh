@@ -46,7 +46,11 @@ __device__ __forceinline__ double rk45_factor(double err2) { return 0.9 * pow(er
 // linspace(0, 1, T_sat[s]) and stores those T_sat[s] samples only (T_sat == nullptr: all T); its sequence table (stride
 // C.table_len) has Ku_sat[s] columns (Ku_sat == nullptr: all C.table_len).  The steps do not depend on the samples.  The
 // counts are clamped into the buffers (T_sat to [0, T], Ku_sat to [2, C.table_len]); the entry points validate them.
-template <int BLOCK, int KIND, bool DRAG, bool J2, bool SPEC, bool RAG = false>
+// PSC: per-satellite constants (mpc_propagate_batch_rk45_units) -- lane s integrates with its own PropParams, from the
+// device table [n_sats] passed in place of the progress words (such a launch has none).  The table travels in an
+// existing parameter because ptxas's register allocation of these ~250-register kernels follows the entry's parameter
+// list: one more parameter changed the SASS of every single-constant instantiation.
+template <int BLOCK, int KIND, bool DRAG, bool J2, bool SPEC, bool RAG = false, bool PSC = false>
 __global__ void __launch_bounds__(BLOCK)
 propagate_rk45_kernel(const double *__restrict__ y0, const double *__restrict__ tf_arr, PropParams P, CtrlParams C,
                       Rk45Opts O, int n_sats, int T, int lpw, double *__restrict__ y_out, double *__restrict__ u_out,
@@ -61,6 +65,14 @@ propagate_rk45_kernel(const double *__restrict__ y0, const double *__restrict__ 
     const int warp = (int)((blockIdx.x * (unsigned)BLOCK + threadIdx.x) >> 5);
     const int s = warp * lpw + lane;
     if (lane >= lpw || s >= n_sats) return;
+    // PSC: `progress` is the table of per-satellite constants (see above), read here and then cleared, so that every use
+    // of the progress words below sees none.  Nothing may read `progress` before this point.
+    static_assert(alignof(PropParams) == alignof(double) && sizeof(PropParams) % alignof(double) == 0,
+                  "the per-satellite table is an array of PropParams at a double-aligned address");
+    if constexpr (PSC) {
+        P = reinterpret_cast<const PropParams *>(progress)[s];
+        progress = nullptr;
+    }
     const double *tab = C.table ? C.table + (C.table_per_sat ? (long long)s * 3 * C.table_len : 0) : nullptr;
     // samples of this lane (T: the stride) and columns of its table (0: C.table_len), held inside the buffers
     const int Tn = (RAG && T_sat) ? min(max(T_sat[s], 0), T) : T;
@@ -309,6 +321,7 @@ propagate_rk45_kernel(const double *__restrict__ y0, const double *__restrict__ 
                 }
                 // a window is released one sample after its last interval ends (its end node's input lookup may reach one
                 // node further, see propagate_kernel), the last window at T-1
+                // (a PSC launch passed its constants table in `progress` and cleared it at thread start: no progress words)
                 if (progress && ti > 1 && (ti - 1) % seg_len == 0 && (ti - 1) < T - 1) {
                     const int b = (ti - 1) / seg_len - 1;
                     __threadfence();
@@ -344,7 +357,7 @@ propagate_rk45_kernel(const double *__restrict__ y0, const double *__restrict__ 
                 uo[T + ti] = qnan;
                 uo[2 * (long long)T + ti] = qnan;
             }
-            if (progress && ti > 1 && (ti - 1) % seg_len == 0 && (ti - 1) < T - 1) {
+            if (progress && ti > 1 && (ti - 1) % seg_len == 0 && (ti - 1) < T - 1) {   // (nullptr in a PSC launch)
                 __threadfence();
                 atomicAdd(progress + ((ti - 1) / seg_len - 1), 1u);
             }

@@ -91,3 +91,12 @@ class SatelliteScale:
 
     def normalize_thrust(self, u):
         return u / self._T0
+
+
+def sat_units(sats):
+    """Each satellite normalized by its own SatelliteScale, as N OptimalControllers of the reference compute it
+    (control.py:164): -> (y0 [N,7] normalized states, [N] Constants).  The constants list goes to propagate_batch,
+    discretize_batch, constraint_terms_batch and BatchedSCP as `const`."""
+    scales = [SatelliteScale(sat=s) for s in sats]
+    y0 = np.array([sc.normalize_state(s.get_state_vector()) for sc, s in zip(scales, sats)], dtype=np.float64).reshape(-1, 7)
+    return y0, [sc.get_normalized_constants() for sc in scales]

@@ -10,7 +10,9 @@ convex subproblem itself (pyomo + ipopt, optimizer.py:251-613) is out of scope a
     solver(hand_off) -> (u_new [N,3,Kmax] padded, or a list of (3,K_s) arrays; tf_new [N])
 where `hand_off.sat(s)` yields exactly the five arrays optimizer.py:327-339 indexes.  Every satellite is linearized on
 its own K_s = int(base_res * tf_s) nodes, as the reference's per-satellite controllers do (control.py:221,227,
-simulator.py:38); batches whose K_s differ run as one ragged launch per leg.  With pyomo/ipopt installed one
+simulator.py:38); batches whose K_s differ run as one ragged launch per leg.  `const` may be one Constants bag or one per
+satellite (model.sat_units: each satellite in the designer units of its own SatelliteScale, as N OptimalControllers of
+the reference plan it); per-satellite constants also run one launch per leg.  With pyomo/ipopt installed one
 wraps the reference's Optimizer in such a callable; `hold_reference_solver` is a deterministic stand-in (it returns the
 reference input unchanged) for boxes without a solver, clearly NOT an optimizer.
 """
@@ -31,6 +33,7 @@ class Linearization:
     tf: np.ndarray           # [N]
     matrices: "batch.DiscretizedBatch"
     K: np.ndarray = None     # [N] nodes of every satellite, int(base_res * tf_s)
+    const: object = None     # the Constants of the pass: one bag or one per satellite (constraint_terms_batch hand-off)
 
     def sat(self, s):
         """(A_k, B_kp, B_kn, Sigma_k, xi_k) of satellite s -- what Optimizer.solve_OPT appends at optimizer.py:243-249."""
@@ -105,8 +108,10 @@ class BatchedSCP:
         tfv = np.ascontiguousarray(np.broadcast_to(np.asarray(tf, dtype=np.float64), (N,)))
         K_sat = node_counts(self.base_res, tfv)
         ragged_law = getattr(spec_from(controller), "table_len", None) is not None
-        if (K_sat != K_sat[0]).any() or ragged_law:
-            # one ragged launch per leg: every satellite on its own grid (the fused pass is rectangular only)
+        units = _lib.sat_consts(self.const, N)[0] is not None
+        if (K_sat != K_sat[0]).any() or ragged_law or units:
+            # one ragged launch per leg: every satellite on its own grid and / or in its own units (the fused pass is
+            # rectangular and single-constant only)
             x, u, _, _ = batch.propagate_batch(y0, tfv, controller, self.const, include_drag=False, include_J2=False,
                                                T=K_sat, device=self.device)
             if self.use_uniform_steps:
@@ -115,7 +120,7 @@ class BatchedSCP:
             else:
                 res = batch.discretize_batch(x, u, tfv, self.const, include_J2=self.include_J2, device=self.device,
                                              adaptive=dict(rtol=1e-3, atol=1e-6, max_step=1e-2), K=K_sat)
-            return Linearization(np.asarray(x), np.asarray(u), tfv, res, K_sat)
+            return Linearization(np.asarray(x), np.asarray(u), tfv, res, K_sat, self.const)
         K = int(K_sat[0])
         if self.use_uniform_steps:
             # (k-major layout: the streamed host pass; the per-satellite views of the result hide it)
@@ -127,7 +132,7 @@ class BatchedSCP:
                                                T=K, device=self.device)
             res = batch.discretize_batch(x, u, tfv, self.const, include_J2=self.include_J2, device=self.device,
                                          adaptive=dict(rtol=1e-3, atol=1e-6, max_step=1e-2))
-        return Linearization(np.asarray(x), np.asarray(u), tfv, res, K_sat)
+        return Linearization(np.asarray(x), np.asarray(u), tfv, res, K_sat, self.const)
 
     def plan(self, y0, solver=hold_reference_solver):
         """OptimalController.update for N satellites: seed trajectory, then n_iterations of (linearize, solve,
@@ -158,6 +163,10 @@ class BatchedSCP:
         (SequenceController(u, tf_u, tf_sim=interval), control.py:217) under the full dynamics."""
         y = np.ascontiguousarray(y0, dtype=np.float64)
         N = y.shape[0]
+        if _lib.sat_consts(self.const, N)[0] is not None:
+            raise NotImplementedError("run_segments with per-satellite constants: the flight runs in the Simulator's one "
+                                      "scale, and carrying each controller's plan across that unit boundary is not "
+                                      "implemented")
         traj, plans = [], []
         for _ in range(n_segments):
             u_tab, lens, tf_u, hist = self._plan(y, solver)
