@@ -496,7 +496,7 @@ typedef struct mpc_sat_consts {
  *   consts_scratch  DEVICE scratch of n_sats * MPC_SAT_SCRATCH_DOUBLES doubles, which the call fills.
  * Not available (MPC_E_UNSUPPORTED): the drag linearisation (include_drag in the discretization), the fixed-step RK4
  * propagator, u on its own grid, the round-1 default-mode kernel (mpc_set_tuning(9)), the fused overlapped pass and the
- * multi-GPU gather entry points.
+ * rectangular multi-GPU gather entry points (mpc_discretize_batch_ragged_gather takes per-satellite constants).
  *
  * mpc_discretize_batch_units: mpc_discretize_batch_ragged with per-satellite constants; K_sat == NULL means a rectangular
  * batch (K = K_max nodes for every satellite; `first` is then not used and may be NULL).  The fixed-step form always
@@ -513,6 +513,28 @@ int mpc_discretize_batch_units_host(mpc_ctx *ctx, const double *x, const double 
                                     const mpc_sat_consts *consts, int n_sats, int K_max, const int32_t *K_sat, int adaptive,
                                     int n_sub, double rtol, double atol, double max_step, double *out_host,
                                     int32_t *status_host, int32_t *n_nodes_host);
+
+/*
+ * mpc_discretize_batch_ragged_gather: one rank's shard of a ragged batch (multi-GPU, satellites sharded over ranks), every
+ * result stored into every rank's gathered buffer.  The gathered layout is the single-GPU ragged layout at a fixed
+ * capacity K_cap: global satellite g on columns g (K_cap - 1) + k, k < K_g - 1.  A rank holding satellites [s0, s1)
+ * passes x [n_sats][7][K_cap], u [n_sats][3][K_cap], tf [n_sats] of those satellites, its own counts K_sat (HOST, each
+ * 2 <= K_s <= K_cap; `first` is their DEVICE scratch of n_sats + 1 prefix sums) and out_offset = s0 (K_cap - 1).
+ *   consts      NULL: one constants bag (p), as mpc_discretize_batch_ragged; else per-satellite constants [n_sats] with
+ *               their consts_scratch, as mpc_discretize_batch_units.
+ *   adaptive    0: fixed step (n_sub), 1: the default quadrature mode (rtol, atol, max_step; n_nodes may be NULL).
+ *   dst         n_dst (1, 2, 4 or 8) buffers [105][out_pitch] (the own one first: it also holds the default mode's scratch
+ *               rows while the kernel runs; the others typically peer-mapped).  Padding columns are never written.
+ *   skip_const  0: rows 42..48 stored everywhere; 1: to dst[0] only; 2: nowhere (buffers filled once by
+ *               mpc_fill_const_rows).
+ *   status, n_nodes  [n_sats (K_cap - 1)] of this rank (not gathered), padding not written.
+ * Satellite s comes out bit for bit as in mpc_discretize_batch_ragged / _units.  Not available: include_drag.
+ */
+int mpc_discretize_batch_ragged_gather(const double *x, const double *u, const double *tf, const mpc_params *p,
+                                       const mpc_sat_consts *consts, int n_sats, int K_cap, const int32_t *K_sat, int64_t *first,
+                                       double *consts_scratch, int adaptive, int n_sub, double rtol, double atol,
+                                       double max_step, double *const *dst, int n_dst, int64_t out_pitch, int64_t out_offset,
+                                       int skip_const, int32_t *status, int32_t *n_nodes, void *stream);
 
 /*
  * mpc_propagate_batch_rk45_units: mpc_propagate_batch_rk45_ragged with per-satellite constants (mu, kj2, 1/(g0 isp) and,

@@ -14,9 +14,10 @@ import numpy as np
 _HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(_HERE, "csrc")
 SO_PATH = os.path.join(CSRC, "libmpc_b200.so")
-# the drag-branch kernels and the per-satellite-constants kernels have a translation unit each
-SOURCES = ["mpc_b200.cu", "mpc_b200_drag.cu", "mpc_b200_units.cu"]
-HEADERS = ["discretize_kernel.cuh", "discretize_adaptive_kernel.cuh", "discretize_default_kernel.cuh", "propagate_kernel.cuh", "propagate_rk45_kernel.cuh", "discretize_group_kernel.cuh", "constraint_terms_kernel.cuh", "discretize_drag_kernel.cuh", "discretize_pair_kernel.cuh", "mpc_b200_drag.h", "mpc_b200_units.h", os.path.join("..", "..", "include", "mpc_b200.h")]
+# the drag-branch kernels, the per-satellite-constants kernels and the multi-destination ragged kernels have a
+# translation unit each
+SOURCES = ["mpc_b200.cu", "mpc_b200_drag.cu", "mpc_b200_units.cu", "mpc_b200_shard.cu"]
+HEADERS = ["discretize_kernel.cuh", "discretize_adaptive_kernel.cuh", "discretize_default_kernel.cuh", "propagate_kernel.cuh", "propagate_rk45_kernel.cuh", "discretize_group_kernel.cuh", "constraint_terms_kernel.cuh", "discretize_drag_kernel.cuh", "discretize_pair_kernel.cuh", "mpc_b200_drag.h", "mpc_b200_units.h", "mpc_b200_shard.h", os.path.join("..", "..", "include", "mpc_b200.h")]
 # No -split-compile: with it nvcc partitions the module for parallel compilation and the register allocation of the
 # 250-register kernels comes out differently from build to build (the same source gave discretize_default_kernel 253
 # registers / 296 B of stack in one build and 255 / 536 B in the next: 1.366 vs 1.390 ms on BASELINE configs[2];
@@ -171,6 +172,8 @@ def lib():
     L.mpc_dynamics_jacobian_ragged.argtypes = [_DP, i64, i64, i, i, _DP, _DP, _DP, _DP, _DP, vp]
     L.mpc_discretize_batch_units.argtypes = [_DP, _DP, _DP, pp, _DP, i, i, _DP, _DP, _DP, i, i, d, d, d, _DP, i64, i64, _DP, _DP, vp]
     L.mpc_discretize_batch_units_host.argtypes = [vp, _DP, _DP, _DP, pp, _DP, i, i, _DP, i, i, d, d, d, _DP, _DP, _DP]
+    L.mpc_discretize_batch_ragged_gather.argtypes = [_DP, _DP, _DP, pp, _DP, i, i, _DP, _DP, _DP, i, i, d, d, d,
+                                                     ctypes.POINTER(ctypes.c_void_p), i, i64, i64, i, _DP, _DP, vp]
     L.mpc_propagate_batch_rk45_units.argtypes = [_DP, _DP, pp, _DP, pc, i, i, _DP, _DP, _DP, d, d, d, _DP, _DP, _DP, _DP, vp]
     L.mpc_propagate_batch_rk45_units_host.argtypes = [vp, _DP, _DP, pp, _DP, pc, i, i, _DP, _DP, d, d, d, _DP, _DP, _DP, _DP]
     L.mpc_constraint_terms_units.argtypes = [_DP, _DP, i, i, _DP, _DP, _DP, _DP, _DP, _DP, _DP, vp]
@@ -188,7 +191,7 @@ def lib():
                  "mpc_constraint_terms_host", "mpc_discretize_batch_push", "mpc_fill_const_rows", "mpc_dynamics_jacobian",
                  "mpc_constraint_terms_ragged", "mpc_constraint_terms_ragged_host", "mpc_dynamics_jacobian_ragged",
                  "mpc_discretize_batch_units", "mpc_discretize_batch_units_host", "mpc_propagate_batch_rk45_units",
-                 "mpc_propagate_batch_rk45_units_host", "mpc_constraint_terms_units", "mpc_constraint_terms_units_host"):
+                 "mpc_propagate_batch_rk45_units_host", "mpc_discretize_batch_ragged_gather", "mpc_constraint_terms_units", "mpc_constraint_terms_units_host"):
         getattr(L, name).restype = i
     _lib = L
     return L
@@ -208,7 +211,7 @@ EXPORTED_SYMBOLS = [
     "mpc_constraint_terms_ragged", "mpc_constraint_terms_ragged_host", "mpc_dynamics_jacobian_ragged",
     "mpc_discretize_batch_units", "mpc_discretize_batch_units_host", "mpc_propagate_batch_rk45_units",
     "mpc_propagate_batch_rk45_units_host", "mpc_constraint_terms_units", "mpc_constraint_terms_units_host",
-    "mpc_fp64_peak_probe", "mpc_set_tuning", "mpc_set_gather_tuning",
+    "mpc_discretize_batch_ragged_gather", "mpc_fp64_peak_probe", "mpc_set_tuning", "mpc_set_gather_tuning",
 ]
 
 

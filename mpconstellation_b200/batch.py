@@ -464,11 +464,12 @@ def discretize_batch_device(x, u, tf, const, include_J2=False, n_sub=100, out=No
 
 
 def propagate_batch_device(y0, tf, controller, const, include_drag=True, include_J2=True, T=100, n_sub=None,
-                           y=None, u_out=None, status=None):
+                           y=None, u_out=None, status=None, T_max=None):
     """Device form of propagate_batch: y0 [N,7], tf [N] float64 CUDA tensors -> y [N,7,T], u [N,3,T], status [N].
     T = int array [N] (host): satellite s sampled at linspace(0, 1, T_s) into the first T_s columns of y / u [.,.,Tmax]
     (the padding columns are not written), the reference integrator only, as propagate_batch; so is a sequence law
-    with per-satellite table lengths (ControllerSpec.table_len).
+    with per-satellite table lengths (ControllerSpec.table_len).  T_max: the column stride of y / u of such a batch
+    (default max T_s; a fixed capacity keeps the layout of a buffer whose counts change from call to call).
     const: one Constants bag or a sequence of N, as in propagate_batch."""
     torch = _torch()
     N = y0.shape[0]
@@ -480,6 +481,10 @@ def propagate_batch_device(y0, tf, controller, const, include_drag=True, include
     if np.ndim(T) != 0:
         T_sat = _counts(T, N, int(np.max(T)) if N else 2, "T")
         T = int(T_sat.max()) if N else 2
+        if T_max is not None:
+            if int(T_max) < T:
+                raise ValueError(f"T_max = {T_max} is below the largest count {T}")
+            T = int(T_max)
     T = int(T)
     if (T_sat is not None or tab_len is not None) and n_sub not in (None, 0):
         raise ValueError("per-satellite sample counts / table lengths need the reference integrator (n_sub=None)")

@@ -95,7 +95,9 @@ __device__ __forceinline__ void df_store_stage(volatile double *sm, int s, const
 // PSC: per-satellite constants (discretize_default_units_kernel): the thread of satellite `sat` reads psc[sat] where the
 // others read P.  The table is read where the constants are used, inside the step loop (it is not __restrict__: the
 // stores to the output buffer keep the loads where they are), so that this 254-register body keeps no more values live.
-template <bool J2, int BLOCK, bool GENU, bool DRAG, bool RAG = false, bool PSC = false>
+// NDST: the results are stored into dst.p[0 .. NDST-1] (the fused all-gather of a sharded batch); the Phi scratch rows
+// stay in dst.p[0], the local buffer.
+template <bool J2, int BLOCK, bool GENU, bool DRAG, bool RAG = false, bool PSC = false, int NDST = 1>
 __device__ __forceinline__ void
 discretize_default_body(const double *__restrict__ x_in, const double *__restrict__ u_in,
                         const double *__restrict__ tf_arr, const DiscParams &P0, int n_sats, int K, int Ku, double rtol, double atol,
@@ -467,7 +469,7 @@ discretize_default_body(const double *__restrict__ x_in, const double *__restric
         }
 #pragma unroll
     for (int q = 0; q < 8; ++q) SM(48 + q) = row6[(long long)q * pitch];   // (the stage slots are dead by now)
-    const int nonfinite = epilogue_store<BLOCK, 1>(sm, pr, pv, tf, 1.0, tf, dst, pitch, offset + gid);
+    const int nonfinite = epilogue_store<BLOCK, NDST>(sm, pr, pv, tf, 1.0, tf, dst, pitch, offset + gid);
     if (status) status[gid] = bad ? 1 : (nonfinite ? 2 : (fail ? 3 : 0));
     if (n_nodes) n_nodes[gid] = nodes;
 }
@@ -526,6 +528,33 @@ discretize_default_units_kernel(const double *__restrict__ x_in, const double *_
 {
     discretize_default_body<J2, BLOCK, false, false, RAG, true>(x_in, u_in, tf_arr, psc[0], n_sats, K, K, rtol, atol, max_step,
                                                                 dst, pitch, offset, status, n_nodes, 0.0, nullptr, first, psc);
+}
+
+// ragged batch (with or without per-satellite constants) stored into NDST > 1 buffers: one rank's shard of the fused
+// all-gather (mpc_discretize_batch_ragged_gather).  The signatures are those of the single-destination forms above.
+template <bool J2, int BLOCK, int NDST>
+__global__ void __launch_bounds__(BLOCK)
+discretize_default_ragged_multi_kernel(const double *__restrict__ x_in, const double *__restrict__ u_in,
+                                       const double *__restrict__ tf_arr, DiscParams P, int n_sats, int K, double rtol,
+                                       double atol, double max_step, DstTab dst, long long pitch, long long offset,
+                                       int32_t *__restrict__ status, int32_t *__restrict__ n_nodes,
+                                       const long long *__restrict__ first)
+{
+    discretize_default_body<J2, BLOCK, false, false, true, false, NDST>(x_in, u_in, tf_arr, P, n_sats, K, K, rtol, atol, max_step,
+                                                                        dst, pitch, offset, status, n_nodes, 0.0, nullptr, first);
+}
+
+template <bool J2, int BLOCK, int NDST>
+__global__ void __launch_bounds__(BLOCK)
+discretize_default_units_multi_kernel(const double *__restrict__ x_in, const double *__restrict__ u_in,
+                                      const double *__restrict__ tf_arr, const DiscParams *psc, int n_sats, int K, double rtol,
+                                      double atol, double max_step, DstTab dst, long long pitch, long long offset,
+                                      int32_t *__restrict__ status, int32_t *__restrict__ n_nodes,
+                                      const long long *__restrict__ first)
+{
+    discretize_default_body<J2, BLOCK, false, false, true, true, NDST>(x_in, u_in, tf_arr, psc[0], n_sats, K, K, rtol, atol,
+                                                                       max_step, dst, pitch, offset, status, n_nodes, 0.0, nullptr,
+                                                                       first, psc);
 }
 
 }  // namespace mpc

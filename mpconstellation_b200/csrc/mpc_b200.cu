@@ -23,6 +23,7 @@
 #include "propagate_rk45_kernel.cuh"
 #include "mpc_b200_drag.h"
 #include "mpc_b200_units.h"
+#include "mpc_b200_shard.h"
 #include "constraint_terms_kernel.cuh"
 #include "discretize_drag_kernel.cuh"
 #include "discretize_pair_kernel.cuh"
@@ -1533,6 +1534,77 @@ int mpc_discretize_batch_units(const double *x, const double *u, const double *t
     return launch_units_disc(x, u, tf, (const mpc::DiscParams *)consts_scratch, p->include_j2, n_sats, K_max, n_units,
                              K_sat ? (const long long *)first : nullptr, adaptive ? &o : nullptr, n_sub, tab, out_pitch,
                              out_offset, status, st);
+}
+
+// ---- one rank's shard of a ragged batch, stored into every rank's gathered buffer ----------------------------------------
+int mpc_discretize_batch_ragged_gather(const double *x, const double *u, const double *tf, const mpc_params *p,
+                                       const mpc_sat_consts *consts, int n_sats, int K_cap, const int32_t *K_sat, int64_t *first,
+                                       double *consts_scratch, int adaptive, int n_sub, double rtol, double atol,
+                                       double max_step, double *const *dst, int n_dst, int64_t out_pitch, int64_t out_offset,
+                                       int skip_const, int32_t *status, int32_t *n_nodes, void *stream)
+{
+    int rc = consts ? check_units_disc(x, u, tf, p, consts, n_sats, K_cap, K_sat, adaptive, n_sub, rtol, atol, max_step)
+                    : check_ragged_disc(x, u, tf, p, n_sats, K_cap, K_sat, adaptive, n_sub, rtol, atol, max_step);
+    if (rc) return rc;
+    if (!K_sat || !first) return fail(MPC_E_INVALID, "null K_sat / first");
+    if (!dst || (n_dst != 1 && n_dst != 2 && n_dst != 4 && n_dst != 8))
+        return fail(MPC_E_INVALID, "n_dst must be 1, 2, 4 or 8 (got %d)", n_dst);
+    for (int d = 0; d < n_dst; ++d)
+        if (!dst[d]) return fail(MPC_E_INVALID, "null destination %d", d);
+    if (skip_const < 0 || skip_const > 2) return fail(MPC_E_INVALID, "skip_const must be 0, 1 or 2 (got %d)", skip_const);
+    if (out_pitch < out_offset + (long long)n_sats * (K_cap - 1) || out_offset < 0)
+        return fail(MPC_E_INVALID, "out_pitch/out_offset do not hold the batch");
+    if (n_sats == 0) return MPC_SUCCESS;
+    cudaStream_t st = (cudaStream_t)stream;
+    if (consts && (rc = upload_sat_table<mpc::DiscParams>(p, consts, n_sats, consts_scratch, st, disc_params))) return rc;
+    const std::vector<long long> f = ragged_first(K_sat, n_sats);
+    CUDA_TRY(cudaMemcpyAsync(first, f.data(), f.size() * sizeof(long long), cudaMemcpyHostToDevice, st));
+    const long long *fd = (const long long *)first;
+    mpc::DstTab tab{};
+    for (int d = 0; d < n_dst; ++d) tab.p[d] = dst[d];
+    tab.skip_const = skip_const;
+    const AdaptiveOpts o{rtol, atol, max_step, n_nodes};
+    const AdaptiveOpts *ad = adaptive ? &o : nullptr;
+    const mpc::DiscParams P = disc_params(p);
+    if (n_dst == 1) {   // the single-GPU launches
+        if (consts)
+            return launch_units_disc(x, u, tf, (const mpc::DiscParams *)consts_scratch, p->include_j2, n_sats, K_cap, f[n_sats], fd,
+                                     ad, n_sub, tab, out_pitch, out_offset, status, st);
+        return p->include_j2 ? launch_ragged<true>(x, u, tf, P, n_sats, K_cap, f[n_sats], fd, ad, n_sub, tab, out_pitch, out_offset, status, st)
+                             : launch_ragged<false>(x, u, tf, P, n_sats, K_cap, f[n_sats], fd, ad, n_sub, tab, out_pitch, out_offset, status, st);
+    }
+    // the block sizes launch_ragged / launch_units_disc choose from the live count (default mode: 32 or 256 threads, the
+    // 128-thread CTA of mpc_set_tuning(21) has no multi-destination build)
+    tab.em = em_level();
+    MpcUnitsDisc a{};
+    a.x = x;
+    a.u = u;
+    a.tf = tf;
+    a.psc = consts ? consts_scratch : nullptr;
+    a.dst_tab = &tab;
+    a.first = fd;
+    a.n_units = f[n_sats];
+    a.include_j2 = p->include_j2;
+    a.n_sats = n_sats;
+    a.K = K_cap;
+    a.n_sub = n_sub;
+    a.adaptive = adaptive;
+    if (adaptive) {
+        a.block = a.n_units < 148LL * 256 ? 32 : 256;
+        a.rtol = rtol;
+        a.atol = atol;
+        a.max_step = max_step;
+        a.n_nodes = n_nodes;
+    } else {
+        a.block = (a.n_units > 148LL * 32 && a.n_units <= 148LL * 128) || a.n_units >= 148LL * 9 * 32 * 2 ? kDiscBlock : 32;
+    }
+    a.pitch = out_pitch;
+    a.offset = out_offset;
+    a.status = status;
+    a.stream = st;
+    CUDA_TRY(mpc_shard_launch_disc(&a, &P, n_dst));
+    g_launches.fetch_add(1, std::memory_order_relaxed);
+    return MPC_SUCCESS;
 }
 
 int mpc_discretize_batch_units_host(mpc_ctx *ctx, const double *x, const double *u, const double *tf, const mpc_params *p,

@@ -18,7 +18,14 @@ Two implementations of the exchange:
 
 `GatheredView` hands out the reference-shaped per-satellite views of either result, so optimizer-side code
 indexes exactly as before (optimizer.py:327-339).
+
+`RaggedGather` is the sharded linearization of the batches `BatchedSCP` produces after the first solve: every satellite on
+its own grid K_s and / or in its own designer units.  Satellites are split by live intervals (`shard_ranges_by_work`),
+the ragged discretization kernels store into every rank's buffer (`mpc_discretize_batch_ragged_gather`) and the
+reference trajectories follow by one copy per peer.
 """
+from dataclasses import dataclass
+
 import numpy as np
 
 from . import _lib
@@ -34,6 +41,23 @@ def shard_range(n_sats, rank, world):
     per = (n_sats + world - 1) // world
     s0 = min(n_sats, rank * per)
     return s0, min(n_sats, s0 + per)
+
+
+def shard_ranges_by_work(K_sat, world):
+    """Contiguous satellite ranges [(s0, s1)] * world balanced by live intervals sum(K_s - 1), not by satellite count
+    (the discretization sets the balance: the propagation costs about the same per satellite up to far larger batches).
+    Rank r takes the satellites up to the first prefix sum >= r ceil(total / world), so each rank's live count is at
+    most ceil(total / world) + max(K_s - 1) - 1.  Ranges may be empty (world > N included)."""
+    w = np.asarray(K_sat, dtype=np.int64).reshape(-1) - 1
+    if world < 1:
+        raise ValueError(f"world must be >= 1, got {world}")
+    if w.size and w.min() < 1:
+        raise ValueError("every K_s must be >= 2")
+    prefix = np.concatenate([[0], np.cumsum(w)])
+    target = -(-int(prefix[-1]) // world)
+    edges = [0] + [int(np.searchsorted(prefix, r * target, side="left")) for r in range(1, world)] + [int(w.size)]
+    edges = [min(e, int(w.size)) for e in edges]
+    return [(edges[r], max(edges[r], edges[r + 1])) for r in range(world)]
 
 
 def _np(a):
@@ -275,3 +299,234 @@ def assemble_rank_major(chunks, bounds, world):
     for t, (c0, c1) in zip(chunks, bounds):
         full[:, :, c0:c1] = t
     return full
+
+
+@dataclass
+class ShardedLinearization:
+    """Result of RaggedGather.linearize on every rank, device-resident and in the single-GPU ragged layout at the
+    capacity K_cap (views of the gatherer's buffers: the next linearize overwrites them; padding columns are not written).
+      soa     [105, N (K_cap - 1)]: satellite s on columns s (K_cap - 1) + k, k < K_s - 1
+      x_bar   [N, 7, K_cap], u_bar [N, 3, K_cap]: the reference trajectories (first K_s columns of satellite s)
+      tf [N], K_sat [N] (host int32), const: what the pass ran with
+      n_nodes [s1 - s0, K_cap - 1] (default mode): node counts of THIS rank's satellites ranges[rank] only
+    Feeds the hand-off as the single-GPU result does: constraint_terms_device(x_bar, u_bar, const, K=K_sat),
+    dynamics_jacobian_device(soa, N, K_cap, K_sat=K_sat)."""
+    soa: object
+    x_bar: object
+    u_bar: object
+    tf: object
+    K_sat: np.ndarray
+    const: object
+    ranges: list
+    n_nodes: object = None
+
+    def sat(self, s):
+        """(A_k, B_kp, B_kn, Sigma_k, xi_k) of GLOBAL satellite s on its K_s - 1 intervals; shapes of
+        linearize_discretize.py:390 (device tensors)."""
+        from .batch import DiscretizedBatch
+        return DiscretizedBatch(self.soa, None, len(self.K_sat), self.x_bar.shape[2], K_sat=self.K_sat).sat(s)
+
+
+def _shard_spec(spec, s0, s1):
+    """the controller law of satellites [s0, s1): the per-satellite tables / end_tau / table lengths sliced"""
+    from .control import ControllerSpec
+    tab = spec.table
+    if tab is not None and np.ndim(tab) == 3:
+        tab = np.ascontiguousarray(np.asarray(tab)[s0:s1])
+    end_tau = spec.end_tau if np.ndim(spec.end_tau) == 0 else np.asarray(spec.end_tau)[s0:s1]
+    lens = None if spec.table_len is None else np.asarray(spec.table_len)[s0:s1]
+    return ControllerSpec(spec.kind, spec.thrust, tab, end_tau, lens)
+
+
+def _raise_status(code, what):
+    """the exceptions of batch.raise_on_status for a status code combined over the ranks"""
+    if code == _lib.ST_MASS:
+        # same exception type / text as simulator.py:135-136
+        raise Exception(f"ERROR: INVALID SATELLITE MASS: non-positive mass in the sharded {what}")
+    if code == _lib.ST_STEP:
+        raise RuntimeError(f"adaptive integration failed (step size underflow) in the sharded {what}")
+    raise FloatingPointError(f"non-finite result in the sharded {what}")
+
+
+class RaggedGather:
+    """Sharded SCP linearization of a ragged and / or per-satellite-units constellation over the ranks of one box.
+
+    The buffers -- matrices [105, N (K_cap - 1)], x_bar [N, 7, K_cap], u_bar [N, 3, K_cap] -- are ONE symmetric-memory
+    allocation made here, once: the node counts change from one SCP iteration to the next, the layout (capacity K_cap)
+    does not, so no allocation or rendezvous happens per call.  Each rank takes the contiguous satellite range
+    shard_ranges_by_work gives it for the call's counts.  On a gloo group (CPU tensors) the buffers are plain tensors and
+    the exchange is a broadcast of every rank's blocks; the computation itself needs CUDA (_compute)."""
+
+    def __init__(self, n_sats, K_cap, group=None, device=None, skip_const=True):
+        import torch
+        import torch.distributed as dist
+        if n_sats < 0 or K_cap < 2:
+            raise ValueError(f"need n_sats >= 0 and K_cap >= 2 (got {n_sats}, {K_cap})")
+        self.group = dist.group.WORLD if group is None else group
+        self.world = dist.get_world_size(self.group)
+        self.rank = dist.get_rank(self.group)
+        self.n_sats, self.K_cap = int(n_sats), int(K_cap)
+        self.pitch = self.n_sats * (self.K_cap - 1)
+        self.cuda = dist.get_backend(self.group) != "gloo"
+        if device is None:
+            device = torch.device("cuda", torch.cuda.current_device()) if self.cuda else torch.device("cpu")
+        self.device = torch.device(device)
+        n_buf, n_x = _lib.MPC_OUT_ROWS * self.pitch, self.n_sats * 7 * self.K_cap
+        n_all = n_buf + n_x + self.n_sats * 3 * self.K_cap
+        self._off = (0, n_buf, n_buf + n_x)             # element offsets of buf, x_bar, u_bar
+        if self.cuda:
+            import torch.distributed._symmetric_memory as symm_mem
+            self.flat = symm_mem.empty((max(1, n_all),), dtype=torch.float64, device=self.device)
+            self.handle = symm_mem.rendezvous(self.flat, self.group)
+        else:
+            self.flat, self.handle = torch.empty((max(1, n_all),), dtype=torch.float64), None
+        self.flat.fill_(float("nan"))
+        self.buf = self.flat[:n_buf].view(_lib.MPC_OUT_ROWS, self.pitch)
+        self.x_bar = self.flat[n_buf:n_buf + n_x].view(self.n_sats, 7, self.K_cap)
+        self.u_bar = self.flat[n_buf + n_x:n_all].view(self.n_sats, 3, self.K_cap)
+        self.skip_const = bool(skip_const) and self.world > 1
+        if self.cuda:
+            ptrs = [int(p) for p in self.handle.buffer_ptrs]
+            self._base = (self.flat.data_ptr() - ptrs[self.rank]) // 8     # the tensor's place in its allocation
+            # own buffer first (the kernel's local destination), then the peers rotated as in FusedGather, padded to
+            # 1/2/4/8 with the own one
+            order = [(self.rank + i) % self.world for i in range(self.world)]
+            self.peers = order[1:]
+            self.dst = [ptrs[r] + 8 * self._base for r in order]
+            while len(self.dst) < _dst_count(self.world):
+                self.dst.append(self.dst[0])
+        if self.skip_const and self.pitch:
+            # rows 42..48 (the last row of A_k: constants 0..0 1) are written once into every buffer here, never sent
+            if self.cuda:
+                _lib.check(_lib.lib().mpc_fill_const_rows(self.buf.data_ptr(), self.pitch,
+                                                          torch.cuda.current_stream(self.device).cuda_stream))
+                torch.cuda.synchronize(self.device)
+            else:
+                self.buf[42:49] = 0.0
+                self.buf[48] = 1.0
+        self._barrier()
+
+    def _barrier(self, channel=0):
+        import torch.distributed as dist
+        if self.world == 1:
+            return
+        if self.cuda:
+            self.handle.barrier(channel=channel)
+        else:
+            dist.barrier(self.group)
+
+    def linearize(self, y0, tf, controller, const, K_sat, include_J2=False, use_uniform_steps=False, integrator_steps=101,
+                  check=True, pre_barrier=True):
+        """One SCP linearization pass of the whole constellation, sharded: run_nonlinear + extract_uk + discretize of
+        every satellite on its own K_s nodes (and, with N Constants, in its own units), as BatchedSCP.linearize computes
+        it on one GPU.  Every rank passes the FULL inputs: y0 [N,7], tf [N] (numpy or tensors), controller (a sequence law
+        may carry per-satellite tables / table lengths), const (one bag or N), K_sat [N] (2 <= K_s <= K_cap).
+        Each rank propagates its shard (RK45 replay, no drag / J2, as OptimalController.run_nonlinear), discretizes it
+        into every rank's buffer, copies its x_bar / u_bar block to every peer and meets the others at a barrier; then
+        the status words are combined over the ranks (max), and with check=True a non-positive mass raises the
+        reference's Exception on every rank (non-finite results / step underflow raise as in raise_on_status).
+        pre_barrier: see FusedGather._pre_barrier.  Returns a ShardedLinearization."""
+        import torch
+        import torch.distributed as dist
+        from .control import spec_from
+        N, Kc = self.n_sats, self.K_cap
+        K_sat = np.ascontiguousarray(K_sat, dtype=np.int32)
+        if K_sat.shape != (N,) or (N and (K_sat.min() < 2 or K_sat.max() > Kc)):
+            raise ValueError(f"K_sat must be [{N}] with every count in [2, {Kc}]")
+        y0 = torch.as_tensor(y0, dtype=torch.float64).to(self.device).contiguous()
+        tfv = torch.as_tensor(tf, dtype=torch.float64, device=self.device).reshape(-1).expand(N).contiguous()
+        if y0.shape != (N, 7):
+            raise ValueError(f"y0 must be [{N}, 7], got {tuple(y0.shape)}")
+        one_bag = hasattr(const, "MU")
+        if not one_bag and len(const) != N:          # (the bags themselves are checked where they are packed)
+            raise ValueError(f"per-satellite constants: expected {N} Constants, got {len(const)}")
+        ranges = shard_ranges_by_work(K_sat, self.world)
+        s0, s1 = ranges[self.rank]
+        shard_const = const if one_bag else list(const)[s0:s1]
+        spec = _shard_spec(spec_from(controller), s0, s1)
+        adaptive = None if use_uniform_steps else dict(rtol=1e-3, atol=1e-6, max_step=1e-2)
+        n_nodes = None if use_uniform_steps else torch.zeros(((s1 - s0), Kc - 1), dtype=torch.int32, device=self.device)
+        if self.world == 1:
+            # the single-GPU calls, into the same buffers
+            if N:
+                from . import batch
+                _, _, st_prop = batch.propagate_batch_device(y0, tfv, spec, const, include_drag=False, include_J2=False,
+                                                             T=K_sat, T_max=Kc, y=self.x_bar, u_out=self.u_bar)
+                _, st_disc = batch.discretize_batch_device(self.x_bar, self.u_bar, tfv, const, include_J2=include_J2,
+                                                           n_sub=integrator_steps - 1, out=self.buf, adaptive=adaptive,
+                                                           n_nodes=n_nodes, K=K_sat)
+                words = torch.stack([st_prop.max(), st_disc.max()])
+            else:
+                words = torch.zeros(2, dtype=torch.int32, device=self.device)
+        else:
+            if pre_barrier:
+                self._barrier(channel=1)
+            words = self._compute(y0[s0:s1], tfv[s0:s1], spec, shard_const, K_sat[s0:s1], s0, include_J2, adaptive,
+                                  integrator_steps - 1, n_nodes)
+            self._publish(ranges)
+            self._barrier()
+            dist.all_reduce(words, op=dist.ReduceOp.MAX, group=self.group)
+        if check:
+            codes = words.tolist()
+            if codes[0]:
+                _raise_status(codes[0], "propagation")
+            if codes[1]:
+                _raise_status(codes[1], "discretization")
+        res = ShardedLinearization(self.buf, self.x_bar, self.u_bar, tfv, K_sat, const, ranges, n_nodes)
+        res.status = words
+        return res
+
+    def _compute(self, y0, tf, spec, const, K_sat, s0, include_J2, adaptive, n_sub, n_nodes):
+        """this rank's shard: propagate into the own x_bar / u_bar rows, discretize into every rank's buffer; returns the
+        device int32 [2] (max propagation status, max discretization status) of the shard"""
+        import ctypes
+        import torch
+        from . import batch
+        n, Kc = y0.shape[0], self.K_cap
+        if n == 0:
+            return torch.zeros(2, dtype=torch.int32, device=self.device)
+        x, u = self.x_bar[s0:s0 + n], self.u_bar[s0:s0 + n]
+        _, _, st_prop = batch.propagate_batch_device(y0, tf, spec, const, include_drag=False, include_J2=False, T=K_sat,
+                                                     T_max=Kc, y=x, u_out=u)
+        psc, one = batch._units_of(const, n)
+        p = _lib.make_params(one, include_J2, False)
+        cur = torch.cuda.current_stream(self.device)
+        status = torch.zeros(n * (Kc - 1), dtype=torch.int32, device=self.device)
+        first = torch.empty(n + 1, dtype=torch.int64, device=self.device)
+        scratch = torch.empty(n * _lib.SAT_SCRATCH_DOUBLES, dtype=torch.float64, device=self.device) if psc is not None else None
+        arr = (ctypes.c_void_p * len(self.dst))(*self.dst)
+        ad = adaptive or {}
+        _lib.check(_lib.lib().mpc_discretize_batch_ragged_gather(
+            x.data_ptr(), u.data_ptr(), tf.data_ptr(), ctypes.byref(p), psc, n, Kc, _lib.addr(K_sat), first.data_ptr(),
+            scratch.data_ptr() if scratch is not None else None, int(adaptive is not None), int(n_sub),
+            float(ad.get("rtol", 1e-3)), float(ad.get("atol", 1e-6)), float(ad.get("max_step", 1e-2)), arr, len(self.dst),
+            self.pitch, s0 * (Kc - 1), 1 if self.skip_const else 0, status.data_ptr(),
+            n_nodes.data_ptr() if n_nodes is not None else None, cur.cuda_stream))
+        for t_ in (first, scratch):
+            if t_ is not None:
+                t_.record_stream(cur)
+        return torch.stack([st_prop.max(), status.max()])
+
+    def _publish(self, ranges):
+        """x_bar / u_bar rows of this rank's satellites into every peer's buffers: one copy per peer and array (the
+        matrices are already there: the kernel stored them).  gloo: every rank's blocks broadcast from their owner."""
+        import torch.distributed as dist
+        Kc = self.K_cap
+        if self.cuda:
+            s0, s1 = ranges[self.rank]
+            if s1 == s0:
+                return
+            for off, rows, arr in ((self._off[1], 7, self.x_bar), (self._off[2], 3, self.u_bar)):
+                n_el = (s1 - s0) * rows * Kc
+                src = arr[s0:s1].reshape(-1)
+                for r in self.peers:
+                    self.handle.get_buffer(r, (n_el,), src.dtype, self._base + off + s0 * rows * Kc).copy_(src)
+            return
+        for r, (a, b) in enumerate(ranges):
+            if b == a:
+                continue
+            for arr in (self.x_bar, self.u_bar):
+                dist.broadcast(arr[a:b], src=r, group=self.group)
+            blk = self.buf[:, a * (Kc - 1):b * (Kc - 1)].contiguous()
+            dist.broadcast(blk, src=r, group=self.group)
+            self.buf[:, a * (Kc - 1):b * (Kc - 1)] = blk
