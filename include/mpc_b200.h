@@ -55,6 +55,7 @@ extern "C" {
 #define MPC_ST_MASS 1      /* mass <= 0 met while integrating: simulator.py:135-136 raises here */
 #define MPC_ST_NONFINITE 2 /* a non-finite result */
 #define MPC_ST_STEP 3      /* adaptive mode: step size underflow / too many steps (solve_ivp would fail) */
+#define MPC_ST_ATMO 4      /* mpc_propagate_batch_rk45_atmo: an altitude outside the fitted atmosphere's range */
 
 /* Normalized constants: the reference's Constants bag (constants.py:11-20) as produced by
  * SatelliteScale.get_normalized_constants (satellite_scale.py:36-44), plus the two module-level
@@ -553,6 +554,45 @@ int mpc_propagate_batch_rk45_units_host(mpc_ctx *ctx, const double *y0, const do
                                         const int32_t *T_sat, const int32_t *table_len_sat, double rtol, double atol,
                                         double max_step, double *y_host, double *u_host, int32_t *status_host,
                                         int32_t *n_steps_host);
+
+/* ---------------------------------------------------------------- altitude-dependent atmosphere */
+
+/*
+ * A density model of the propagator's drag: log rho (kg/m^3) as a Chebyshev series sum_k coef[k] T_k(t) in
+ * t = (log h - (log h_min + log h_max) / 2) * 2 / (log h_max - log h_min), h the altitude in metres, valid on
+ * [h_min, h_max].  Fitted and checked against the user's rho(h) by mpconstellation_b200.fit_atmosphere.
+ * Satellite s flies at the altitude h = |r| L - r_earth, L = r_earth / r_e the metres per unit length of its constants
+ * (SatelliteScale: r_e = R_EARTH / r0, so L is its r0), and its drag acceleration is
+ *     -(0.5 c_d s_area / rho) rho(h) / m |v| v
+ * in those units: the dynamics of simulator.py:150-153 with rho(h) in place of Simulator.get_atmo_density.
+ */
+typedef struct mpc_atmosphere {
+    double h_min, h_max;  /* m, 0 < h_min < h_max */
+    double r_earth;       /* m */
+    int32_t n;            /* terms, 1 .. MPC_RHO_CHEB */
+    int32_t reserved;
+    double coef[32];
+} mpc_atmosphere;
+
+/*
+ * mpc_propagate_batch_rk45_atmo: the RK45 replay with drag under the atmosphere *atmo (passed by value to the kernel).
+ * The arguments of mpc_propagate_batch_rk45_units plus atmo; consts == NULL: one constants bag (p; consts_scratch is
+ * then not used and may be NULL), otherwise satellite s in the units of consts[s] (its own L and rho).  T_sat == NULL:
+ * a rectangular batch.  p->include_drag must be set (rho_atm is not read).  The first stage evaluation at an altitude
+ * outside [h_min, h_max] ends that satellite's run with status MPC_ST_ATMO (no extrapolation), as a non-positive mass
+ * ends it with MPC_ST_MASS.  MPC_E_INVALID: a bad atmosphere (n, range, non-finite coefficients), r_e <= 0, or drag off.
+ */
+int mpc_propagate_batch_rk45_atmo(const double *y0, const double *tf, const mpc_params *p, const mpc_sat_consts *consts,
+                                  const mpc_controller *ctrl, int n_sats, int T_max, const int32_t *T_sat,
+                                  const int32_t *table_len_sat, double *consts_scratch, double rtol, double atol,
+                                  double max_step, double *y, double *u_out, int32_t *status, int32_t *n_steps,
+                                  const mpc_atmosphere *atmo, void *stream);
+/* Host-buffer form: T_sat / table_len_sat are host arrays or NULL, as in mpc_propagate_batch_rk45_units_host. */
+int mpc_propagate_batch_rk45_atmo_host(mpc_ctx *ctx, const double *y0, const double *tf, const mpc_params *p,
+                                       const mpc_sat_consts *consts, const mpc_controller *ctrl, int n_sats, int T_max,
+                                       const int32_t *T_sat, const int32_t *table_len_sat, double rtol, double atol,
+                                       double max_step, double *y_host, double *u_host, int32_t *status_host,
+                                       int32_t *n_steps_host, const mpc_atmosphere *atmo);
 
 /*
  * mpc_constraint_terms_units: the terminal terms of satellite s with consts[s].mu (the only constant the constraint terms

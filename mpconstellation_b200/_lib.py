@@ -14,10 +14,10 @@ import numpy as np
 _HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(_HERE, "csrc")
 SO_PATH = os.path.join(CSRC, "libmpc_b200.so")
-# the drag-branch kernels, the per-satellite-constants kernels and the multi-destination ragged kernels have a
-# translation unit each
-SOURCES = ["mpc_b200.cu", "mpc_b200_drag.cu", "mpc_b200_units.cu", "mpc_b200_shard.cu"]
-HEADERS = ["discretize_kernel.cuh", "discretize_adaptive_kernel.cuh", "discretize_default_kernel.cuh", "propagate_kernel.cuh", "propagate_rk45_kernel.cuh", "discretize_group_kernel.cuh", "constraint_terms_kernel.cuh", "discretize_drag_kernel.cuh", "discretize_pair_kernel.cuh", "mpc_b200_drag.h", "mpc_b200_units.h", "mpc_b200_shard.h", os.path.join("..", "..", "include", "mpc_b200.h")]
+# the drag-branch kernels, the per-satellite-constants kernels, the multi-destination ragged kernels and the RK45 replay
+# under an altitude-dependent atmosphere have a translation unit each
+SOURCES = ["mpc_b200.cu", "mpc_b200_drag.cu", "mpc_b200_units.cu", "mpc_b200_shard.cu", "mpc_b200_atmo.cu"]
+HEADERS = ["discretize_kernel.cuh", "discretize_adaptive_kernel.cuh", "discretize_default_kernel.cuh", "propagate_kernel.cuh", "propagate_rk45_kernel.cuh", "discretize_group_kernel.cuh", "constraint_terms_kernel.cuh", "discretize_drag_kernel.cuh", "discretize_pair_kernel.cuh", "mpc_b200_drag.h", "mpc_b200_units.h", "mpc_b200_shard.h", "mpc_b200_atmo.h", os.path.join("..", "..", "include", "mpc_b200.h")]
 # No -split-compile: with it nvcc partitions the module for parallel compilation and the register allocation of the
 # 250-register kernels comes out differently from build to build (the same source gave discretize_default_kernel 253
 # registers / 296 B of stack in one build and 255 / 536 B in the next: 1.366 vs 1.390 ms on BASELINE configs[2];
@@ -29,7 +29,7 @@ NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", 
 MPC_OUT_ROWS = 105
 ROW_A, ROW_BP, ROW_BN, ROW_SIGMA, ROW_XI = 0, 49, 70, 91, 98
 CTRL_ZERO, CTRL_CONSTANT, CTRL_TANGENTIAL, CTRL_SEQUENCE = 0, 1, 2, 3
-ST_OK, ST_MASS, ST_NONFINITE, ST_STEP = 0, 1, 2, 3
+ST_OK, ST_MASS, ST_NONFINITE, ST_STEP, ST_ATMO = 0, 1, 2, 3, 4
 FINAL_TERMS = 32
 # key -> (offset, length) inside the per-satellite terminal block (include/mpc_b200.h MPC_FT_*); length 0 = scalar
 FINAL_TERM_LAYOUT = {"rf_hat": (0, 3), "Vc": (3, 0), "DrVc": (4, 3), "DrVc_rbar": (7, 0), "Vt": (8, 0),
@@ -56,6 +56,12 @@ class MpcSatConsts(ctypes.Structure):
 
 
 SAT_SCRATCH_DOUBLES = 8    # MPC_SAT_SCRATCH_DOUBLES
+
+
+class MpcAtmosphere(ctypes.Structure):
+    """mpc_atmosphere: log rho as a Chebyshev series in log h over [h_min, h_max] (atmosphere.fit_atmosphere)"""
+    _fields_ = [("h_min", ctypes.c_double), ("h_max", ctypes.c_double), ("r_earth", ctypes.c_double),
+                ("n", ctypes.c_int32), ("reserved", ctypes.c_int32), ("coef", ctypes.c_double * 32)]
 
 
 class MpcController(ctypes.Structure):
@@ -176,6 +182,9 @@ def lib():
                                                      ctypes.POINTER(ctypes.c_void_p), i, i64, i64, i, _DP, _DP, vp]
     L.mpc_propagate_batch_rk45_units.argtypes = [_DP, _DP, pp, _DP, pc, i, i, _DP, _DP, _DP, d, d, d, _DP, _DP, _DP, _DP, vp]
     L.mpc_propagate_batch_rk45_units_host.argtypes = [vp, _DP, _DP, pp, _DP, pc, i, i, _DP, _DP, d, d, d, _DP, _DP, _DP, _DP]
+    pa = ctypes.POINTER(MpcAtmosphere)
+    L.mpc_propagate_batch_rk45_atmo.argtypes = [_DP, _DP, pp, _DP, pc, i, i, _DP, _DP, _DP, d, d, d, _DP, _DP, _DP, _DP, pa, vp]
+    L.mpc_propagate_batch_rk45_atmo_host.argtypes = [vp, _DP, _DP, pp, _DP, pc, i, i, _DP, _DP, d, d, d, _DP, _DP, _DP, _DP, pa]
     L.mpc_constraint_terms_units.argtypes = [_DP, _DP, i, i, _DP, _DP, _DP, _DP, _DP, _DP, _DP, vp]
     L.mpc_constraint_terms_units_host.argtypes = [vp, _DP, _DP, i, i, _DP, _DP, _DP, _DP, _DP]
     L.mpc_fp64_peak_probe.argtypes = [i, i, ctypes.POINTER(ctypes.c_double), ctypes.POINTER(ctypes.c_double)]
@@ -183,7 +192,7 @@ def lib():
     L.mpc_set_gather_tuning.restype = i
     L.mpc_set_tuning.argtypes = [i]
     L.mpc_set_tuning.restype = i
-    for name in ("mpc_propagate_discretize_host_layout", "mpc_discretize_batch_gather", "mpc_propagate_discretize_gather", "mpc_propagate_batch_rk45", "mpc_propagate_batch_rk45_host", "mpc_device_info", "mpc_discretize_batch", "mpc_discretize_batch_multi", "mpc_propagate_batch",
+    for name in ("mpc_propagate_batch_rk45_atmo", "mpc_propagate_batch_rk45_atmo_host", "mpc_propagate_discretize_host_layout", "mpc_discretize_batch_gather", "mpc_propagate_discretize_gather", "mpc_propagate_batch_rk45", "mpc_propagate_batch_rk45_host", "mpc_device_info", "mpc_discretize_batch", "mpc_discretize_batch_multi", "mpc_propagate_batch",
                  "mpc_discretize_batch_adaptive", "mpc_discretize_batch_adaptive_host",
                  "mpc_discretize_batch_ugrid", "mpc_discretize_batch_ugrid_host",
                  "mpc_ctx_create", "mpc_ctx_destroy", "mpc_discretize_batch_host", "mpc_propagate_batch_host",
@@ -212,6 +221,7 @@ EXPORTED_SYMBOLS = [
     "mpc_discretize_batch_units", "mpc_discretize_batch_units_host", "mpc_propagate_batch_rk45_units",
     "mpc_propagate_batch_rk45_units_host", "mpc_constraint_terms_units", "mpc_constraint_terms_units_host",
     "mpc_discretize_batch_ragged_gather", "mpc_fp64_peak_probe", "mpc_set_tuning", "mpc_set_gather_tuning",
+    "mpc_propagate_batch_rk45_atmo", "mpc_propagate_batch_rk45_atmo_host",
 ]
 
 

@@ -94,11 +94,15 @@ class DiscretizedBatch:
         raise_on_status(self.status)
 
 
-def raise_on_status(status):
+def raise_on_status(status, atmosphere=None):
     st = np.asarray(status)
     if st.size and st.max() != 0:
         idx = np.argwhere(st != 0)[0]
         code = int(st[tuple(idx)])
+        if code == _lib.ST_ATMO:
+            rng = "" if atmosphere is None else f" [{atmosphere.h_min:.6g}, {atmosphere.h_max:.6g}] m"
+            raise ValueError(f"satellite {int(idx[0])}: the altitude left the range of the fitted atmosphere{rng}; "
+                             "the density is not extrapolated")
         if code == _lib.ST_MASS:
             # same exception type / text as simulator.py:135-136
             raise Exception(f"ERROR: INVALID SATELLITE MASS: non-positive mass at unit {tuple(int(i) for i in idx)}")
@@ -225,6 +229,28 @@ def _rk4_units(const, n, n_sub):
                          "propagator has no per-satellite form")
 
 
+def _atmosphere(atmosphere, include_drag, n_sub):
+    """the mpc_atmosphere of an Atmosphere (None: the constant density), after the checks that raise before any device
+    work: the model is the density of the drag, flown by the reference integrator"""
+    if atmosphere is None:
+        return None
+    from .atmosphere import Atmosphere
+    if not isinstance(atmosphere, Atmosphere):
+        raise ValueError(f"atmosphere must be an Atmosphere (fit_atmosphere), got {type(atmosphere).__name__}")
+    if not include_drag:
+        raise ValueError("an atmosphere is the density of the drag: it needs include_drag=True")
+    if n_sub not in (None, 0):
+        raise ValueError("an atmosphere needs the reference integrator (n_sub=None); the fixed-step RK4 propagator "
+                         "flies the constant density only")
+    return atmosphere.struct()
+
+
+def _no_atmosphere(atmosphere, what):
+    if atmosphere is not None:
+        raise ValueError(f"{what} flies the constant density only: propagate with propagate_batch[_device]"
+                         "(atmosphere=...) instead")
+
+
 def _ctrl_struct(spec, n_sats, table_addr=None, end_tau_addr=None):
     c = _lib.MpcController()
     c.kind = spec.kind
@@ -263,7 +289,7 @@ def default_n_sub(T, max_step=0.001):
 
 
 def propagate_batch(y0, tf, controller, const, include_drag=True, include_J2=True, T=100, n_sub=None,
-                    want_u=True, device=0, check=True, y_out=None, u_out=None, rk45=None, n_steps=None):
+                    want_u=True, device=0, check=True, y_out=None, u_out=None, rk45=None, n_steps=None, atmosphere=None):
     """Propagate N satellites over tau in [0,1] and sample at linspace(0,1,T) (host arrays).
 
     y0 [N,7] normalized states; returns (y [N,7,T], u [N,3,T] or None, t [T], status [N]).
@@ -281,12 +307,17 @@ def propagate_batch(y0, tf, controller, const, include_drag=True, include_J2=Tru
 
     const: one Constants bag, or a sequence of N (satellite s integrated in the units of its own scale, one launch; N bags
     that agree bit for bit take the single-constant launch).  Per-satellite constants need the reference integrator.
+
+    atmosphere: an Atmosphere (fit_atmosphere) -- the drag's density rho(h) at every stage instead of the constant of
+    Simulator.get_atmo_density, satellite s at the altitude |r| r0 - R_EARTH of its own scale.  Needs include_drag and
+    the reference integrator (ValueError otherwise); a satellite that leaves the fitted range raises ValueError.
     """
     y0 = _f64(y0)
     if y0.ndim != 2 or y0.shape[1] != 7:
         raise ValueError(f"y0 must be [N,7], got {y0.shape}")
     N = y0.shape[0]
     _rk4_units(const, N, n_sub)
+    atmo = _atmosphere(atmosphere, include_drag, n_sub)
     ctx = _ctx(device)
     spec = spec_from(controller)
     T_sat = tab_len = None
@@ -322,7 +353,12 @@ def propagate_batch(y0, tf, controller, const, include_drag=True, include_J2=Tru
         if n_steps is not None and (n_steps.shape != (N,) or n_steps.dtype != np.int32):
             raise ValueError("n_steps must be int32 [N]")
         with _lock(device):
-            if psc is not None:
+            if atmo is not None:
+                _lib.check(_lib.lib().mpc_propagate_batch_rk45_atmo_host(
+                    ctx, _lib.addr(y0), _lib.addr(tfv), ctypes.byref(p), psc, ctypes.byref(c), N, T, _lib.addr(T_sat),
+                    _lib.addr(tab_len), float(o.get("rtol", 1e-3)), float(o.get("atol", 1e-6)), float(o.get("max_step", 1e-3)),
+                    _lib.addr(y), _lib.addr(uo), _lib.addr(status), _lib.addr(n_steps), ctypes.byref(atmo)))
+            elif psc is not None:
                 _lib.check(_lib.lib().mpc_propagate_batch_rk45_units_host(
                     ctx, _lib.addr(y0), _lib.addr(tfv), ctypes.byref(p), psc, ctypes.byref(c), N, T, _lib.addr(T_sat),
                     _lib.addr(tab_len), float(o.get("rtol", 1e-3)), float(o.get("atol", 1e-6)), float(o.get("max_step", 1e-3)),
@@ -344,18 +380,20 @@ def propagate_batch(y0, tf, controller, const, include_drag=True, include_J2=Tru
                                                            ctypes.byref(c), N, T, int(n_sub), _lib.addr(y),
                                                            _lib.addr(uo), _lib.addr(status)))
     if check:
-        raise_on_status(status)
+        raise_on_status(status, atmosphere)
     return y, uo, t, status
 
 
 def propagate_discretize(y0, tf, controller, const, T, prop_drag=False, prop_J2=False, disc_J2=False,
                          n_sub_prop=None, n_sub_disc=100, out=None, y_out=None, u_out=None, device=0, check=True,
-                         status=None, layout="satmajor"):
+                         status=None, layout="satmajor", atmosphere=None):
     """One SCP linearization pass on the device: propagate -> extract_uk -> discretize, the reference
     trajectory staying in HBM between the kernels (control.py:180-188 pattern).  K = T.
     layout="kmajor": the matrices come back in the k-major layout (DiscretizedBatch views hide it) through the streamed
     pass -- windows along k gated on the propagation's progress, every window read back while the next one runs.
-    Returns (DiscretizedBatch, y [N,7,T], u [N,3,T])."""
+    Returns (DiscretizedBatch, y [N,7,T], u [N,3,T]).  An atmosphere raises ValueError: the fused pass flies the constant
+    density only."""
+    _no_atmosphere(atmosphere, "propagate_discretize")
     ctx = _ctx(device)
     y0 = _f64(y0)
     N = y0.shape[0]
@@ -464,13 +502,15 @@ def discretize_batch_device(x, u, tf, const, include_J2=False, n_sub=100, out=No
 
 
 def propagate_batch_device(y0, tf, controller, const, include_drag=True, include_J2=True, T=100, n_sub=None,
-                           y=None, u_out=None, status=None, T_max=None):
+                           y=None, u_out=None, status=None, T_max=None, atmosphere=None):
     """Device form of propagate_batch: y0 [N,7], tf [N] float64 CUDA tensors -> y [N,7,T], u [N,3,T], status [N].
     T = int array [N] (host): satellite s sampled at linspace(0, 1, T_s) into the first T_s columns of y / u [.,.,Tmax]
     (the padding columns are not written), the reference integrator only, as propagate_batch; so is a sequence law
     with per-satellite table lengths (ControllerSpec.table_len).  T_max: the column stride of y / u of such a batch
     (default max T_s; a fixed capacity keeps the layout of a buffer whose counts change from call to call).
-    const: one Constants bag or a sequence of N, as in propagate_batch."""
+    const: one Constants bag or a sequence of N, as in propagate_batch; atmosphere as in propagate_batch (the status
+    words report a satellite that left the fitted range as ST_ATMO; raise_on_status(status, atmosphere) raises for it)."""
+    atmo = _atmosphere(atmosphere, include_drag, n_sub)
     torch = _torch()
     N = y0.shape[0]
     _rk4_units(const, N, n_sub)
@@ -506,7 +546,18 @@ def propagate_batch_device(y0, tf, controller, const, include_drag=True, include
     psc, const = _units_of(const, N)
     p = _lib.make_params(const, include_J2, include_drag)
     stream = torch.cuda.current_stream(y0.device).cuda_stream
-    if psc is not None:
+    if atmo is not None:
+        cnt_dev = torch.as_tensor(T_sat).to(y0.device) if T_sat is not None else None
+        len_dev = torch.as_tensor(tab_len).to(y0.device) if tab_len is not None else None
+        scratch = torch.empty(N * _lib.SAT_SCRATCH_DOUBLES, dtype=torch.float64, device=y0.device) if psc is not None else None
+        _lib.check(_lib.lib().mpc_propagate_batch_rk45_atmo(
+            y0.data_ptr(), tf.data_ptr(), ctypes.byref(p), psc, ctypes.byref(c), N, T,
+            cnt_dev.data_ptr() if cnt_dev is not None else None, len_dev.data_ptr() if len_dev is not None else None,
+            scratch.data_ptr() if scratch is not None else None, 1e-3, 1e-6, 1e-3, y.data_ptr(), u_out.data_ptr(),
+            status.data_ptr(), None, ctypes.byref(atmo), stream))
+        if scratch is not None:
+            scratch.record_stream(torch.cuda.current_stream(y0.device))
+    elif psc is not None:
         cnt_dev = torch.as_tensor(T_sat).to(y0.device) if T_sat is not None else None
         len_dev = torch.as_tensor(tab_len).to(y0.device) if tab_len is not None else None
         scratch = torch.empty(N * _lib.SAT_SCRATCH_DOUBLES, dtype=torch.float64, device=y0.device)
@@ -536,7 +587,7 @@ def propagate_batch_device(y0, tf, controller, const, include_drag=True, include
 def propagate_discretize_device(y0, tf, controller, const, T, prop_drag=False, prop_J2=False, disc_J2=False,
                                 n_sub_prop=None, n_sub_disc=100, y=None, u_out=None, out=None, out_pitch=None,
                                 out_offset=0, status_prop=None, status_disc=None, n_windows=0, extra_dst=None,
-                                out_ptr=None, gather=None):
+                                out_ptr=None, gather=None, atmosphere=None):
     """Device form of propagate_discretize: one SCP linearization pass (control.py:180-188) on CUDA tensors, enqueued on
     torch's current stream, with the propagation overlapped with the discretization (mpc_propagate_discretize: the
     intervals are discretized window by window along k as the propagation publishes its progress).  Bit-identical to
@@ -545,7 +596,9 @@ def propagate_discretize_device(y0, tf, controller, const, T, prop_drag=False, p
     (total 1, 2, 4 or 8: the fused all-gather); `out_ptr`: raw address used instead of out.data_ptr() (a multicast
     mapping of `out`); `gather`: an _lib.MpcGatherOpts -- layout (satellite- or k-major), n_sats_total, sat_offset and the
     gather options for this call (then out_pitch / out_offset are implied).
-    Returns (out [105, pitch], y [N,7,T], u [N,3,T], status_prop [N], status_disc [N*(T-1)])."""
+    Returns (out [105, pitch], y [N,7,T], u [N,3,T], status_prop [N], status_disc [N*(T-1)]).  An atmosphere raises
+    ValueError: the overlapped, streamed and gathered passes fly the constant density only."""
+    _no_atmosphere(atmosphere, "propagate_discretize_device")
     torch = _torch()
     N = y0.shape[0]
     T = int(T)

@@ -24,6 +24,7 @@
 #include "mpc_b200_drag.h"
 #include "mpc_b200_units.h"
 #include "mpc_b200_shard.h"
+#include "mpc_b200_atmo.h"
 #include "constraint_terms_kernel.cuh"
 #include "discretize_drag_kernel.cuh"
 #include "discretize_pair_kernel.cuh"
@@ -75,7 +76,66 @@ mpc::PropParams prop_params(const mpc_params *p)
     return d;
 }
 
+// ---- altitude-dependent atmosphere (mpc_propagate_batch_rk45_atmo) ----------------------------------------------------
+// The kernel constants of a satellite under the atmosphere: drag_k without the density (rho(h) multiplies it in the
+// kernel) and the metres per unit length of its constants, r_earth / r_e
+mpc::PropParams atmo_prop_params(const mpc_params *p)
+{
+    mpc::PropParams d = prop_params(p);
+    d.drag_k = 0.5 * p->c_d * p->s_area / p->rho;
+    return d;
+}
+
+mpc::AtmoSat atmo_sat(const mpc_params *q, double r_earth)
+{
+    mpc::AtmoSat a;
+    a.P = atmo_prop_params(q);
+    a.len = r_earth / q->r_e;
+    return a;
+}
+
+mpc::AtmoParams atmo_params(const mpc_atmosphere *a, double len)
+{
+    mpc::AtmoParams A{};
+    for (int k = 0; k < a->n; ++k) A.coef[k] = a->coef[k];
+    A.n = a->n;
+    const double lo = std::log(a->h_min), hi = std::log(a->h_max);
+    A.s_mid = 0.5 * (lo + hi);
+    A.s_ihalf = 2.0 / (hi - lo);
+    A.h_min = a->h_min;
+    A.h_max = a->h_max;
+    A.r_earth = a->r_earth;
+    A.len = len;
+    return A;
+}
+
+bool positive(double x) { return std::isfinite(x) && x > 0.0; }
+
+// the model, and what the drag under it divides by (r_e for the length unit, rho), of p or of every consts[s]
+int check_atmo(const mpc_atmosphere *a, const mpc_params *p, const mpc_sat_consts *c, int n)
+{
+    if (!a || !p) return fail(MPC_E_INVALID, "null atmosphere / params");
+    if (!p->include_drag) return fail(MPC_E_INVALID, "an atmosphere is the density of the drag: it needs include_drag");
+    if (a->n < 1 || a->n > MPC_RHO_CHEB) return fail(MPC_E_INVALID, "atmosphere: need 1 <= n <= %d (got %d)", MPC_RHO_CHEB, a->n);
+    if (!positive(a->h_min) || !(std::isfinite(a->h_max) && a->h_max > a->h_min))
+        return fail(MPC_E_INVALID, "atmosphere: need 0 < h_min < h_max (got %g, %g)", a->h_min, a->h_max);
+    if (!positive(a->r_earth)) return fail(MPC_E_INVALID, "atmosphere: need r_earth > 0 (got %g)", a->r_earth);
+    for (int k = 0; k < a->n; ++k)
+        if (!std::isfinite(a->coef[k])) return fail(MPC_E_INVALID, "atmosphere: coef[%d] is not finite", k);
+    if (!std::isfinite(p->c_d) || !std::isfinite(p->s_area)) return fail(MPC_E_INVALID, "need finite c_d and s_area");
+    if (!c) {
+        if (!positive(p->r_e) || !positive(p->rho))
+            return fail(MPC_E_INVALID, "an atmosphere needs r_e > 0 and rho > 0 (got %g, %g)", p->r_e, p->rho);
+        return MPC_SUCCESS;
+    }
+    for (int s = 0; s < n; ++s)
+        if (!positive(c[s].r_e) || !positive(c[s].rho))
+            return fail(MPC_E_INVALID, "consts[%d]: an atmosphere needs r_e > 0 and rho > 0 (got %g, %g)", s, c[s].r_e, c[s].rho);
+    return MPC_SUCCESS;
+}
+
 // ---- per-satellite designer units (the *_units entry points) ---------------------------------------------------------
+static_assert(sizeof(mpc::AtmoSat) <= MPC_SAT_SCRATCH_DOUBLES * sizeof(double), "per-satellite scratch too small");
 static_assert(sizeof(mpc::PropParams) <= MPC_SAT_SCRATCH_DOUBLES * sizeof(double) &&
               sizeof(mpc::DiscParams) <= MPC_SAT_SCRATCH_DOUBLES * sizeof(double), "per-satellite scratch too small");
 
@@ -115,6 +175,10 @@ int upload_sat_table(const mpc_params *p, const mpc_sat_consts *c, int n, void *
         mpc_units_sizeof(2) != sizeof(mpc::PropParams) || mpc_units_sizeof(3) != sizeof(mpc::CtrlParams) ||
         mpc_units_sizeof(4) != sizeof(mpc::Rk45Opts))
         return fail(MPC_E_CUDA, "mpc_b200_units.cu was built against different parameter structs");
+    if (mpc_atmo_sizeof(0) != sizeof(mpc::PropParams) || mpc_atmo_sizeof(1) != sizeof(mpc::CtrlParams) ||
+        mpc_atmo_sizeof(2) != sizeof(mpc::Rk45Opts) || mpc_atmo_sizeof(3) != sizeof(mpc::AtmoParams) ||
+        mpc_atmo_sizeof(4) != sizeof(mpc::AtmoSat))
+        return fail(MPC_E_CUDA, "mpc_b200_atmo.cu was built against different parameter structs");
     std::vector<T> v((size_t)n);
     mpc_params q = *p;
     for (int s = 0; s < n; ++s) {
@@ -776,11 +840,15 @@ void launch_rk45_ragged(bool spec, unsigned n_warps, cudaStream_t st, const doub
 int prop_device(const double *y0, const double *tf, const mpc_params *p, const mpc_controller *c,
                 const double *table_dev, const double *end_tau_dev, int n_sats, int T, const PropMode &mode, double *y, double *u_out, int32_t *status,
                 cudaStream_t st, unsigned int *progress = nullptr, int seg_len = 0, unsigned int *progress_target = nullptr,
-                const int32_t *T_sat_dev = nullptr, const int32_t *ku_dev = nullptr, const mpc::PropParams *psc_dev = nullptr)
+                const int32_t *T_sat_dev = nullptr, const int32_t *ku_dev = nullptr, const void *psc_dev = nullptr,
+                const mpc::AtmoParams *atmo = nullptr)
 {
+    // psc_dev: device mpc::PropParams [n_sats] (mpc::AtmoSat [n_sats] with an atmosphere) or NULL
     if (!y0 || !tf || !p || !y) return fail(MPC_E_INVALID, "null pointer argument");
     if (psc_dev && (!mode.rk45() || progress))
         return fail(MPC_E_UNSUPPORTED, "per-satellite constants need the RK45 propagator (n_sub = 0) outside the fused pass");
+    if (atmo && (!mode.rk45() || progress))
+        return fail(MPC_E_UNSUPPORTED, "an atmosphere needs the RK45 propagator (n_sub = 0) outside the fused pass");
     // per-satellite counts (device arrays here): the RK45 propagator on its own only
     const bool ragged = T_sat_dev || ku_dev;
     if (ragged && (!mode.rk45() || progress))
@@ -806,7 +874,7 @@ int prop_device(const double *y0, const double *tf, const mpc_params *p, const m
     if (c->kind != MPC_CTRL_SEQUENCE) ku_dev = nullptr;
     const unsigned grid = (unsigned)((n_sats + kPropBlock - 1) / kPropBlock);
     const unsigned grid_ov = (unsigned)((n_sats + kPropBlockOverlap - 1) / kPropBlockOverlap);
-    const mpc::PropParams PP = prop_params(p);
+    const mpc::PropParams PP = atmo ? atmo_prop_params(p) : prop_params(p);
     int dev = 0, sms = 148;
     CUDA_TRY(cudaGetDevice(&dev));
     CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
@@ -815,7 +883,7 @@ int prop_device(const double *y0, const double *tf, const mpc_params *p, const m
     const unsigned n_warps = (unsigned)((n_sats + lpw - 1) / lpw);
     const bool spec = g_rk45_spec.load(std::memory_order_relaxed) != 0;
     if (progress_target) *progress_target = mode.rk45() ? (unsigned)n_sats : (unsigned)((n_sats + 31) / 32);
-    if (psc_dev) {   // per-satellite constants: one-warp CTAs, mpc_b200_units.cu
+    if (psc_dev || atmo) {   // per-satellite constants / the atmosphere: one-warp CTAs, mpc_b200_units.cu / mpc_b200_atmo.cu
         MpcUnitsProp a{};
         a.y0 = y0;
         a.tf = tf;
@@ -836,7 +904,9 @@ int prop_device(const double *y0, const double *tf, const mpc_params *p, const m
         a.T_sat = T_sat_dev;
         a.ku = ku_dev;
         a.stream = st;
-        CUDA_TRY(mpc_units_launch_rk45(&a));
+        a.prop = &PP;
+        if (atmo) CUDA_TRY(mpc_atmo_launch_rk45(&a, atmo));
+        else CUDA_TRY(mpc_units_launch_rk45(&a));
         g_launches.fetch_add(1, std::memory_order_relaxed);
         return MPC_SUCCESS;
     }
@@ -1436,7 +1506,7 @@ static int upload_table(mpc_ctx *ctx, const mpc_controller *ctrl, int n_sats, cu
 static int prop_host(mpc_ctx *ctx, const double *y0, const double *tf, const mpc_params *p, const mpc_controller *ctrl,
                      int n_sats, int T, PropMode mode, double *y_host, double *u_host, int32_t *status_host,
                      int32_t *n_steps_host, const int32_t *T_sat = nullptr, const int32_t *ku_in = nullptr,
-                     const mpc_sat_consts *consts = nullptr)
+                     const mpc_sat_consts *consts = nullptr, const mpc_atmosphere *atmo = nullptr)
 {
     if (!ctx || !y0 || !tf || !p || !y_host) return fail(MPC_E_INVALID, "null pointer argument");
     if (n_sats < 0 || T < 0 || mode.n_sub < 0) return fail(MPC_E_INVALID, "need n_sats >= 0, T >= 0, n_sub >= 0");
@@ -1446,6 +1516,7 @@ static int prop_host(mpc_ctx *ctx, const double *y0, const double *tf, const mpc
     if (T_sat && (rc = check_counts(T_sat, n_sats, T, "T_sat"))) return rc;
     if (ku && (rc = check_counts(ku, n_sats, ctrl->table_len, "table_len_sat"))) return rc;
     if (consts && (rc = check_sat_consts(consts, n_sats))) return rc;
+    if (atmo && (rc = check_atmo(atmo, p, consts, n_sats))) return rc;
     if (n_sats == 0 || T == 0) return MPC_SUCCESS;
     CUDA_TRY(cudaSetDevice(ctx->device));
     if ((rc = ensure(ctx->d_y0, ctx->cap_y0, (size_t)n_sats * 7))) return rc;
@@ -1472,11 +1543,19 @@ static int prop_host(mpc_ctx *ctx, const double *y0, const double *tf, const mpc
     }
     if (consts) {
         if ((rc = ensure(ctx->d_psc, ctx->cap_psc, (size_t)n_sats * MPC_SAT_SCRATCH_DOUBLES))) return rc;
-        if ((rc = upload_sat_table<mpc::PropParams>(p, consts, n_sats, ctx->d_psc, st, prop_params))) return rc;
+        if (atmo) {
+            const double r_earth = atmo->r_earth;
+            rc = upload_sat_table<mpc::AtmoSat>(p, consts, n_sats, ctx->d_psc, st,
+                                                [r_earth](const mpc_params *q) { return atmo_sat(q, r_earth); });
+        } else {
+            rc = upload_sat_table<mpc::PropParams>(p, consts, n_sats, ctx->d_psc, st, prop_params);
+        }
+        if (rc) return rc;
     }
+    const mpc::AtmoParams A = atmo ? atmo_params(atmo, atmo->r_earth / p->r_e) : mpc::AtmoParams{};
     if ((rc = prop_device(ctx->d_y0, ctx->d_tf, p, ctrl, ctx->d_tab, ctrl->end_tau_per_sat ? ctx->d_endtau : nullptr, n_sats, T, mode,
                           ctx->d_x, ctx->d_u, ctx->d_status2, st, nullptr, 0, nullptr, T_sat ? ctx->d_cnt : nullptr,
-                          ku ? ctx->d_cnt + n_sats : nullptr, consts ? (const mpc::PropParams *)ctx->d_psc : nullptr)))
+                          ku ? ctx->d_cnt + n_sats : nullptr, consts ? ctx->d_psc : nullptr, atmo ? &A : nullptr)))
         return rc;
     CUDA_TRY(cudaMemcpyAsync(y_host, ctx->d_x, (size_t)n_sats * 7 * T * sizeof(double), cudaMemcpyDeviceToHost, st));
     if (u_host) CUDA_TRY(cudaMemcpyAsync(u_host, ctx->d_u, (size_t)n_sats * 3 * T * sizeof(double), cudaMemcpyDeviceToHost, st));
@@ -1655,6 +1734,44 @@ int mpc_propagate_batch_rk45_units_host(mpc_ctx *ctx, const double *y0, const do
     m.rk = mpc::Rk45Opts{rtol, atol, max_step};
     return prop_host(ctx, y0, tf, p, ctrl, n_sats, T_max, m, y_host, u_host, status_host, n_steps_host, T_sat, table_len_sat,
                      consts);
+}
+
+int mpc_propagate_batch_rk45_atmo(const double *y0, const double *tf, const mpc_params *p, const mpc_sat_consts *consts,
+                                  const mpc_controller *ctrl, int n_sats, int T_max, const int32_t *T_sat,
+                                  const int32_t *table_len_sat, double *consts_scratch, double rtol, double atol,
+                                  double max_step, double *y, double *u_out, int32_t *status, int32_t *n_steps,
+                                  const mpc_atmosphere *atmo, void *stream)
+{
+    if (!p) return fail(MPC_E_INVALID, "null pointer argument");
+    if (T_sat && T_max < 2) return fail(MPC_E_INVALID, "need T_max >= 2 (got %d)", T_max);
+    int rc = consts ? check_sat_consts(consts, n_sats) : MPC_SUCCESS;
+    if (rc || (rc = check_atmo(atmo, p, consts, n_sats))) return rc;
+    if (consts && n_sats > 0 && T_max > 0) {
+        const double r_earth = atmo->r_earth;
+        if ((rc = upload_sat_table<mpc::AtmoSat>(p, consts, n_sats, consts_scratch, (cudaStream_t)stream,
+                                                 [r_earth](const mpc_params *q) { return atmo_sat(q, r_earth); })))
+            return rc;
+    }
+    const mpc::AtmoParams A = atmo_params(atmo, atmo->r_earth / p->r_e);
+    PropMode m;
+    m.rk = mpc::Rk45Opts{rtol, atol, max_step};
+    m.n_steps = n_steps;
+    return prop_device(y0, tf, p, ctrl, ctrl ? ctrl->table : nullptr, ctrl ? ctrl->end_tau_per_sat : nullptr, n_sats, T_max, m,
+                       y, u_out, status, (cudaStream_t)stream, nullptr, 0, nullptr, T_sat, table_len_sat,
+                       consts ? consts_scratch : nullptr, &A);
+}
+
+int mpc_propagate_batch_rk45_atmo_host(mpc_ctx *ctx, const double *y0, const double *tf, const mpc_params *p,
+                                       const mpc_sat_consts *consts, const mpc_controller *ctrl, int n_sats, int T_max,
+                                       const int32_t *T_sat, const int32_t *table_len_sat, double rtol, double atol,
+                                       double max_step, double *y_host, double *u_host, int32_t *status_host,
+                                       int32_t *n_steps_host, const mpc_atmosphere *atmo)
+{
+    if (!atmo) return fail(MPC_E_INVALID, "null atmosphere");
+    PropMode m;
+    m.rk = mpc::Rk45Opts{rtol, atol, max_step};
+    return prop_host(ctx, y0, tf, p, ctrl, n_sats, T_max, m, y_host, u_host, status_host, n_steps_host, T_sat, table_len_sat,
+                     consts, atmo);
 }
 
 int mpc_propagate_batch_host(mpc_ctx *ctx, const double *y0, const double *tf, const mpc_params *p,

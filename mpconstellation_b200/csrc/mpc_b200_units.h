@@ -31,6 +31,7 @@ struct MpcUnitsProp {
     int32_t *status, *n_steps;
     const int32_t *T_sat, *ku;  // device, may be NULL (all T / all table_len)
     cudaStream_t stream;
+    const void *prop;          // mpc::PropParams of a launch without per-satellite constants (mpc_b200_atmo.cu only)
 };
 
 size_t mpc_units_sizeof(int which);   // 0 DiscParams, 1 DstTab, 2 PropParams, 3 CtrlParams, 4 Rk45Opts

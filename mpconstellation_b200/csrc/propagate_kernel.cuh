@@ -131,13 +131,46 @@ __device__ __forceinline__ void ctrl_eval_foh_cached(const CtrlParams &C, const 
     uz = on ? vz : 0.0;
 }
 
-// f(y,u) without the tf factor (simulator.py:130-160); returns nonzero on non-positive mass.  fc: the knot-interval cache
-// of the table law (KIND 3 only; nullptr = evaluate the law from scratch); ku: see ctrl_eval
-template <int KIND, bool DRAG, bool J2>
+// An altitude-dependent atmosphere (mpc_atmosphere, fitted and checked on the host: atmosphere.fit_atmosphere): log rho
+// as a Chebyshev series in t = (log h - s_mid) s_ihalf, h = |r| len - r_earth the altitude in metres, valid on
+// [h_min, h_max].  With it the drag coefficient drag_k of PropParams is 0.5 C_D S / RHO and the density rho(h) multiplies
+// it at every stage evaluation.
+constexpr int kAtmoCheb = 32;
+struct AtmoParams {
+    double coef[kAtmoCheb];
+    double s_mid, s_ihalf, h_min, h_max, r_earth;
+    double len;                 // metres per unit length of the launch-wide constants (per-satellite: AtmoSat::len)
+    int n, pad;
+};
+// one satellite's entry of the per-satellite constants table of the atmosphere kernels
+struct AtmoSat {
+    PropParams P;
+    double len;
+};
+
+__device__ __forceinline__ double atmo_density(const AtmoParams &A, double h)
+{
+    const double t = (log(h) - A.s_mid) * A.s_ihalf;
+    // Clenshaw: sum_k c_k T_k(t)
+    double b1 = 0.0, b2 = 0.0;
+    const double t2 = 2.0 * t;
+    for (int k = A.n - 1; k >= 1; --k) {
+        const double b = fma(t2, b1, A.coef[k]) - b2;
+        b2 = b1;
+        b1 = b;
+    }
+    return exp(fma(t, b1, A.coef[0]) - b2);
+}
+
+// f(y,u) without the tf factor (simulator.py:130-160); returns nonzero on non-positive mass (1) and, with ATMO, an
+// altitude outside the fitted atmosphere (4, MPC_ST_ATMO).  fc: the knot-interval cache of the table law (KIND 3 only;
+// nullptr = evaluate the law from scratch); ku: see ctrl_eval; A / len: the atmosphere and the satellite's length unit
+template <int KIND, bool DRAG, bool J2, bool ATMO = false>
 __device__ __forceinline__ int prop_rhs(const PropParams &P, const CtrlParams &C, const double *__restrict__ tab,
                                         double end_tau, const double (&y)[7], double tau, double (&dy)[7],
-                                        FohCache *fc = nullptr, int ku = 0)
+                                        FohCache *fc = nullptr, int ku = 0, const AtmoParams *A = nullptr, double len = 0.0)
 {
+    int out = 0;
     const double m = y[6];
     const double r2 = fma(y[0], y[0], fma(y[1], y[1], y[2] * y[2]));
     const double ir = fast_rsqrt(r2);
@@ -165,7 +198,13 @@ __device__ __forceinline__ int prop_rhs(const PropParams &P, const CtrlParams &C
     if (DRAG) {
         const double v2 = fma(y[3], y[3], fma(y[4], y[4], y[5] * y[5]));
         const double vn = (v2 > 0.0) ? v2 * fast_rsqrt(v2) : 0.0;
-        const double c = -P.drag_k * im * vn;
+        double kd = P.drag_k;
+        if constexpr (ATMO) {
+            const double h = fma(r2 * ir, len, -A->r_earth);
+            if (h < A->h_min || h > A->h_max) out = 4;
+            kd *= atmo_density(*A, h);
+        }
+        const double c = -kd * im * vn;
         ax = fma(c, y[3], ax);
         ay = fma(c, y[4], ay);
         az = fma(c, y[5], az);
@@ -193,7 +232,8 @@ __device__ __forceinline__ int prop_rhs(const PropParams &P, const CtrlParams &C
     dy[4] = ay;
     dy[5] = az;
     dy[6] = -un * P.inv_ve;
-    return !(m > 0.0);
+    if constexpr (ATMO) return (int)!(m > 0.0) | out;
+    else return !(m > 0.0);
 }
 
 template <int BLOCK, int KIND, bool DRAG, bool J2>

@@ -23,7 +23,9 @@
 // step size (the controller almost always returns max_step again) while the error norm of the current one is still
 // being formed; a wrong prediction just recomputes that stage.  `lpw` lanes of every warp carry satellites (the rest
 // exit at once): fewer satellites per warp spread a small batch over more SM sub-partitions.
-#pragma once
+#ifndef MPC_RK45_BODY
+#ifndef MPC_PROPAGATE_RK45_KERNEL_CUH
+#define MPC_PROPAGATE_RK45_KERNEL_CUH
 #include "propagate_kernel.cuh"
 
 namespace mpc {
@@ -50,6 +52,8 @@ __device__ __forceinline__ double rk45_factor(double err2) { return 0.9 * pow(er
 // device table [n_sats] passed in place of the progress words (such a launch has none).  The table travels in an
 // existing parameter because ptxas's register allocation of these ~250-register kernels follows the entry's parameter
 // list: one more parameter changed the SASS of every single-constant instantiation.
+// ATMO (propagate_rk45_atmo_kernel): drag under the altitude-dependent atmosphere A, in a kernel of its own for that
+// reason; with PSC its per-satellite table is `asat` (AtmoSat: the constants and the satellite's length unit).
 template <int BLOCK, int KIND, bool DRAG, bool J2, bool SPEC, bool RAG = false, bool PSC = false>
 __global__ void __launch_bounds__(BLOCK)
 propagate_rk45_kernel(const double *__restrict__ y0, const double *__restrict__ tf_arr, PropParams P, CtrlParams C,
@@ -57,6 +61,55 @@ propagate_rk45_kernel(const double *__restrict__ y0, const double *__restrict__ 
                       int32_t *__restrict__ status, int32_t *__restrict__ n_steps, unsigned int *progress, int seg_len,
                       const int32_t *__restrict__ T_sat = nullptr, const int32_t *__restrict__ Ku_sat = nullptr)
 {
+#define MPC_RK45_ATMO 0
+#define MPC_RK45_BODY
+#include "propagate_rk45_kernel.cuh"
+#undef MPC_RK45_BODY
+#undef MPC_RK45_ATMO
+}
+
+// The RK45 replay with drag under the altitude-dependent atmosphere A (mpc_propagate_batch_rk45_atmo): always the ragged
+// form (T_sat / Ku_sat == nullptr: the rectangular run), one-warp CTAs.  PSC: satellite s takes its constants and its
+// length unit from asat[s] (P is then not read).  No progress words: never beside the discretization.  The speculative
+// first stage (which changes the schedule, not the result) is on except for the table law: its knot-interval cache
+// already holds that kernel at 254-255 registers, and log, exp and the series on top of the speculative stage's state
+// spilled.
+template <int KIND, bool J2, bool PSC>
+__global__ void __launch_bounds__(32)
+propagate_rk45_atmo_kernel(const double *__restrict__ y0, const double *__restrict__ tf_arr, PropParams P, CtrlParams C,
+                           Rk45Opts O, int n_sats, int T, int lpw, double *__restrict__ y_out, double *__restrict__ u_out,
+                           int32_t *__restrict__ status, int32_t *__restrict__ n_steps, const int32_t *__restrict__ T_sat,
+                           const int32_t *__restrict__ Ku_sat, const __grid_constant__ AtmoParams Aparam,
+                           const AtmoSat *__restrict__ asat)
+{
+    constexpr int BLOCK = 32;
+    constexpr bool DRAG = true, SPEC = (KIND != 3), RAG = true;
+    const AtmoParams *const A = &Aparam;
+    unsigned int *progress = nullptr;
+    const int seg_len = 0;
+#define MPC_RK45_ATMO 1
+#define MPC_RK45_BODY
+#include "propagate_rk45_kernel.cuh"
+#undef MPC_RK45_BODY
+#undef MPC_RK45_ATMO
+}
+
+}  // namespace mpc
+
+#endif  // MPC_PROPAGATE_RK45_KERNEL_CUH
+#else   // MPC_RK45_BODY
+// The body of the RK45 replay, included by this file into its two kernels above (and nowhere else).  It is one body for
+// both; it is included rather than called because ptxas's code generation of these ~250-register kernels follows their
+// structure: the same body behind an inlined call changed the SASS of every existing instantiation, and so does any
+// difference in its text.  MPC_RK45_ATMO (0 / 1, set by the including kernel) switches the atmosphere's lines in by the
+// preprocessor, so that the other kernels compile the text they always had.  In scope: the template flags BLOCK, KIND,
+// DRAG, J2, SPEC, RAG, PSC, the kernel parameters and, with MPC_RK45_ATMO, A (the atmosphere) and asat (its
+// per-satellite table, PSC).
+#if MPC_RK45_ATMO
+#define MPC_RK45_ATMO_ARGS , A, alen
+#else
+#define MPC_RK45_ATMO_ARGS
+#endif
     // progress != nullptr (the overlapped pass, see propagate_kernel): window b of the discretization needs the samples
     // up to e_b = min((b+1) seg_len, T-1).  Lanes may take different numbers of steps here, so every LANE that has stored
     // sample e_b counts itself into progress[b] (fence first; lanes of a warp that arrive together are aggregated into
@@ -69,10 +122,20 @@ propagate_rk45_kernel(const double *__restrict__ y0, const double *__restrict__ 
     // of the progress words below sees none.  Nothing may read `progress` before this point.
     static_assert(alignof(PropParams) == alignof(double) && sizeof(PropParams) % alignof(double) == 0,
                   "the per-satellite table is an array of PropParams at a double-aligned address");
+#if MPC_RK45_ATMO
+    double alen;                  // metres per unit length of this satellite's constants
+    if constexpr (PSC) {
+        P = asat[s].P;
+        alen = asat[s].len;
+    } else {
+        alen = A->len;
+    }
+#else
     if constexpr (PSC) {
         P = reinterpret_cast<const PropParams *>(progress)[s];
         progress = nullptr;
     }
+#endif
     const double *tab = C.table ? C.table + (C.table_per_sat ? (long long)s * 3 * C.table_len : 0) : nullptr;
     // samples of this lane (T: the stride) and columns of its table (0: C.table_len), held inside the buffers
     const int Tn = (RAG && T_sat) ? min(max(T_sat[s], 0), T) : T;
@@ -103,7 +166,7 @@ propagate_rk45_kernel(const double *__restrict__ y0, const double *__restrict__ 
     FohCache foh;                 // KIND 3: knot interval of the table law shared by consecutive stage evaluations
     foh_cache_init(foh, RAG && ku > 0 ? ku : C.table_len, end_tau);
     FohCache *const fc = (KIND == 3) ? &foh : nullptr;
-    bad |= prop_rhs<KIND, DRAG, J2>(P, C, tab, end_tau, y, 0.0, K[0], nullptr, ku);
+    bad |= prop_rhs<KIND, DRAG, J2, MPC_RK45_ATMO>(P, C, tab, end_tau, y, 0.0, K[0], nullptr, ku MPC_RK45_ATMO_ARGS);
     // ---- select_initial_step (common.py), f = tf * k ------------------------------------------------------------
     double h_abs;
     {
@@ -119,7 +182,7 @@ propagate_rk45_kernel(const double *__restrict__ y0, const double *__restrict__ 
         h0 = fmin(h0, 1.0);
 #pragma unroll
         for (int i = 0; i < 7; ++i) y1[i] = fma(h0 * tf, K[0][i], y[i]);
-        bad |= prop_rhs<KIND, DRAG, J2>(P, C, tab, end_tau, y1, h0, k1, nullptr, ku);
+        bad |= prop_rhs<KIND, DRAG, J2, MPC_RK45_ATMO>(P, C, tab, end_tau, y1, h0, k1, nullptr, ku MPC_RK45_ATMO_ARGS);
 #pragma unroll
         for (int i = 0; i < 7; ++i) {
             const double q = tf * (k1[i] - K[0][i]) / (atol + fabs(y[i]) * rtol);
@@ -158,7 +221,7 @@ propagate_rk45_kernel(const double *__restrict__ y0, const double *__restrict__ 
 #pragma unroll
                 for (int i = 0; i < NC; ++i) ys[i] = fma(K[0][i], a10, y[i]);
                 if (CM) ys[6] = fma(K[0][6], hs * (1.0 / 5), y[6]);
-                bad |= prop_rhs<KIND, DRAG, J2>(P, C, tab, end_tau, ys, t + (1.0 / 5) * h, K[1], fc, ku);
+                bad |= prop_rhs<KIND, DRAG, J2, MPC_RK45_ATMO>(P, C, tab, end_tau, ys, t + (1.0 / 5) * h, K[1], fc, ku MPC_RK45_ATMO_ARGS);
             }
             have_k1 = false;
             {
@@ -167,7 +230,7 @@ propagate_rk45_kernel(const double *__restrict__ y0, const double *__restrict__ 
 #pragma unroll
                 for (int i = 0; i < NC; ++i) ys[i] = fma(K[1][i], a1, fma(K[0][i], a0, y[i]));
                 if (CM) ys[6] = fma(K[0][6], hs * (3.0 / 10), y[6]);
-                bad |= prop_rhs<KIND, DRAG, J2>(P, C, tab, end_tau, ys, t + (3.0 / 10) * h, K[2], fc, ku);
+                bad |= prop_rhs<KIND, DRAG, J2, MPC_RK45_ATMO>(P, C, tab, end_tau, ys, t + (3.0 / 10) * h, K[2], fc, ku MPC_RK45_ATMO_ARGS);
             }
             {
                 double ys[7];
@@ -175,7 +238,7 @@ propagate_rk45_kernel(const double *__restrict__ y0, const double *__restrict__ 
 #pragma unroll
                 for (int i = 0; i < NC; ++i) ys[i] = fma(K[2][i], a2, fma(K[1][i], a1, fma(K[0][i], a0, y[i])));
                 if (CM) ys[6] = fma(K[0][6], hs * (4.0 / 5), y[6]);
-                bad |= prop_rhs<KIND, DRAG, J2>(P, C, tab, end_tau, ys, t + (4.0 / 5) * h, K[3], fc, ku);
+                bad |= prop_rhs<KIND, DRAG, J2, MPC_RK45_ATMO>(P, C, tab, end_tau, ys, t + (4.0 / 5) * h, K[3], fc, ku MPC_RK45_ATMO_ARGS);
             }
             {
                 double ys[7];
@@ -185,7 +248,7 @@ propagate_rk45_kernel(const double *__restrict__ y0, const double *__restrict__ 
                 for (int i = 0; i < NC; ++i)
                     ys[i] = fma(K[3][i], a3, fma(K[2][i], a2, fma(K[1][i], a1, fma(K[0][i], a0, y[i]))));
                 if (CM) ys[6] = fma(K[0][6], hs * (8.0 / 9), y[6]);
-                bad |= prop_rhs<KIND, DRAG, J2>(P, C, tab, end_tau, ys, t + (8.0 / 9) * h, K[4], fc, ku);
+                bad |= prop_rhs<KIND, DRAG, J2, MPC_RK45_ATMO>(P, C, tab, end_tau, ys, t + (8.0 / 9) * h, K[4], fc, ku MPC_RK45_ATMO_ARGS);
             }
             {
                 double ys[7];
@@ -195,7 +258,7 @@ propagate_rk45_kernel(const double *__restrict__ y0, const double *__restrict__ 
                 for (int i = 0; i < NC; ++i)
                     ys[i] = fma(K[4][i], a4, fma(K[3][i], a3, fma(K[2][i], a2, fma(K[1][i], a1, fma(K[0][i], a0, y[i])))));
                 if (CM) ys[6] = fma(K[0][6], hs, y[6]);
-                bad |= prop_rhs<KIND, DRAG, J2>(P, C, tab, end_tau, ys, t + h, K[5], fc, ku);
+                bad |= prop_rhs<KIND, DRAG, J2, MPC_RK45_ATMO>(P, C, tab, end_tau, ys, t + h, K[5], fc, ku MPC_RK45_ATMO_ARGS);
             }
             {
                 const double b0 = hs * (35.0 / 384), b2 = hs * (500.0 / 1113), b3 = hs * (125.0 / 192),
@@ -204,7 +267,7 @@ propagate_rk45_kernel(const double *__restrict__ y0, const double *__restrict__ 
                 for (int i = 0; i < NC; ++i)
                     yn[i] = fma(K[5][i], b5, fma(K[4][i], b4, fma(K[3][i], b3, fma(K[2][i], b2, fma(K[0][i], b0, y[i])))));
                 if (CM) yn[6] = fma(K[0][6], hs, y[6]);
-                bad |= prop_rhs<KIND, DRAG, J2>(P, C, tab, end_tau, yn, t + h, K[6], fc, ku);
+                bad |= prop_rhs<KIND, DRAG, J2, MPC_RK45_ATMO>(P, C, tab, end_tau, yn, t + h, K[6], fc, ku MPC_RK45_ATMO_ARGS);
             }
             double k1n[7];
             int bad_n = 0;
@@ -219,7 +282,7 @@ propagate_rk45_kernel(const double *__restrict__ y0, const double *__restrict__ 
 #pragma unroll
                 for (int i = 0; i < NC; ++i) ys[i] = fma(K[6][i], a10, yn[i]);
                 if (CM) ys[6] = fma(K[0][6], a10, yn[6]);
-                bad_n = prop_rhs<KIND, DRAG, J2>(P, C, tab, end_tau, ys, t_new + (1.0 / 5) * h_pred, k1n, fc, ku);
+                bad_n = prop_rhs<KIND, DRAG, J2, MPC_RK45_ATMO>(P, C, tab, end_tau, ys, t_new + (1.0 / 5) * h_pred, k1n, fc, ku MPC_RK45_ATMO_ARGS);
             }
             // -- error norm (rk.py _estimate_error_norm) ---------------------------------------------------------------
             double eh[NC], esum0 = 0.0;
@@ -367,8 +430,12 @@ propagate_rk45_kernel(const double *__restrict__ y0, const double *__restrict__ 
             }
         }
     }
+#if MPC_RK45_ATMO
+    // prop_rhs reports the atmosphere's range as 4 (MPC_ST_ATMO); a non-positive mass takes precedence
+    if (status) status[s] = bad ? ((bad & 1) ? 1 : 4) : (fail ? 3 : 0);
+#else
     if (status) status[s] = bad ? 1 : (fail ? 3 : 0);
+#endif
     if (n_steps) n_steps[s] = steps;
-}
-
-}  // namespace mpc
+#undef MPC_RK45_ATMO_ARGS
+#endif  // MPC_RK45_BODY

@@ -157,12 +157,14 @@ class BatchedSCP:
         return tab, lens, tf_u, history
 
     def run_segments(self, y0, n_segments, solver=hold_reference_solver, include_drag=True, include_J2=True,
-                     sim_base_res=100):
+                     sim_base_res=100, atmosphere=None):
         """Simulator.run_segments with an OptimalController (test_simulator.py:79-95) for N satellites: before every
         segment the controller re-plans (plan), then the satellites fly `interval` with the planned inputs
-        (SequenceController(u, tf_u, tf_sim=interval), control.py:217) under the full dynamics."""
+        (SequenceController(u, tf_u, tf_sim=interval), control.py:217) under the full dynamics.  atmosphere: an
+        Atmosphere (fit_atmosphere), the density of the flight's drag; the plans stay drag-free (control.py:238-239)."""
         y = np.ascontiguousarray(y0, dtype=np.float64)
         N = y.shape[0]
+        batch._atmosphere(atmosphere, include_drag, None)     # (raises before any device work)
         if _lib.sat_consts(self.const, N)[0] is not None:
             raise NotImplementedError("run_segments with per-satellite constants: the flight runs in the Simulator's one "
                                       "scale, and carrying each controller's plan across that unit boundary is not "
@@ -175,7 +177,7 @@ class BatchedSCP:
             ctrl = ControllerSpec(_lib.CTRL_SEQUENCE, (0.0, 0.0, 0.0), u_tab, end_tau, lens)
             T = int(sim_base_res * self.interval)
             ys, _, _, _ = batch.propagate_batch(y, self.interval, ctrl, self.const, include_drag=include_drag,
-                                                include_J2=include_J2, T=T, device=self.device)
+                                                include_J2=include_J2, T=T, device=self.device, atmosphere=atmosphere)
             traj.append(np.array(ys))
             y = np.ascontiguousarray(ys[:, :, -1])
             if self.horizon - self.interval > 0.1:          # control.py:234-235

@@ -35,6 +35,9 @@ class Simulator:
         self.integrator = "rk45"
         self.last_n_steps = None
         self.device = 0
+        # an Atmosphere (fit_atmosphere): the density of the drag as a function of the altitude instead of the constant of
+        # get_atmo_density; used when include_drag is set (the reference integrator only)
+        self.atmosphere = None
 
     # -- batched core --------------------------------------------------------------------------------
     def _propagate(self, sats, tf, controller):
@@ -49,8 +52,10 @@ class Simulator:
             raise ValueError(f"unknown integrator {self.integrator!r} (rk45 | rk4)")
         if self.integrator == "rk45":
             mode["n_steps"] = np.zeros(len(sats), dtype=np.int32)
+        atmosphere = self.atmosphere if self.include_drag else None
         y, u, t, _ = batch.propagate_batch(y0, tf, controller, const, include_drag=self.include_drag,
-                                           include_J2=self.include_J2, T=T, device=self.device, **mode)
+                                           include_J2=self.include_J2, T=T, device=self.device, atmosphere=atmosphere,
+                                           **mode)
         # steps attempted per satellite by the replayed integrator (scipy's sol.nfev = 2 + 6 steps)
         self.last_n_steps = mode.get("n_steps")
         return y, u, t
