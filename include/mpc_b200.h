@@ -516,6 +516,28 @@ int mpc_discretize_batch_units_host(mpc_ctx *ctx, const double *x, const double 
                                     int32_t *status_host, int32_t *n_nodes_host);
 
 /*
+ * mpc_discretize_batch_rk23: the default quadrature mode (as mpc_discretize_batch_adaptive) with scipy's RK23 in place of
+ * RK45 -- the reference's Discretizer.ivp_solver = 'RK23' (solve_ivp(method='RK23')): Bogacki-Shampine 3(2), its own
+ * initial step and step-size controller, replayed per interval; the quadrature on the steps it accepts.  The arguments
+ * are those of mpc_discretize_batch_units without adaptive and n_sub:
+ *   consts    NULL: one constants bag (p; consts_scratch is then not used and may be NULL); else per-satellite
+ *             constants [n_sats], validated as in mpc_discretize_batch_units, with their DEVICE consts_scratch.
+ *   K_sat     NULL: a rectangular batch (K_max nodes everywhere; first may be NULL); else a ragged batch as in
+ *             mpc_discretize_batch_ragged (host counts, `first` their device prefix sums).
+ * n_nodes [n_sats (K_max - 1)] (may be NULL) receives len(sol.t) of every interval.  Not available: include_drag
+ * (MPC_E_UNSUPPORTED); u is on the nodes of x.
+ */
+int mpc_discretize_batch_rk23(const double *x, const double *u, const double *tf, const mpc_params *p,
+                              const mpc_sat_consts *consts, int n_sats, int K_max, const int32_t *K_sat, int64_t *first,
+                              double *consts_scratch, double rtol, double atol, double max_step, double *out, int64_t out_pitch,
+                              int64_t out_offset, int32_t *status, int32_t *n_nodes, void *stream);
+/* Host-buffer form (context-owned scratch); consts and K_sat as above. */
+int mpc_discretize_batch_rk23_host(mpc_ctx *ctx, const double *x, const double *u, const double *tf, const mpc_params *p,
+                                   const mpc_sat_consts *consts, int n_sats, int K_max, const int32_t *K_sat, double rtol,
+                                   double atol, double max_step, double *out_host, int32_t *status_host,
+                                   int32_t *n_nodes_host);
+
+/*
  * mpc_discretize_batch_ragged_gather: one rank's shard of a ragged batch (multi-GPU, satellites sharded over ranks), every
  * result stored into every rank's gathered buffer.  The gathered layout is the single-GPU ragged layout at a fixed
  * capacity K_cap: global satellite g on columns g (K_cap - 1) + k, k < K_g - 1.  A rank holding satellites [s0, s1)

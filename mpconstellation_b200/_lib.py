@@ -14,10 +14,10 @@ import numpy as np
 _HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(_HERE, "csrc")
 SO_PATH = os.path.join(CSRC, "libmpc_b200.so")
-# the drag-branch kernels, the per-satellite-constants kernels, the multi-destination ragged kernels and the RK45 replay
-# under an altitude-dependent atmosphere have a translation unit each
-SOURCES = ["mpc_b200.cu", "mpc_b200_drag.cu", "mpc_b200_units.cu", "mpc_b200_shard.cu", "mpc_b200_atmo.cu"]
-HEADERS = ["discretize_kernel.cuh", "discretize_adaptive_kernel.cuh", "discretize_default_kernel.cuh", "propagate_kernel.cuh", "propagate_rk45_kernel.cuh", "discretize_group_kernel.cuh", "constraint_terms_kernel.cuh", "discretize_drag_kernel.cuh", "discretize_pair_kernel.cuh", "mpc_b200_drag.h", "mpc_b200_units.h", "mpc_b200_shard.h", "mpc_b200_atmo.h", os.path.join("..", "..", "include", "mpc_b200.h")]
+# the drag-branch kernels, the per-satellite-constants kernels, the multi-destination ragged kernels, the RK45 replay
+# under an altitude-dependent atmosphere and the default quadrature mode with RK23 have a translation unit each
+SOURCES = ["mpc_b200.cu", "mpc_b200_drag.cu", "mpc_b200_units.cu", "mpc_b200_shard.cu", "mpc_b200_atmo.cu", "mpc_b200_rk23.cu"]
+HEADERS = ["discretize_kernel.cuh", "discretize_adaptive_kernel.cuh", "discretize_default_kernel.cuh", "propagate_kernel.cuh", "propagate_rk45_kernel.cuh", "discretize_group_kernel.cuh", "constraint_terms_kernel.cuh", "discretize_drag_kernel.cuh", "discretize_pair_kernel.cuh", "mpc_b200_drag.h", "mpc_b200_units.h", "mpc_b200_shard.h", "mpc_b200_atmo.h", "discretize_rk23_kernel.cuh", "mpc_b200_rk23.h", os.path.join("..", "..", "include", "mpc_b200.h")]
 # No -split-compile: with it nvcc partitions the module for parallel compilation and the register allocation of the
 # 250-register kernels comes out differently from build to build (the same source gave discretize_default_kernel 253
 # registers / 296 B of stack in one build and 255 / 536 B in the next: 1.366 vs 1.390 ms on BASELINE configs[2];
@@ -182,6 +182,8 @@ def lib():
                                                      ctypes.POINTER(ctypes.c_void_p), i, i64, i64, i, _DP, _DP, vp]
     L.mpc_propagate_batch_rk45_units.argtypes = [_DP, _DP, pp, _DP, pc, i, i, _DP, _DP, _DP, d, d, d, _DP, _DP, _DP, _DP, vp]
     L.mpc_propagate_batch_rk45_units_host.argtypes = [vp, _DP, _DP, pp, _DP, pc, i, i, _DP, _DP, d, d, d, _DP, _DP, _DP, _DP]
+    L.mpc_discretize_batch_rk23.argtypes = [_DP, _DP, _DP, pp, _DP, i, i, _DP, _DP, _DP, d, d, d, _DP, i64, i64, _DP, _DP, vp]
+    L.mpc_discretize_batch_rk23_host.argtypes = [vp, _DP, _DP, _DP, pp, _DP, i, i, _DP, d, d, d, _DP, _DP, _DP]
     pa = ctypes.POINTER(MpcAtmosphere)
     L.mpc_propagate_batch_rk45_atmo.argtypes = [_DP, _DP, pp, _DP, pc, i, i, _DP, _DP, _DP, d, d, d, _DP, _DP, _DP, _DP, pa, vp]
     L.mpc_propagate_batch_rk45_atmo_host.argtypes = [vp, _DP, _DP, pp, _DP, pc, i, i, _DP, _DP, d, d, d, _DP, _DP, _DP, _DP, pa]
@@ -200,7 +202,8 @@ def lib():
                  "mpc_constraint_terms_host", "mpc_discretize_batch_push", "mpc_fill_const_rows", "mpc_dynamics_jacobian",
                  "mpc_constraint_terms_ragged", "mpc_constraint_terms_ragged_host", "mpc_dynamics_jacobian_ragged",
                  "mpc_discretize_batch_units", "mpc_discretize_batch_units_host", "mpc_propagate_batch_rk45_units",
-                 "mpc_propagate_batch_rk45_units_host", "mpc_discretize_batch_ragged_gather", "mpc_constraint_terms_units", "mpc_constraint_terms_units_host"):
+                 "mpc_propagate_batch_rk45_units_host", "mpc_discretize_batch_ragged_gather", "mpc_constraint_terms_units", "mpc_constraint_terms_units_host",
+                 "mpc_discretize_batch_rk23", "mpc_discretize_batch_rk23_host"):
         getattr(L, name).restype = i
     _lib = L
     return L
@@ -222,6 +225,7 @@ EXPORTED_SYMBOLS = [
     "mpc_propagate_batch_rk45_units_host", "mpc_constraint_terms_units", "mpc_constraint_terms_units_host",
     "mpc_discretize_batch_ragged_gather", "mpc_fp64_peak_probe", "mpc_set_tuning", "mpc_set_gather_tuning",
     "mpc_propagate_batch_rk45_atmo", "mpc_propagate_batch_rk45_atmo_host",
+    "mpc_discretize_batch_rk23", "mpc_discretize_batch_rk23_host",
 ]
 
 

@@ -121,6 +121,22 @@ def _counts(c, n, cmax, what):
     return c
 
 
+def _rk23(adaptive, include_drag=False, ugrid=False):
+    """True when adaptive asks for scipy's RK23 (adaptive["method"]; missing or "RK45": the RK45 replay).  Raises
+    NotImplementedError, before any device work, for another method and for what RK23 has no device form of."""
+    method = (adaptive or {}).get("method", "RK45")
+    if method == "RK45":
+        return False
+    if method != "RK23":
+        raise NotImplementedError(f"adaptive method {method!r}: the device replays scipy's RK45 and RK23 only; "
+                                  "DOP853 and the implicit methods have no device form and there is no CPU fallback")
+    if include_drag:
+        raise NotImplementedError("RK23 with include_drag: the drag linearisation is replayed with RK45 only")
+    if ugrid:
+        raise NotImplementedError("RK23 with u on its own grid: the RK23 replay needs u on the nodes of x")
+    return True
+
+
 def discretize_batch(x, u, tf, const, include_J2=False, include_drag=False, n_sub=100, out=None, status=None,
                      device=0, check=True, adaptive=None, disc_drag=None, K=None):
     """Discretize every interval of every satellite in one launch sequence (host arrays).
@@ -135,6 +151,9 @@ def discretize_batch(x, u, tf, const, include_J2=False, include_drag=False, n_su
     include_drag=True needs disc_drag=(CD, rho): const.CD and the (constant) value of rho_func the reference's drag
     branch reads (linearize_discretize.py:162-168); without them the call is rejected like the reference's.
 
+    adaptive=dict(method="RK23", ...): the same with scipy's RK23 controller (Discretizer.ivp_solver = 'RK23'); u on the
+    nodes of x, no drag.  A missing method or "RK45" is the RK45 replay; any other method raises NotImplementedError.
+
     K=None: every satellite on the K = x.shape[2] nodes.  K = int array [N]: a ragged batch -- satellite s on its own
     K_s <= x.shape[2] nodes (the first K_s columns of x[s], u[s]), one launch for all; the result keeps the layout of
     Kmax = x.shape[2] with NaN in the padding columns (DiscretizedBatch.sat(s) returns K_s - 1 intervals).  u must be on
@@ -145,6 +164,8 @@ def discretize_batch(x, u, tf, const, include_J2=False, include_drag=False, n_su
     the seven per-scale fields take the single-constant launches.  Per-satellite constants need u on the nodes of x and
     are not available with include_drag.
     """
+    rk23 = adaptive is not None and _rk23(adaptive, include_drag, np.ndim(u) == 3 and np.ndim(x) == 3 and
+                                          np.shape(u)[2] != np.shape(x)[2])
     ctx = _ctx(device)
     counts, K = K, None
     x = _f64(x)
@@ -172,7 +193,13 @@ def discretize_batch(x, u, tf, const, include_J2=False, include_drag=False, n_su
         if Ku != K:
             raise ValueError("a ragged batch needs u on the nodes of x ([N,3,Kmax])")
     with _lock(device):
-        if psc is not None:
+        if rk23:
+            n_nodes = np.zeros(n_int, dtype=np.int32)
+            _lib.check(_lib.lib().mpc_discretize_batch_rk23_host(
+                ctx, _lib.addr(x), _lib.addr(u), _lib.addr(tfv), ctypes.byref(p), psc, N, K, _lib.addr(K_sat),
+                float(adaptive.get("rtol", 1e-3)), float(adaptive.get("atol", 1e-6)), float(adaptive.get("max_step", 1e-2)),
+                _lib.addr(out), _lib.addr(status), _lib.addr(n_nodes)))
+        elif psc is not None:
             ad = adaptive or {}
             n_nodes = np.zeros(n_int, dtype=np.int32) if adaptive is not None else None
             _lib.check(_lib.lib().mpc_discretize_batch_units_host(
@@ -443,7 +470,11 @@ def discretize_batch_device(x, u, tf, const, include_J2=False, n_sub=100, out=No
     K = int array [N] (host): a ragged batch as in discretize_batch (x, u [N,.,Kmax]); `first` is an int64 CUDA tensor
     [N+1] the call fills with the prefix sums of K_s - 1 (allocated when None).  The padding columns of `out` are not
     written; status (zeroed when allocated here) and n_nodes keep the [N*(Kmax-1)] layout.
-    const: one Constants bag or a sequence of N, as in discretize_batch (no extra_dst with per-satellite constants)."""
+    const: one Constants bag or a sequence of N, as in discretize_batch (no extra_dst with per-satellite constants).
+    adaptive=dict(method="RK23", ...): scipy's RK23 controller, as in discretize_batch (one destination)."""
+    rk23 = adaptive is not None and _rk23(adaptive)
+    if rk23 and extra_dst:
+        raise NotImplementedError("RK23 stores into one destination (no extra_dst)")
     torch = _torch()
     N, _, K_ = x.shape
     n_int = N * (K_ - 1)
@@ -467,7 +498,17 @@ def discretize_batch_device(x, u, tf, const, include_J2=False, n_sub=100, out=No
     p = _lib.make_params(const, include_J2, False)
     stream = torch.cuda.current_stream(x.device).cuda_stream
     L = _lib.lib()
-    if psc is not None:
+    if rk23:
+        scratch = None if psc is None else torch.empty(N * _lib.SAT_SCRATCH_DOUBLES, dtype=torch.float64, device=x.device)
+        _lib.check(L.mpc_discretize_batch_rk23(
+            x.data_ptr(), u.data_ptr(), tf.data_ptr(), ctypes.byref(p), psc, N, K_, _lib.addr(K_sat),
+            first.data_ptr() if first is not None else None, scratch.data_ptr() if scratch is not None else None,
+            float(adaptive.get("rtol", 1e-3)), float(adaptive.get("atol", 1e-6)), float(adaptive.get("max_step", 1e-2)),
+            out.data_ptr(), pitch, int(out_offset), status.data_ptr(), n_nodes.data_ptr() if n_nodes is not None else None,
+            stream))
+        if scratch is not None:
+            scratch.record_stream(torch.cuda.current_stream(x.device))
+    elif psc is not None:
         ad = adaptive or {}
         scratch = torch.empty(N * _lib.SAT_SCRATCH_DOUBLES, dtype=torch.float64, device=x.device)
         _lib.check(L.mpc_discretize_batch_units(

@@ -25,6 +25,7 @@
 #include "mpc_b200_units.h"
 #include "mpc_b200_shard.h"
 #include "mpc_b200_atmo.h"
+#include "mpc_b200_rk23.h"
 #include "constraint_terms_kernel.cuh"
 #include "discretize_drag_kernel.cuh"
 #include "discretize_pair_kernel.cuh"
@@ -348,6 +349,7 @@ struct AdaptiveOpts {   // scipy solve_ivp(RK45) controls of the reference's def
     int drag = 0;           // drag branch of the linearisation (set from mpc_params by with_drag)
     double kf = 0.0;
     mpc::DragLin lin{};     // density model of the Jacobian's drag terms
+    int rk23 = 0;           // scipy's RK23 in place of RK45 (mpc_discretize_batch_rk23[_host]; mpc_b200_rk23.cu)
 };
 
 template <bool J2, bool GENU>
@@ -757,6 +759,54 @@ int check_ragged_disc(const double *x, const double *u, const double *tf, const 
     if (p->include_drag) return fail(MPC_E_UNSUPPORTED, "the drag linearisation is not implemented for ragged batches");
     if (adaptive && (rc = check_adaptive(rtol, atol, max_step))) return rc;
     return check_counts(K_sat, n_sats, K_max, "K_sat");
+}
+
+// ---- the default quadrature mode with scipy's RK23 (mpc_discretize_batch_rk23[_host]) ------------------------------------
+// consts == nullptr: one constants bag; K_sat == nullptr: a rectangular batch.  The constants are validated as the
+// *_units entries validate them; there is no drag branch.
+int check_rk23_disc(const double *x, const double *u, const double *tf, const mpc_params *p, const mpc_sat_consts *consts,
+                    int n_sats, int K_max, const int32_t *K_sat, double rtol, double atol, double max_step)
+{
+    int rc = check_disc_args(x, u, tf, p, n_sats, K_max, 1);
+    if (rc) return rc;
+    if (p->include_drag) return fail(MPC_E_UNSUPPORTED, "the drag linearisation is not implemented with RK23");
+    if ((rc = check_adaptive(rtol, atol, max_step))) return rc;
+    if (K_sat && (rc = check_counts(K_sat, n_sats, K_max, "K_sat"))) return rc;
+    if (consts && (rc = check_sat_consts(consts, n_sats))) return rc;
+    if (mpc_rk23_sizeof() != sizeof(mpc::DiscParams)) return fail(MPC_E_CUDA, "mpc_b200_rk23.cu was built against different parameter structs");
+    return MPC_SUCCESS;
+}
+
+// One launch for the batch (psc: device DiscParams [n_sats] or nullptr; first: device prefix sums or nullptr).  The
+// block size follows the default-mode launchers: one-warp CTAs below 148 x 256 threads, full 256-thread CTAs otherwise.
+int launch_rk23(const double *x, const double *u, const double *tf, const mpc::DiscParams &P, const mpc::DiscParams *psc,
+                bool j2, int n_sats, int K, long long n_units, const long long *first, const AdaptiveOpts &o, double *out,
+                long long pitch, long long offset, int32_t *status, cudaStream_t st)
+{
+    MpcRk23Disc a{};
+    a.x = x;
+    a.u = u;
+    a.tf = tf;
+    a.P = &P;
+    a.psc = psc;
+    a.first = first;
+    a.n_units = n_units;
+    a.include_j2 = j2;
+    a.n_sats = n_sats;
+    a.K = K;
+    a.block = n_units < 148LL * 256 ? 32 : 256;
+    a.rtol = o.rtol;
+    a.atol = o.atol;
+    a.max_step = o.max_step;
+    a.out = out;
+    a.pitch = pitch;
+    a.offset = offset;
+    a.status = status;
+    a.n_nodes = o.n_nodes;
+    a.stream = st;
+    CUDA_TRY(mpc_rk23_launch_disc(&a));
+    g_launches.fetch_add(1, std::memory_order_relaxed);
+    return MPC_SUCCESS;
 }
 
 int check_ctrl(const mpc_controller *c)
@@ -1344,7 +1394,9 @@ static int disc_host(mpc_ctx *ctx, const double *x, const double *u, const doubl
                      int32_t *n_nodes_host, const int32_t *K_sat = nullptr, const mpc_sat_consts *consts = nullptr)
 {
     if (!ctx || !out_host) return fail(MPC_E_INVALID, "null ctx/out");
-    int rc = consts ? check_units_disc(x, u, tf, p, consts, n_sats, K, K_sat, ad != nullptr, n_sub, ad ? ad->rtol : 0.0,
+    const bool rk23 = ad && ad->rk23;
+    int rc = rk23 ? check_rk23_disc(x, u, tf, p, consts, n_sats, K, K_sat, ad->rtol, ad->atol, ad->max_step)
+           : consts ? check_units_disc(x, u, tf, p, consts, n_sats, K, K_sat, ad != nullptr, n_sub, ad ? ad->rtol : 0.0,
                                        ad ? ad->atol : 0.0, ad ? ad->max_step : 0.0)
            : K_sat ? check_ragged_disc(x, u, tf, p, n_sats, K, K_sat, ad != nullptr, n_sub, ad ? ad->rtol : 0.0, ad ? ad->atol : 0.0,
                                        ad ? ad->max_step : 0.0)
@@ -1387,7 +1439,20 @@ static int disc_host(mpc_ctx *ctx, const double *x, const double *u, const doubl
         mpc::DstTab tab{};
         tab.p[0] = ctx->d_out;
         const long long off = (long long)s0 * (K - 1);
-        if (consts && !K_sat) {
+        if (rk23) {
+            AdaptiveOpts o = *ad;
+            o.n_nodes = n_nodes_host ? ctx->d_nodes + off : nullptr;
+            long long n_units = (long long)ns * (K - 1);
+            if (K_sat) {   // the padding columns as in the ragged branch below
+                CUDA_TRY(cudaMemset2DAsync(ctx->d_out + off, (size_t)n_int * sizeof(double), 0xFF, (size_t)n_units * sizeof(double),
+                                           MPC_OUT_ROWS, ctx->s_compute));
+                CUDA_TRY(cudaMemsetAsync(ctx->d_status + off, 0, (size_t)n_units * sizeof(int32_t), ctx->s_compute));
+                if (n_nodes_host) CUDA_TRY(cudaMemsetAsync(ctx->d_nodes + off, 0, (size_t)n_units * sizeof(int32_t), ctx->s_compute));
+                n_units = first[s0 + ns] - first[s0];
+            }
+            rc = launch_rk23(dx, du, ctx->d_tf + s0, P, consts ? psc + s0 : nullptr, p->include_j2, ns, K, n_units,
+                             K_sat ? ctx->d_first + s0 : nullptr, o, ctx->d_out, n_int, off, ctx->d_status + off, ctx->s_compute);
+        } else if (consts && !K_sat) {
             AdaptiveOpts o = ad ? *ad : AdaptiveOpts{};
             o.n_nodes = (ad && n_nodes_host) ? ctx->d_nodes + off : nullptr;
             rc = launch_units_disc(dx, du, ctx->d_tf + s0, psc + s0, p->include_j2, ns, K, (long long)ns * (K - 1), nullptr,
@@ -1700,6 +1765,42 @@ int mpc_discretize_batch_units_host(mpc_ctx *ctx, const double *x, const double 
     }
     return disc_host(ctx, x, u, tf, p, n_sats, K_max, adaptive ? 1 : n_sub, adaptive ? &o : nullptr, out_host, status_host,
                      adaptive ? n_nodes_host : nullptr, K_sat, consts);
+}
+
+// ---- the default quadrature mode with scipy's RK23 ---------------------------------------------------------------------
+int mpc_discretize_batch_rk23(const double *x, const double *u, const double *tf, const mpc_params *p,
+                              const mpc_sat_consts *consts, int n_sats, int K_max, const int32_t *K_sat, int64_t *first,
+                              double *consts_scratch, double rtol, double atol, double max_step, double *out, int64_t out_pitch,
+                              int64_t out_offset, int32_t *status, int32_t *n_nodes, void *stream)
+{
+    int rc = check_rk23_disc(x, u, tf, p, consts, n_sats, K_max, K_sat, rtol, atol, max_step);
+    if (rc) return rc;
+    if (!out || (K_sat && !first)) return fail(MPC_E_INVALID, "null output / first");
+    if (out_pitch < out_offset + (long long)n_sats * (K_max - 1) || out_offset < 0)
+        return fail(MPC_E_INVALID, "out_pitch/out_offset do not hold the batch");
+    if (n_sats == 0) return MPC_SUCCESS;
+    cudaStream_t st = (cudaStream_t)stream;
+    if (consts && (rc = upload_sat_table<mpc::DiscParams>(p, consts, n_sats, consts_scratch, st, disc_params))) return rc;
+    long long n_units = (long long)n_sats * (K_max - 1);
+    if (K_sat) {
+        const std::vector<long long> f = ragged_first(K_sat, n_sats);
+        CUDA_TRY(cudaMemcpyAsync(first, f.data(), f.size() * sizeof(long long), cudaMemcpyHostToDevice, st));
+        n_units = f[n_sats];
+    }
+    const AdaptiveOpts o{rtol, atol, max_step, n_nodes};
+    return launch_rk23(x, u, tf, disc_params(p), consts ? (const mpc::DiscParams *)consts_scratch : nullptr, p->include_j2,
+                       n_sats, K_max, n_units, K_sat ? (const long long *)first : nullptr, o, out, out_pitch, out_offset,
+                       status, st);
+}
+
+int mpc_discretize_batch_rk23_host(mpc_ctx *ctx, const double *x, const double *u, const double *tf, const mpc_params *p,
+                                   const mpc_sat_consts *consts, int n_sats, int K_max, const int32_t *K_sat, double rtol,
+                                   double atol, double max_step, double *out_host, int32_t *status_host,
+                                   int32_t *n_nodes_host)
+{
+    AdaptiveOpts o{rtol, atol, max_step, nullptr};
+    o.rk23 = 1;
+    return disc_host(ctx, x, u, tf, p, n_sats, K_max, 1, &o, out_host, status_host, n_nodes_host, K_sat, consts);
 }
 
 int mpc_propagate_batch_rk45_units(const double *y0, const double *tf, const mpc_params *p, const mpc_sat_consts *consts,

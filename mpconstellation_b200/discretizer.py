@@ -110,9 +110,16 @@ class Discretizer:
                 raise AttributeError("'Constants' object has no attribute 'CD'")
             if self.drho_func is None:
                 raise TypeError("'NoneType' object is not callable")
-        if self.ivp_solver != 'RK45':
-            raise NotImplementedError(f"ivp_solver={self.ivp_solver!r}: the device integrator is a fixed-step 4th-order Runge-Kutta method "
-                                      "on the reference's node grid (stated against RK45)")
+        if self.ivp_solver not in ('RK45', 'RK23'):
+            raise NotImplementedError(f"ivp_solver={self.ivp_solver!r}: the device replays scipy's RK45 and RK23 only; "
+                                      "DOP853 and the implicit methods have no device form and there is no CPU fallback")
+        if self.ivp_solver == 'RK23' and self.use_uniform_steps:
+            raise NotImplementedError(
+                "ivp_solver='RK23' with use_uniform_steps=True: the reference then integrates on RK23's dense output at "
+                "the integrator_steps nodes, which is 1.9e-6 from the converged flow, so the fixed-step device integrator "
+                "is no stand-in; only the default quadrature mode (use_uniform_steps=False) replays RK23")
+        if self.ivp_solver == 'RK23' and self.include_drag:
+            raise NotImplementedError("ivp_solver='RK23' with include_drag: the drag linearisation is replayed with RK45 only")
         if self.use_uniform_steps and int(self.integrator_steps) < 2:
             raise ValueError("integrator_steps must be >= 2")
 
@@ -156,8 +163,9 @@ class Discretizer:
         # use_uniform_steps=False (the reference default): quadrature on the steps scipy's RK45 controller accepts
         # (replayed on the device, scipy's default rtol/atol as the reference passes none);
         # use_uniform_steps=True: fixed-step fourth-order Runge-Kutta(-Nystrom) on the uniform integrator_steps grid.
+        # ivp_solver = 'RK23' (default mode only, _check_options): scipy's RK23 controller replayed the same way.
         adaptive = None if self.use_uniform_steps else dict(rtol=self.ivp_rtol, atol=self.ivp_atol,
-                                                            max_step=float(self.ivp_max_step))
+                                                            max_step=float(self.ivp_max_step), method=self.ivp_solver)
         return batch.discretize_batch(x, u, tf, self.const, include_J2=self.include_J2,
                                       include_drag=bool(self.include_drag), disc_drag=self._disc_drag(x),
                                       n_sub=max(1, int(self.integrator_steps) - 1), out=out, device=self.device,
