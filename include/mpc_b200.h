@@ -629,6 +629,50 @@ int mpc_constraint_terms_units_host(mpc_ctx *ctx, const double *x, const double 
                                     const int32_t *K_sat, const mpc_sat_consts *consts, double *rbar_hat, double *ubar_hat,
                                     double *final_terms);
 
+/* ---------------------------------------------------------------- conjunction screening */
+
+/*
+ * Close approaches between every pair of satellites of one propagation (mpc_propagate_batch*: y [n_sats][7][T],
+ * normalized, sampled at T common instants).  Satellite s is taken to SI with scale[s] = (R0_s, R0_s / s0_s): position
+ * y[0:3] R0_s (m), velocity y[3:6] R0_s / s0_s (m/s); the run lasts `duration` seconds for every satellite (sample k at
+ * t_k = k h, h = duration / (T - 1)); the mass row is not read.  Between two samples each satellite follows the cubic
+ * Hermite curve through its positions and velocities there.  An event is a local minimum of a pair's distance d(t) on
+ * [0, duration] with d < threshold: t = 0 counts when d increases there, t = duration when d does not increase there,
+ * and a minimum belongs to the interval whose half-open [t_k, t_k+1) holds it (the last interval is closed).
+ * An interval with a non-finite end sample of satellite s is skipped for every pair with s, and counted in skipped[s].
+ */
+typedef struct mpc_conjunction {
+    int32_t i, j;      /* satellites, i < j */
+    int32_t k;         /* interval [t_k, t_k+1] */
+    int32_t flags;     /* MPC_CONJ_FLAG_* */
+    double t_ca;       /* s from the start of the run */
+    double d_min;      /* m */
+    double v_rel;      /* m/s at t_ca */
+} mpc_conjunction;
+/* the root isolation reached its depth cap (pieces of 2^-20 of an interval) before isolating this minimum: t_ca is
+ * then known to that width only */
+#define MPC_CONJ_FLAG_DEPTH 1
+
+/* doubles of device scratch mpc_screen_conjunctions needs: n_sats (6 T + 4 (T - 1) + 2) */
+int64_t mpc_conjunction_scratch_doubles(int n_sats, int T);
+
+/*
+ * mpc_screen_conjunctions: y [n_sats][7][T] DEVICE; scale [n_sats][2] HOST (every value finite and > 0); duration > 0
+ * (s) and threshold > 0 (m) finite; scratch DEVICE of mpc_conjunction_scratch_doubles(n_sats, T); events DEVICE
+ * [capacity] (capacity >= 0; may be NULL when 0) in no particular order; counters DEVICE [2] receives the number of
+ * events found (which may exceed capacity: only the first `capacity` are stored) and the number with
+ * MPC_CONJ_FLAG_DEPTH; skipped DEVICE [n_sats].  Two kernel launches on `stream`; nothing is synchronized.
+ * MPC_E_INVALID before any device call: a null pointer, n_sats < 2, T < 2, a bad duration, threshold or scale.
+ */
+int mpc_screen_conjunctions(const double *y, int n_sats, int T, const double *scale, double duration, double threshold,
+                            double *scratch, mpc_conjunction *events, int64_t capacity, uint64_t *counters,
+                            int32_t *skipped, void *stream);
+/* Host-buffer form (context-owned device buffers; returns when the results are in the host buffers): *count and
+ * *n_flagged as counters above; min(*count, capacity) events in events_host, in no particular order. */
+int mpc_screen_conjunctions_host(mpc_ctx *ctx, const double *y, int n_sats, int T, const double *scale, double duration,
+                                 double threshold, mpc_conjunction *events_host, int64_t capacity, int64_t *count,
+                                 int64_t *n_flagged, int32_t *skipped_host);
+
 /* ---------------------------------------------------------------- measurement helpers */
 
 /* FP64 FMA-chain microbenchmark: measured DFMA peak of `device` in TFLOP/s (2 flop per FMA). */

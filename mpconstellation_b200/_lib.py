@@ -15,9 +15,11 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(_HERE, "csrc")
 SO_PATH = os.path.join(CSRC, "libmpc_b200.so")
 # the drag-branch kernels, the per-satellite-constants kernels, the multi-destination ragged kernels, the RK45 replay
-# under an altitude-dependent atmosphere and the default quadrature mode with RK23 have a translation unit each
-SOURCES = ["mpc_b200.cu", "mpc_b200_drag.cu", "mpc_b200_units.cu", "mpc_b200_shard.cu", "mpc_b200_atmo.cu", "mpc_b200_rk23.cu"]
-HEADERS = ["discretize_kernel.cuh", "discretize_adaptive_kernel.cuh", "discretize_default_kernel.cuh", "propagate_kernel.cuh", "propagate_rk45_kernel.cuh", "discretize_group_kernel.cuh", "constraint_terms_kernel.cuh", "discretize_drag_kernel.cuh", "discretize_pair_kernel.cuh", "mpc_b200_drag.h", "mpc_b200_units.h", "mpc_b200_shard.h", "mpc_b200_atmo.h", "discretize_rk23_kernel.cuh", "mpc_b200_rk23.h", os.path.join("..", "..", "include", "mpc_b200.h")]
+# under an altitude-dependent atmosphere, the default quadrature mode with RK23 and the conjunction screening have a
+# translation unit each
+SOURCES = ["mpc_b200.cu", "mpc_b200_drag.cu", "mpc_b200_units.cu", "mpc_b200_shard.cu", "mpc_b200_atmo.cu", "mpc_b200_rk23.cu",
+           "mpc_b200_conj.cu"]
+HEADERS = ["discretize_kernel.cuh", "discretize_adaptive_kernel.cuh", "discretize_default_kernel.cuh", "propagate_kernel.cuh", "propagate_rk45_kernel.cuh", "discretize_group_kernel.cuh", "constraint_terms_kernel.cuh", "discretize_drag_kernel.cuh", "discretize_pair_kernel.cuh", "mpc_b200_drag.h", "mpc_b200_units.h", "mpc_b200_shard.h", "mpc_b200_atmo.h", "discretize_rk23_kernel.cuh", "mpc_b200_rk23.h", "conjunction_kernel.cuh", "mpc_b200_conj.h", os.path.join("..", "..", "include", "mpc_b200.h")]
 # No -split-compile: with it nvcc partitions the module for parallel compilation and the register allocation of the
 # 250-register kernels comes out differently from build to build (the same source gave discretize_default_kernel 253
 # registers / 296 B of stack in one build and 255 / 536 B in the next: 1.366 vs 1.390 ms on BASELINE configs[2];
@@ -76,6 +78,11 @@ class MpcGatherOpts(ctypes.Structure):
 
 
 LAYOUT_SAT_MAJOR, LAYOUT_K_MAJOR = 0, 1
+
+# mpc_conjunction, one close approach (include/mpc_b200.h)
+CONJUNCTION_DTYPE = np.dtype([("i", "<i4"), ("j", "<i4"), ("k", "<i4"), ("flags", "<i4"), ("t_ca", "<f8"), ("d_min", "<f8"),
+                              ("v_rel", "<f8")])
+CONJ_FLAG_DEPTH = 1     # MPC_CONJ_FLAG_DEPTH
 
 
 class MpcError(RuntimeError):
@@ -189,6 +196,10 @@ def lib():
     L.mpc_propagate_batch_rk45_atmo_host.argtypes = [vp, _DP, _DP, pp, _DP, pc, i, i, _DP, _DP, d, d, d, _DP, _DP, _DP, _DP, pa]
     L.mpc_constraint_terms_units.argtypes = [_DP, _DP, i, i, _DP, _DP, _DP, _DP, _DP, _DP, _DP, vp]
     L.mpc_constraint_terms_units_host.argtypes = [vp, _DP, _DP, i, i, _DP, _DP, _DP, _DP, _DP]
+    L.mpc_conjunction_scratch_doubles.argtypes = [i, i]
+    L.mpc_conjunction_scratch_doubles.restype = i64
+    L.mpc_screen_conjunctions.argtypes = [_DP, i, i, _DP, d, d, _DP, _DP, i64, _DP, _DP, vp]
+    L.mpc_screen_conjunctions_host.argtypes = [vp, _DP, i, i, _DP, d, d, _DP, i64, ctypes.POINTER(i64), ctypes.POINTER(i64), _DP]
     L.mpc_fp64_peak_probe.argtypes = [i, i, ctypes.POINTER(ctypes.c_double), ctypes.POINTER(ctypes.c_double)]
     L.mpc_set_gather_tuning.argtypes = [i, i]
     L.mpc_set_gather_tuning.restype = i
@@ -203,7 +214,8 @@ def lib():
                  "mpc_constraint_terms_ragged", "mpc_constraint_terms_ragged_host", "mpc_dynamics_jacobian_ragged",
                  "mpc_discretize_batch_units", "mpc_discretize_batch_units_host", "mpc_propagate_batch_rk45_units",
                  "mpc_propagate_batch_rk45_units_host", "mpc_discretize_batch_ragged_gather", "mpc_constraint_terms_units", "mpc_constraint_terms_units_host",
-                 "mpc_discretize_batch_rk23", "mpc_discretize_batch_rk23_host"):
+                 "mpc_discretize_batch_rk23", "mpc_discretize_batch_rk23_host", "mpc_screen_conjunctions",
+                 "mpc_screen_conjunctions_host"):
         getattr(L, name).restype = i
     _lib = L
     return L
@@ -226,6 +238,7 @@ EXPORTED_SYMBOLS = [
     "mpc_discretize_batch_ragged_gather", "mpc_fp64_peak_probe", "mpc_set_tuning", "mpc_set_gather_tuning",
     "mpc_propagate_batch_rk45_atmo", "mpc_propagate_batch_rk45_atmo_host",
     "mpc_discretize_batch_rk23", "mpc_discretize_batch_rk23_host",
+    "mpc_conjunction_scratch_doubles", "mpc_screen_conjunctions", "mpc_screen_conjunctions_host",
 ]
 
 

@@ -26,6 +26,7 @@
 #include "mpc_b200_shard.h"
 #include "mpc_b200_atmo.h"
 #include "mpc_b200_rk23.h"
+#include "mpc_b200_conj.h"
 #include "constraint_terms_kernel.cuh"
 #include "discretize_drag_kernel.cuh"
 #include "discretize_pair_kernel.cuh"
@@ -1023,6 +1024,10 @@ struct mpc_ctx {
     size_t cap_first = 0, cap_cnt = 0;
     double *d_psc = nullptr;                 // per-satellite constants: the derived kernel constants (*_units_host)
     size_t cap_psc = 0;
+    double *d_conj = nullptr;                // conjunction screening (mpc_screen_conjunctions_host): scratch, events,
+    double *d_conj_ev = nullptr;             // counters
+    unsigned long long *d_conj_cnt = nullptr;
+    size_t cap_conj = 0, cap_conj_ev = 0, cap_conj_cnt = 0;
     cudaStream_t s_pushk = nullptr;          // high-priority stream of the copy kernels (push gather, SM-driven variant)
     cudaStream_t s_aux[3] = {};              // compute streams the chunk kernels of the push gather rotate over
     cudaStream_t s_push[MPC_MAX_DST] = {};   // one stream per peer for the copy-engine gather (mpc_discretize_batch_push)
@@ -1365,6 +1370,9 @@ int mpc_ctx_destroy(mpc_ctx *c)
     cudaFree(c->d_first);
     cudaFree(c->d_cnt);
     cudaFree(c->d_psc);
+    cudaFree(c->d_conj);
+    cudaFree(c->d_conj_ev);
+    cudaFree(c->d_conj_cnt);
     if (c->h_stage) cudaFreeHost(c->h_stage);
     delete c;
     return MPC_SUCCESS;
@@ -1801,6 +1809,79 @@ int mpc_discretize_batch_rk23_host(mpc_ctx *ctx, const double *x, const double *
     AdaptiveOpts o{rtol, atol, max_step, nullptr};
     o.rk23 = 1;
     return disc_host(ctx, x, u, tf, p, n_sats, K_max, 1, &o, out_host, status_host, n_nodes_host, K_sat, consts);
+}
+
+// ---- conjunction screening (mpc_screen_conjunctions[_host]; mpc_b200_conj.cu) -------------------------------------------
+
+static int check_conj(const double *y, int n_sats, int T, const double *scale, double duration, double threshold)
+{
+    if (!y || !scale) return fail(MPC_E_INVALID, "null y / scale");
+    if (n_sats < 2 || T < 2) return fail(MPC_E_INVALID, "need n_sats >= 2 and T >= 2 (got %d, %d)", n_sats, T);
+    if (!(std::isfinite(duration) && duration > 0.0)) return fail(MPC_E_INVALID, "need a finite duration > 0 (got %g)", duration);
+    if (!(std::isfinite(threshold) && threshold > 0.0))
+        return fail(MPC_E_INVALID, "need a finite threshold > 0 (got %g)", threshold);
+    for (int s = 0; s < n_sats; ++s)
+        for (int c = 0; c < 2; ++c)
+            if (!(std::isfinite(scale[2 * s + c]) && scale[2 * s + c] > 0.0))
+                return fail(MPC_E_INVALID, "scale[%d][%d] = %g: every scale must be finite and > 0", s, c, scale[2 * s + c]);
+    if (mpc_conj_record_size() != sizeof(mpc_conjunction))
+        return fail(MPC_E_CUDA, "mpc_b200_conj.cu was built against a different event record");
+    return MPC_SUCCESS;
+}
+
+int64_t mpc_conjunction_scratch_doubles(int n_sats, int T)
+{
+    return n_sats < 0 || T < 2 ? 0 : (int64_t)mpc_conj_scratch_doubles(n_sats, T);
+}
+
+int mpc_screen_conjunctions(const double *y, int n_sats, int T, const double *scale, double duration, double threshold,
+                            double *scratch, mpc_conjunction *events, int64_t capacity, uint64_t *counters,
+                            int32_t *skipped, void *stream)
+{
+    int rc = check_conj(y, n_sats, T, scale, duration, threshold);
+    if (rc) return rc;
+    if (!scratch || !counters || !skipped || capacity < 0 || (capacity > 0 && !events))
+        return fail(MPC_E_INVALID, "null scratch / counters / skipped, or no events buffer for capacity %lld", (long long)capacity);
+    MpcConjLaunch a{y, scratch, scale, n_sats, T, duration / (T - 1), threshold, events, capacity,
+                    (unsigned long long *)counters, skipped, (cudaStream_t)stream};
+    CUDA_TRY(mpc_conj_launch(&a));
+    g_launches.fetch_add(2, std::memory_order_relaxed);
+    return MPC_SUCCESS;
+}
+
+int mpc_screen_conjunctions_host(mpc_ctx *ctx, const double *y, int n_sats, int T, const double *scale, double duration,
+                                 double threshold, mpc_conjunction *events_host, int64_t capacity, int64_t *count,
+                                 int64_t *n_flagged, int32_t *skipped_host)
+{
+    if (!ctx || !count || !n_flagged || !skipped_host || capacity < 0 || (capacity > 0 && !events_host))
+        return fail(MPC_E_INVALID, "null ctx / count / n_flagged / skipped, or no events buffer for capacity %lld", (long long)capacity);
+    int rc = check_conj(y, n_sats, T, scale, duration, threshold);
+    if (rc) return rc;
+    CUDA_TRY(cudaSetDevice(ctx->device));
+    const size_t ev_doubles = (size_t)std::max<int64_t>(capacity, 1) * (sizeof(mpc_conjunction) / sizeof(double));
+    if ((rc = ensure(ctx->d_x, ctx->cap_x, (size_t)n_sats * 7 * T))) return rc;
+    if ((rc = ensure(ctx->d_conj, ctx->cap_conj, (size_t)mpc_conj_scratch_doubles(n_sats, T)))) return rc;
+    if ((rc = ensure(ctx->d_conj_ev, ctx->cap_conj_ev, ev_doubles))) return rc;
+    if ((rc = ensure(ctx->d_conj_cnt, ctx->cap_conj_cnt, 2))) return rc;
+    if ((rc = ensure(ctx->d_status, ctx->cap_status, (size_t)n_sats))) return rc;
+    cudaStream_t st = ctx->s_compute;
+    CUDA_TRY(cudaMemcpyAsync(ctx->d_x, y, (size_t)n_sats * 7 * T * sizeof(double), cudaMemcpyHostToDevice, st));
+    MpcConjLaunch a{ctx->d_x, ctx->d_conj, scale, n_sats, T, duration / (T - 1), threshold, ctx->d_conj_ev, capacity,
+                    ctx->d_conj_cnt, ctx->d_status, st};
+    CUDA_TRY(mpc_conj_launch(&a));
+    g_launches.fetch_add(2, std::memory_order_relaxed);
+    unsigned long long cnt[2];
+    CUDA_TRY(cudaMemcpyAsync(cnt, ctx->d_conj_cnt, sizeof cnt, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaMemcpyAsync(skipped_host, ctx->d_status, (size_t)n_sats * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    const long long n_out = std::min<long long>((long long)cnt[0], capacity);
+    if (n_out > 0) {
+        CUDA_TRY(cudaMemcpyAsync(events_host, ctx->d_conj_ev, (size_t)n_out * sizeof(mpc_conjunction), cudaMemcpyDeviceToHost, st));
+        CUDA_TRY(cudaStreamSynchronize(st));
+    }
+    *count = (int64_t)cnt[0];
+    *n_flagged = (int64_t)cnt[1];
+    return MPC_SUCCESS;
 }
 
 int mpc_propagate_batch_rk45_units(const double *y0, const double *tf, const mpc_params *p, const mpc_sat_consts *consts,
